@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- MC-dropout tiles/sec of the B200-native Xception-UQ + UQ-thresholding hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one synthetic whole-slide image per GPU (BASELINE.json
@@ -59,7 +59,13 @@ def parse():
     ap.add_argument("--workload", default="wsi", choices=["wsi", "cohort"],
                     help="wsi: BASELINE configs[1] (headline, weak scaling); cohort: configs[2], --slides x --tiles sharded by "
                          "whole slides over the ranks (strong scaling), slide-level thresholding through apply_sharded")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (per-tile mean / std, apply "
+                         "results, kept-slide table) as DIR/<name>.npy, to compare two builds output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs needs --impl native")
+    return args
 
 
 def measured_peaks():
@@ -183,6 +189,38 @@ def run_reference_arm(args, rank, world):
 # --------------------------------------------------------------------------------------------------
 # native arm
 # --------------------------------------------------------------------------------------------------
+DUMP_BYTES = 60_000_000          # array payload of --dump-outputs: under 64 MB with the .npy headers
+
+
+def dump_outputs(out_dir, rank, world, mean, std, results, s_df):
+    """--dump-outputs: the arrays a caller of one step receives, as float32 / float64 .npy files.  Rank 0 writes the
+    apply results that are defined (apply returns None, or NaN for an empty confusion cell, where a result has no value:
+    on a single slide, for one, there is no slide-level ROC) and the kept-slide table (identical on every rank); each
+    rank writes its own per-tile mean / std, suffixed `_rank<r>` when there are several.  Everything stays within
+    DUMP_BYTES: past that the tile arrays are a fixed seeded sample of rows, whose indices go to tile_sample_index."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {}
+    if rank == 0:
+        for k, v in results.items():
+            if v is not None and np.isfinite(v):
+                arrays[f"apply_{k}"] = np.float64(v)
+        if s_df is not None:
+            for c in s_df.columns:
+                if s_df[c].dtype.kind in "biuf":
+                    arrays[f"slide_{c}"] = s_df[c].to_numpy(np.float64)
+    budget = (DUMP_BYTES - sum(a.nbytes for a in arrays.values())) // world
+    sfx = "" if world == 1 else f"_rank{rank}"
+    rows = np.arange(len(mean))
+    if mean.nbytes + std.nbytes > budget:
+        k = budget // (mean[:1].nbytes + std[:1].nbytes + 8)
+        rows = np.sort(np.random.default_rng(0).choice(len(mean), k, replace=False))
+        arrays["tile_sample_index" + sfx] = rows.astype(np.float64)
+    arrays["tile_mean" + sfx] = mean[rows]
+    arrays["tile_std" + sfx] = std[rows]
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def synth_tiles_device(n, device, seed):
     """uint8 NHWC tiles generated on the device: per-tile colour bias + gaussian texture"""
     import torch
@@ -241,7 +279,7 @@ def run_native_arm(args, rank, world, local_rank):
         with torch.cuda.stream(ext_stream):
             e0.record()
         for s in range(steps):
-            one_step(tiles, first_step + s)
+            last = one_step(tiles, first_step + s)
         with torch.cuda.stream(ext_stream):
             e1.record()
         barrier()
@@ -251,7 +289,7 @@ def run_native_arm(args, rank, world, local_rank):
             t = torch.tensor([ms, wall * 1e3], dtype=torch.float64, device=device)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms, wall = float(t[0]), float(t[1]) / 1e3
-        return ms, wall
+        return ms, wall, last
 
     # ---- warm-up, then the timed region on HBM-resident tiles
     for s in range(args.warmup):
@@ -260,9 +298,11 @@ def run_native_arm(args, rank, world, local_rank):
     launches0 = ctx.launches
     if rank == 0:
         sampler.start()
-    ms, wall = timed(tiles_dev, args.steps, args.warmup)
+    ms, wall, last = timed(tiles_dev, args.steps, args.warmup)
     clocks = sampler.stop() if rank == 0 else None
     launches = ctx.launches - launches0
+    if args.dump_outputs:                                    # before the steps below overwrite mean / std
+        dump_outputs(args.dump_outputs, rank, world, mean, std, *last)
     total_tiles = n * args.steps * world
     value = total_tiles / (ms / 1e3)
 
@@ -280,16 +320,16 @@ def run_native_arm(args, rank, world, local_rank):
         torch.cuda.synchronize()
         host_np = host.numpy()
         one_step(host_np, 0)
-        ems, _ = timed(host_np, args.steps, 100)
+        ems, _, _ = timed(host_np, args.steps, 100)
         h2d = n * TILE_BYTES + n * (4 + 4 + 1 + 4)            # tiles + (y_pred, uncertainty, y_true, codes) table
         d2h = n * 2 * 4 * 2 + n * (8 + 1 + 1) + 64 * args.slides
         e2e = {"value": total_tiles / (ems / 1e3), "unit": "tiles/s", "h2d_bytes_per_step": h2d,
                "d2h_bytes_per_step": d2h, "ms_per_step": ems / args.steps, "host_memory": "pinned"}
-        # what a NumPy / DataFrame caller passes is PAGEABLE memory: two steps of the same call on a plain ndarray
+        # what a NumPy / DataFrame caller passes is PAGEABLE memory: the same call on a plain ndarray
         pageable = np.array(host_np, copy=True)
         one_step(pageable, 0)
-        pms, _ = timed(pageable, 2, 100)
-        e2e["pageable_value"] = n * 2 * world / (pms / 1e3)
+        pms, _, _ = timed(pageable, args.steps, 100)
+        e2e["pageable_value"] = n * args.steps * world / (pms / 1e3)
         del host, host_np, pageable
 
     if rank != 0:
@@ -408,6 +448,8 @@ def run_cohort_arm(args, rank, world, local_rank):
         ms, wall = float(t[0]), float(t[1]) / 1e3
     clocks = sampler.stop() if rank == 0 else None
     launches = ctx.launches - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, rank, world, mean, std, res, s_df)
     # sharded decisions == single-process apply on the concatenated table (bit for bit), checked on rank 0
     same = None
     if world > 1:

@@ -1,17 +1,18 @@
 """TEST INFRASTRUCTURE ONLY -- never imported by the product path (biscuit_b200/).
 
-Import shim that loads the UNMODIFIED reference package `/root/reference/biscuit`
-in this build container so its `threshold.apply / detect / from_cv` can be executed
-as the ground truth for the thresholding half of the hot path (SURVEY.md App. C).
+Import shim that loads the UNMODIFIED reference package `biscuit` from a checkout of the
+original project named by the environment variable BISCUIT_REFERENCE_ROOT, so its
+`threshold.apply / detect / from_cv` can be executed as the ground truth for the
+thresholding half of the hot path (SURVEY.md App. C).
 
 The reference imports matplotlib / seaborn / skmisc / slideflow at module import time
 (reference biscuit/__init__.py:1-2, threshold.py:2-10, utils.py:6-9); none of those is
 installed here and none is on the arithmetic path, so they are stubbed in
 ``sys.modules``.  sklearn / pandas / numpy / scipy are the REAL installed packages.
 
-`/root/reference` does not exist on the GPU box: only `oracle/make_golden.py` (run here,
-output committed under tests/golden/) and the CPU-side oracle-pinning tests (skipped
-when the reference is absent) may call :func:`load_reference`.
+The reference is not part of this repository: only the `oracle/make_golden*.py` scripts
+(output committed under tests/golden/) and the CPU-side live-reference tests (skipped
+unless BISCUIT_REFERENCE_ROOT is set) may call :func:`load_reference`.
 """
 import importlib
 import logging
@@ -19,11 +20,11 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = os.environ.get("BISCUIT_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("BISCUIT_REFERENCE_ROOT", "")
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "biscuit", "threshold.py"))
+    return bool(REFERENCE_ROOT) and os.path.isfile(os.path.join(REFERENCE_ROOT, "biscuit", "threshold.py"))
 
 
 def _stub(name, **attrs):
@@ -38,7 +39,8 @@ def load_reference():
     if "biscuit" in sys.modules and getattr(sys.modules["biscuit"], "_is_reference", False):
         return sys.modules["biscuit"]
     if not reference_available():
-        raise RuntimeError(f"reference not found under {REFERENCE_ROOT}")
+        raise RuntimeError(f"reference not found: set BISCUIT_REFERENCE_ROOT to a checkout of the original biscuit "
+                           f"project (now {REFERENCE_ROOT!r})")
 
     log = logging.getLogger("slideflow_stub")
     log.addHandler(logging.NullHandler())

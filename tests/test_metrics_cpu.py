@@ -34,7 +34,7 @@ def test_oracle_matches_golden(name):
     check(res, dl, GOLD["cases"][name], name)
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not reference_available(), reason="needs a checkout of the original biscuit project in BISCUIT_REFERENCE_ROOT")
 def test_live_reference_matches_oracle():
     R = load_reference()
     rng = np.random.default_rng(77)

@@ -186,7 +186,7 @@ def test_device_resident_tiles(iface, tiles):
     assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1])
 
 
-def test_simt_debug_path_agrees():
+def test_simt_debug_path_agrees(tmp_path):
     """BQ_GEMM=simt (plain CUDA-core GEMM, debug only) vs the default tcgen05 path: same bf16 inputs, fp32
     accumulation in a different order"""
     code = (
@@ -199,7 +199,7 @@ def test_simt_debug_path_agrees():
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     outs = []
     for mode in ("simt", "tcgen05"):
-        path = f"/tmp/bq_{mode}.npy"
+        path = str(tmp_path / f"bq_{mode}.npy")
         env = dict(os.environ, BQ_GEMM=mode, PYTHONPATH=root)
         subprocess.run([sys.executable, "-c", code, path], check=True, env=env, cwd=root, timeout=600)
         outs.append(np.load(path))
@@ -367,7 +367,7 @@ def test_config1_end_to_end_512_tiles_4_slides(weights, bench_iface):
         assert len(common) == int(far.sum()), (list(s1["slide"]), list(s2["slide"]))
 
 
-def test_fused_middle_flow_agrees_with_separate_kernels():
+def test_fused_middle_flow_agrees_with_separate_kernels(tmp_path):
     """Default: the 728-wide middle flow runs in `sepconv_mid_kernel` (depthwise produced on-chip into the N-side
     operand of a transposed cta_group::2 GEMM, zero-padded flattened layout).  BQ_SEPMID=off: stand-alone depthwise
     kernel + pointwise GEMM.  Same bf16 rounding points and the same fp32 depthwise tap order; only the tensor-core
@@ -385,7 +385,7 @@ def test_fused_middle_flow_agrees_with_separate_kernels():
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     outs = []
     for mode in ("off", "on"):
-        path = f"/tmp/bq_sepmid_{mode}.npy"
+        path = str(tmp_path / f"bq_sepmid_{mode}.npy")
         env = dict(os.environ, BQ_SEPMID=mode, PYTHONPATH=root)
         subprocess.run([sys.executable, "-c", code, path], check=True, env=env, cwd=root, timeout=600)
         outs.append(np.load(path))

@@ -26,7 +26,7 @@ def test_oracle_matches_golden(name, tmp_path):
     assert_matches_golden(df, th, case, name)
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not reference_available(), reason="needs a checkout of the original biscuit project in BISCUIT_REFERENCE_ROOT")
 def test_live_reference_matches_oracle(tmp_path):
     load_reference()
     import slideflow as sf

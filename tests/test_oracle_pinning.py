@@ -1,6 +1,6 @@
 """CPU tier: pin the oracle (oracle/threshold_oracle.py) against
   (1) the committed outputs of the unmodified reference (tests/golden/threshold_golden.json),
-  (2) the live reference through oracle/ref_shim.py when /root/reference exists (build container),
+  (2) the live reference through oracle/ref_shim.py when BISCUIT_REFERENCE_ROOT names a checkout of it,
   (3) the installed sklearn / pandas / numpy for the library-free tier the kernels implement.
 """
 import warnings
@@ -65,7 +65,7 @@ def test_oracle_from_cv_matches_golden():
     assert_same_results(r2, {k: dec(v) for k, v in g["nested_second"].items()})
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference tree not present on this box")
+@pytest.mark.skipif(not reference_available(), reason="needs a checkout of the original biscuit project in BISCUIT_REFERENCE_ROOT")
 def test_oracle_matches_live_reference():
     R = load_reference().threshold
     for seed in range(16):
@@ -92,7 +92,7 @@ def test_oracle_matches_live_reference():
                 assert_same_df(a, b, f"apply tile df seed {seed}")
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference tree not present on this box")
+@pytest.mark.skipif(not reference_available(), reason="needs a checkout of the original biscuit project in BISCUIT_REFERENCE_ROOT")
 def test_reference_error_behaviour_matches_oracle():
     R = load_reference()
     df = synth.tile_table(8, 20, seed=3)
