@@ -1,11 +1,14 @@
-"""Multi-GPU sharding of the hot path: one process per GPU, tiles sharded by WHOLE slides, and a single
-all-gather of the small per-slide aggregates (SURVEY.md 8e).
+"""Multi-GPU sharding of the hot path: one process per GPU, tiles sharded by WHOLE slides, and all-gathers
+of small per-rank messages (SURVEY.md 8e).
 
 Why slide-aligned: the reference's slide means are row-order Kahan sums in the column dtype
 (pandas `group_mean`, reference threshold.py:191-192); summing per-GPU partials would change the
 rounding and can flip a threshold decision, so a slide is never split across ranks and every slide's
-reduction stays local and bit-exact.  The only exchange step is `all_gather_groups`: <= 40 B per slide
-over NCCL/NVLink (gloo in the CPU tests) -- latency-, not bandwidth-bound.
+reduction stays local and bit-exact.  What crosses ranks (`threshold.ShardedTable`): the validation counts
+and row counts (`all_gather_meta`), the per-slide aggregates and slide names (`all_gather_groups`: 52 B per
+slide plus its name) and, only where a tile-level ROC is detected over the whole cohort, the per-tile
+`(pred, unc, label)` triples (`pack_tiles`) -- over NCCL/NVLink (gloo in the CPU tests), latency-, not
+bandwidth-bound for the group level.
 
 `torch.distributed` is plumbing only; the arithmetic stays in libbiscuit_b200.so.
 """
@@ -49,31 +52,6 @@ def pack_groups(code_offset, counts, first_rows, row_offset, y_pred, uncertainty
     msg[:, 4] = uncertainty
     msg[:, 5] = y_true_mean
     return msg
-
-
-def all_gather_groups(msg: np.ndarray, group=None, device=None):
-    """All-gather variable-length [L_r, 6] float64 blocks from every rank -> [sum L_r, 6] in rank
-    order (== table order, because shards are contiguous).  Works on NCCL (device tensors) and gloo."""
-    import torch
-    import torch.distributed as dist
-    if not dist.is_available() or not dist.is_initialized() or dist.get_world_size(group) == 1:
-        return msg
-    world = dist.get_world_size(group)
-    backend = dist.get_backend(group)
-    dev = torch.device("cpu") if backend == "gloo" else torch.device(device if device is not None else "cuda")
-    n_local = torch.tensor([msg.shape[0]], dtype=torch.int64, device=dev)
-    sizes = [torch.zeros(1, dtype=torch.int64, device=dev) for _ in range(world)]
-    dist.all_gather(sizes, n_local, group=group)
-    sizes = [int(s.item()) for s in sizes]
-    width = msg.shape[1]
-    pad = max(sizes) if sizes else 0
-    buf = torch.zeros((pad, width), dtype=torch.float64, device=dev)
-    if msg.shape[0]:
-        buf[: msg.shape[0]] = torch.from_numpy(np.ascontiguousarray(msg)).to(dev)
-    out = [torch.empty_like(buf) for _ in range(world)]
-    dist.all_gather(out, buf, group=group)
-    parts = [o[:s].cpu().numpy() for o, s in zip(out, sizes)]
-    return np.concatenate(parts, axis=0) if parts else msg
 
 
 # ----------------------------------------------------------------------------------------------------------------
@@ -215,3 +193,30 @@ def unpack_groups(msg: np.ndarray, dtype):
     return {"code": m[:, 0].astype(np.int64), "count": m[:, 1].astype(np.int64),
             "y_pred": m[:, 3].astype(dtype), "uncertainty": m[:, 4].astype(dtype),
             "y_true": m[:, 5].astype(np.uint8)}
+
+
+def all_gather_groups(names, groups, n_rows, n_keys, dtype, group=None, device=None):
+    """The exchange of the group level: every rank's per-group aggregates and group names -> the cohort's.
+
+    names: this rank's group names in code order; groups: its `(y_pred, uncertainty, y_true_mean, count, first_row)`
+    arrays, one entry per name (`first_row` counts from the start of the shard, -1 where no tile survived the filter);
+    n_rows: the shard's row count; n_keys: its key count before the filter.  One meta all-gather (the sizes) and ONE
+    payload all-gather (the aggregate records and the names, as bytes).
+    -> (the surviving groups as `unpack_groups` returns them in `dtype`, every rank's names in rank order, the cohort's
+    key count).  Every rank must call it, with an empty shard too (no names, empty arrays, n_rows 0)."""
+    y_pred, uncertainty, y_true_mean, counts, first_rows = groups
+    name_buf, name_len = pack_names(names)
+    meta = all_gather_meta([n_rows, len(names), n_keys, name_buf.shape[0]], group=group, device=device)
+    _, _, rank = _dist_state(group)
+    msg = pack_groups(int(meta[:rank, 1].sum()), counts, first_rows, int(meta[:rank, 0].sum()),
+                      y_pred, uncertainty, y_true_mean)
+    payload = np.concatenate([msg.view(np.uint8).reshape(-1), name_len.view(np.uint8), name_buf])
+    rec = msg.itemsize * len(GROUP_FIELDS)                  # bytes of one group's aggregates
+    nrec = rec + name_len.itemsize                          # ... and its name length
+    parts = all_gather_bytes(payload, [int(L) * nrec + int(nb) for _, L, _, nb in meta], group=group, device=device)
+    msgs, all_names = [], []
+    for (_, L, _, nb), part in zip(meta, parts):
+        L, nb = int(L), int(nb)
+        msgs.append(part[:L * rec].copy().view(np.float64).reshape(L, len(GROUP_FIELDS)))
+        all_names += unpack_names(part[L * nrec:L * nrec + nb], part[L * rec:L * nrec].copy().view(np.int32))
+    return unpack_groups(np.concatenate(msgs, axis=0), dtype), all_names, int(meta[:, 2].sum())

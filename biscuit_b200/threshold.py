@@ -30,7 +30,7 @@ import warnings
 import numpy as np
 import pandas as pd
 
-from . import _ffi, errors
+from . import _ffi, dist as bdist, errors
 
 log = logging.getLogger("biscuit_b200")
 
@@ -71,10 +71,6 @@ def _label_col(a: np.ndarray, what="y_true") -> np.ndarray:
     if not np.array_equal(b, a):
         raise ValueError(f"{what}: labels must be 0/1 (continuous / multiclass format is not supported)")
     return np.ascontiguousarray(b)
-
-
-def _roc_struct():
-    return _ffi.RocResult()
 
 
 class _DeviceTable:
@@ -134,7 +130,7 @@ class _DeviceTable:
         return err, cor, ybin
 
     def tile_roc(self, score_sel, label_sel):
-        r = _roc_struct()
+        r = _ffi.RocResult()
         _ffi.check(self.ctx.handle, self.lib.bq_tile_roc(self.h, score_sel, label_sel, C.byref(r)),
                    "bq_tile_roc")
         return r
@@ -168,7 +164,7 @@ def _roc(ctx, score, label, include=None):
     score = _float_col(np.asarray(score))
     label = np.ascontiguousarray(label, dtype=np.uint8)
     inc = None if include is None else np.ascontiguousarray(include, dtype=np.uint8)
-    r = _roc_struct()
+    r = _ffi.RocResult()
     code = _ffi.BQ_F32 if score.dtype == np.float32 else _ffi.BQ_F64
     _ffi.check(ctx.handle,
                ctx.lib.bq_roc(ctx.handle, _ffi.ptr(score), code, _ffi.ptr(label), _ffi.ptr(inc),
@@ -176,13 +172,29 @@ def _roc(ctx, score, label, include=None):
     return r
 
 
+_EMPTY_INPUT = "Found array with 0 sample(s) while a minimum of 1 is required."   # sklearn's check_array
+
+
 def _youden_or_raise(r):
     """The reference's `max(zip(tpr,fpr))` / `.index()` idiom raises ValueError for single-class
     labels (SURVEY App. A.1); empty input makes sklearn raise ValueError too."""
     if r.status != 0:
-        raise ValueError("(nan, nan) is not in list" if r.status == 1
-                         else "Found array with 0 sample(s) while a minimum of 1 is required.")
+        raise ValueError("(nan, nan) is not in list" if r.status == 1 else _EMPTY_INPUT)
     return np.float64(r.threshold)
+
+
+def _raise_invalid(n_rows, flags):
+    """Raise what the reference raises for a tile table of `n_rows` rows with these `bq_table_validate` counts:
+    the NaN check of threshold.py:141, then sklearn's input checks in the first roc_curve."""
+    n_nan, n_nonfinite, _, n_badlabel = flags
+    if n_nan:
+        raise errors.PredsContainNaNError
+    if n_nonfinite:
+        raise ValueError("Input contains infinity or a value too large for dtype.")
+    if n_badlabel:
+        raise ValueError("multiclass format is not supported")
+    if n_rows == 0:
+        raise ValueError(_EMPTY_INPUT)
 
 
 def _check_columns(df):
@@ -192,9 +204,9 @@ def _check_columns(df):
                          f"Got: {', '.join(map(str, df.columns))}")
 
 
-def _open_table(df, ctx=None) -> _DeviceTable:
-    unc = df["uncertainty"].to_numpy() if "uncertainty" in df.columns else np.zeros(len(df), df["y_pred"].to_numpy().dtype)
-    return _DeviceTable(df["y_pred"].to_numpy(), unc, df["y_true"].to_numpy(), ctx=ctx)
+def _factorize(keys: pd.Series):
+    codes, uniques = pd.factorize(keys, use_na_sentinel=True)   # first-appearance order, NaN -> -1
+    return codes.astype(np.int32, copy=False), uniques
 
 
 class ResidentTable:
@@ -210,15 +222,27 @@ class ResidentTable:
 
     A later call with another tile-UQ threshold only re-runs the filter + reference-order slide reduction and the
     slide-level stage.  `apply_resident` / `detect_resident` are the entry points; `apply` / `detect` are the same code on
-    a table that lives for one call.  The DataFrame is mutated exactly as the reference mutates it."""
+    a table that lives for one call, and `apply_sharded` / `detect_sharded` on a :class:`ShardedTable`.  The DataFrame
+    is mutated exactly as the reference mutates it.
 
-    def __init__(self, df, ctx=None):
-        _check_columns(df)
+    `tile_only=True` opens a table for the tile stage alone, which needs no `uncertainty` column
+    (`process_tile_predictions`)."""
+
+    def __init__(self, df, ctx=None, tile_only=False):
+        if not tile_only:
+            _check_columns(df)
         self.df = df
-        self.tab = _open_table(df, ctx=ctx)
-        self.ctx = self.tab.ctx
-        self._tile_done = {}
+        self.ctx = ctx or _ffi.default_context()
+        self.tab = self._open()
+        self.dtype = None if self.tab is None else self.tab.dtype
+        self.n_unc_nonfinite = 0      # sklearn's finiteness check fires only where the uncertainty feeds a ROC
+        self._tile_key = self.pred_thresh = None
         self._keys = {}
+
+    def _open(self):
+        df = self.df
+        unc = df["uncertainty"].to_numpy() if "uncertainty" in df.columns else np.zeros(len(df), df["y_pred"].to_numpy().dtype)
+        return _DeviceTable(df["y_pred"].to_numpy(), unc, df["y_true"].to_numpy(), ctx=self.ctx)
 
     def close(self):
         if self.tab is not None:
@@ -231,83 +255,193 @@ class ResidentTable:
     def __exit__(self, *exc):
         self.close()
 
-    @property
-    def dtype(self):
-        return self.tab.dtype
-
+    # ------------------------------------------------------------------------------------
+    # tile level
+    # ------------------------------------------------------------------------------------
     def tile_stage(self, tile_pred, patients):
         """-> the tile prediction threshold in force (detected once per table when 'detect')."""
         key = "detect" if _is_detect(tile_pred) else (type(tile_pred).__name__, float(tile_pred))
-        if key not in self._tile_done:
+        if key != self._tile_key:
             # a different numeric threshold rewrites the derived columns; the incorrect flags on the device follow
-            self._tile_done = {key: _tile_stage(self.tab, self.df, tile_pred, patients)}
+            self.pred_thresh = self._tile_stage(tile_pred, patients)
+            self._tile_key = key
         elif patients is not None and "patient" not in self.df.columns:
-            self.df["patient"] = _map_slides(self.tab, self.df, patients)
-        return self._tile_done[key]
+            self.df["patient"] = self._map_slides(patients)
+        return self.pred_thresh
 
+    def _tile_stage(self, pred_thresh, patients):
+        """threshold.py:140-177; mutates df; returns pred_thresh used."""
+        n_rows, flags = self._validate()
+        self.n_unc_nonfinite = flags[2]
+        _raise_invalid(n_rows, flags)                                     # :141-142
+        if _is_detect(pred_thresh):                                       # :145-159
+            r = self._roc_table().tile_roc(_ffi.SCORE_Y_PRED, _ffi.LABEL_Y_TRUE)
+            if r.status == 1:
+                log.debug("Unable to calculate tile prediction threshold; using 0.5")
+                pred_thresh = 0.5                                         # :153-155
+            else:
+                pred_thresh = _youden_or_raise(r)
+            log.debug(f"Auto-detected tile prediction threshold: {pred_thresh:.4f}")
+        else:
+            log.debug(f"Using tile prediction threshold: {pred_thresh:.4f}")  # :161
+        if self.tab is None:                                              # an empty shard is left as it is
+            return pred_thresh
+        df = self.df
+        if patients is not None:                                          # :163-166
+            df["patient"] = self._map_slides(patients)
+        else:
+            log.debug("Patients not provided; assuming 1:1 slide:patient mapping")
+        err, cor, ybin = self.tab.tile_process(_cmp_scalar(pred_thresh, df["y_pred"].to_numpy().dtype))
+        # dtypes as pandas gives them: |int64 - float| -> float64 (narrow ints keep the float width)
+        err_dtype = np.result_type(df["y_true"].to_numpy().dtype, df["y_pred"].to_numpy().dtype)
+        df["error"] = err if err_dtype == np.float64 else err.astype(err_dtype)   # :170
+        df["correct"] = cor.view(np.bool_)                                # :171-174
+        df["incorrect"] = (cor ^ 1).astype(int)                           # :175
+        df["y_pred_bin"] = ybin.astype(int)                               # :176
+        return pred_thresh
+
+    def _validate(self):
+        """-> (rows, bq_table_validate counts) of the table whose errors the reference would raise"""
+        return self.tab.n, self.tab.validate()
+
+    def _roc_table(self):
+        """the device table the tile-level ROCs run on"""
+        return self.tab
+
+    def tile_uq_threshold(self):
+        """threshold.py:416-426: Youden's J on the tile ROC of `incorrect ~ uncertainty` (after the tile stage)."""
+        if self.n_unc_nonfinite:                                          # roc_curve -> assert_all_finite (uncaught at :419)
+            raise ValueError("Input contains NaN or infinity.")
+        return _youden_or_raise(self._roc_table().tile_roc(_ffi.SCORE_UNCERTAINTY, _ffi.LABEL_INCORRECT))
+
+    def _map_slides(self, patients):
+        """``df['slide'].map(patients)`` computed on the UNIQUE slide names and expanded through the factorisation
+        codes (same `Series.map` on the same values, so the same dtype inference and NaN for unknown slides), instead
+        of a hash lookup per tile row; the factorisation is the one the slide-level grouping uses."""
+        df = self.df
+        codes, uniques = self.keys("slide")
+        if len(codes) == 0 or codes.min() < 0:                            # NaN slide names: leave it to pandas
+            return df["slide"].map(patients)
+        mapped = pd.Series(uniques, dtype=df["slide"].dtype).map(patients)
+        return pd.Series(mapped.array.take(codes), index=df.index)
+
+    # ------------------------------------------------------------------------------------
+    # group (slide / patient) level
+    # ------------------------------------------------------------------------------------
     def keys(self, level):
         """(codes, uniques) of df[level] in first-appearance order, factorised once per level"""
         if level not in self._keys:
-            fact = getattr(self.tab, "slide_factorized", None) if level == "slide" else None
-            self._keys[level] = fact if fact is not None else _factorize(self.df[level])
+            self._keys[level] = _factorize(self.df[level])
         return self._keys[level]
 
-    def groups(self, level, tile_uq_eff, pred_thresh):
-        return _group_stage(self.tab, self.df, level, tile_uq_eff, pred_thresh, factorized=self.keys(level))
+    def _reduce(self, level, tile_uq_eff):
+        """threshold.py:190-192 with the tile-UQ filter: -> (keys, number of keys before the filter with NaN counted as
+        one, per-key (y_pred, uncertainty, y_true) means, surviving tile counts and first surviving rows)"""
+        codes, uniques = self.keys(level)
+        self.tab.set_groups(codes, len(uniques))
+        self.tab.set_filter(tile_uq_eff)
+        return uniques, len(uniques) + int((codes < 0).any()), self.tab.group_reduce()
 
+    def _groups(self, level, tile_uq_eff):
+        """-> (keys, y_pred, uncertainty, y_true truncated to uint8, keys before the filter) of the groups with a
+        surviving tile, in first-appearance order after the filter"""
+        uniques, n_keys, (gp, gu, gt, cnt, first) = self._reduce(level, tile_uq_eff)
+        alive = np.flatnonzero(cnt > 0)
+        order = alive[np.argsort(first[alive], kind="stable")]
+        return [uniques[i] for i in order], gp[order], gu[order], gt[order].astype(np.uint8), n_keys
 
-# ----------------------------------------------------------------------------------------
-# tile level
-# ----------------------------------------------------------------------------------------
-
-def _tile_stage(tab: _DeviceTable, df, pred_thresh, patients):
-    """threshold.py:140-177 on an open device table; mutates df; returns pred_thresh used."""
-    n_nan, n_nonfinite, n_unc_nonfinite, n_badlabel = tab.validate()
-    tab.n_unc_nonfinite = int(n_unc_nonfinite)      # sklearn's check fires only where the uncertainty feeds a ROC
-    if n_nan:                                                         # :141-142
-        raise errors.PredsContainNaNError
-    if n_nonfinite:
-        raise ValueError("Input contains infinity or a value too large for dtype.")
-    if n_badlabel:
-        raise ValueError("multiclass format is not supported")
-    if _is_detect(pred_thresh):                                       # :145-159
-        r = tab.tile_roc(_ffi.SCORE_Y_PRED, _ffi.LABEL_Y_TRUE)
-        if r.status == 0:
+    def group_table(self, level, tile_uq_eff, pred_thresh):
+        """threshold.py:188-245 with the tile-UQ filter (threshold.py:298/412/426) applied on the device: the per-group
+        means (:190-200), optional Youden detection on the group ROC, then the group DataFrame.
+        -> (group DataFrame, pred_thresh used, number of keys before the filter)"""
+        levels, yp, u, yt, n_keys = self._groups(level, tile_uq_eff)
+        if not len(yt):                                                   # :205-206
+            raise errors.ROCFailedError("Unable to generate ROC; preds are empty.")
+        if _is_detect(pred_thresh):                                       # :217-223
+            r = _roc(self.ctx, yp, yt)
+            if r.status != 0:
+                raise errors.ROCFailedError(f"Unable to generate {level}-level ROC")
             pred_thresh = np.float64(r.threshold)
-        elif r.status == 1:
-            log.debug("Unable to calculate tile prediction threshold; using 0.5")
-            pred_thresh = 0.5                                         # :153-155
+            log.debug(f"Using detected prediction threshold: {pred_thresh:.4f}")
         else:
-            raise ValueError("Found array with 0 sample(s) while a minimum of 1 is required.")
-        log.debug(f"Auto-detected tile prediction threshold: {pred_thresh:.4f}")
-    else:
-        if tab.n == 0:
-            raise ValueError("Found array with 0 sample(s) while a minimum of 1 is required.")
-        log.debug(f"Using tile prediction threshold: {pred_thresh:.4f}")  # :161
-    if patients is not None:                                          # :163-166
-        df["patient"] = _map_slides(tab, df, patients)
-    else:
-        log.debug("Patients not provided; assuming 1:1 slide:patient mapping")
-    err, cor, ybin = tab.tile_process(_cmp_scalar(pred_thresh, df["y_pred"].to_numpy().dtype))
-    # dtypes as pandas gives them: |int64 - float| -> float64 (narrow ints keep the float width)
-    err_dtype = np.result_type(df["y_true"].to_numpy().dtype, df["y_pred"].to_numpy().dtype)
-    df["error"] = err if err_dtype == np.float64 else err.astype(err_dtype)   # :170
-    df["correct"] = cor.view(np.bool_)                                # :171-174
-    df["incorrect"] = (cor ^ 1).astype(int)                           # :175
-    df["y_pred_bin"] = ybin.astype(int)                               # :176
-    return pred_thresh
+            log.debug(f"Using {level} prediction threshold: {pred_thresh:.4f}")   # :225
+        cols = _group_columns(self.ctx, yp, u, yt, pred_thresh, pred_thresh, _ffi.KEEP_ALL, 0.0)
+        l_df = pd.DataFrame({                                             # :235-244
+            level: pd.Series(levels),
+            "error": pd.Series(cols["error"]),
+            "uncertainty": pd.Series(u),
+            "correct": cols["correct"].view(np.bool_),
+            "incorrect": pd.Series(cols["incorrect"]).astype(int),
+            "y_true": pd.Series(yt),
+            "y_pred": pd.Series(yp),
+            "y_pred_bin": pd.Series(cols["y_pred_bin"].view(np.bool_)).astype(int),
+        })
+        return l_df, pred_thresh, n_keys
 
 
-def _map_slides(tab, df, patients):
-    """``df['slide'].map(patients)`` computed on the UNIQUE slide names and expanded through the factorisation
-    codes (same `Series.map` on the same values, so the same dtype inference and NaN for unknown slides), instead
-    of a hash lookup per tile row; the factorisation is kept on the table for the slide-level grouping."""
-    codes, uniques = _factorize(df["slide"])
-    tab.slide_factorized = (codes, uniques)
-    if len(codes) == 0 or codes.min() < 0:                            # NaN slide names: leave it to pandas
-        return df["slide"].map(patients)
-    mapped = pd.Series(uniques, dtype=df["slide"].dtype).map(patients)
-    return pd.Series(mapped.array.take(codes), index=df.index)
+class ShardedTable(ResidentTable):
+    """This rank's shard of a cohort sharded over ranks (SURVEY.md 8e): one process per GPU, torch.distributed
+    initialised or a `dist.NativeComm` passed as `group`.  Every rank holds a contiguous, slide-aligned shard of the tile
+    table (see `dist.shard_bounds`; a slide / patient must not straddle ranks; a shard may be empty) and runs the same
+    calls in the same order, so every rank makes the same collectives:
+
+      * validation counts are summed over the ranks, so every rank raises what the concatenated table raises (a rank
+        that raised alone would leave the others blocked in a collective);
+      * the tile-level ROCs run over ALL tiles of the cohort: the per-tile `(pred, unc, label)` triples are all-gathered
+        into a second `bq_table` on every GPU (deterministic kernels: replicated, identical thresholds);
+      * tile processing and the reference-order per-group reduction stay local and bit-exact; the per-group aggregates
+        and names are all-gathered (`dist.all_gather_groups`) and the group level runs replicated.
+
+    An empty shard opens no `bq_table` and contributes zero groups."""
+
+    def __init__(self, df, group=None):
+        self.group, self.cohort = group, None
+        self.rows, self.cohort_dtype = [], None        # every rank's row count and the cohort dtype, from the validation
+        super().__init__(df)
+        self.device = f"cuda:{self.ctx.device}"
+
+    def _open(self):
+        return super()._open() if len(self.df) else None
+
+    def close(self):
+        super().close()
+        if self.cohort is not None:
+            self.cohort.close()
+            self.cohort = None
+
+    def _validate(self):
+        n_rows, flags = super()._validate() if self.tab is not None else (0, (0, 0, 0, 0))
+        dcode = -1 if self.dtype is None else int(self.dtype == np.float64)
+        meta = bdist.all_gather_meta([n_rows, dcode, *flags], group=self.group, device=self.device)
+        self.rows = [int(n) for n in meta[:, 0]]
+        self.cohort_dtype = np.dtype(np.float64 if (meta[:, 1] == 1).any() else np.float32)
+        return sum(self.rows), tuple(int(f) for f in meta[:, 2:].sum(axis=0))
+
+    def _roc_table(self):
+        if self.cohort is None:
+            dt, df = self.cohort_dtype, self.df
+            buf = bdist.pack_tiles(_float_col(df["y_pred"].to_numpy()).astype(dt, copy=False),
+                                   _float_col(df["uncertainty"].to_numpy()).astype(dt, copy=False),
+                                   _label_col(df["y_true"].to_numpy()))
+            parts = bdist.all_gather_bytes(buf, [n * (2 * dt.itemsize + 1) for n in self.rows],
+                                           group=self.group, device=self.device)
+            cols = [bdist.unpack_tiles(part, n, dt) for n, part in zip(self.rows, parts)]
+            self.cohort = _DeviceTable(*(np.concatenate(c) for c in zip(*cols)), ctx=self.ctx)
+        return self.cohort
+
+    def tile_uq_threshold(self):
+        cohort = self._roc_table()
+        cohort.tile_process(_cmp_scalar(self.pred_thresh, cohort.dtype), want_columns=False)   # its incorrect flags
+        return super().tile_uq_threshold()
+
+    def _groups(self, level, tile_uq_eff):
+        names, n_keys, local = [], 0, (np.zeros(0),) * 5
+        if self.tab is not None:
+            uniques, n_keys, local = self._reduce(level, tile_uq_eff)
+            names = [str(u) for u in uniques]
+        g, names, n_keys = bdist.all_gather_groups(names, local, len(self.df), n_keys, self.cohort_dtype,
+                                                   group=self.group, device=self.device)
+        return [names[c] for c in g["code"]], g["y_pred"], g["uncertainty"], g["y_true"], n_keys
 
 
 def process_tile_predictions(df, pred_thresh=0.5, patients=None):
@@ -315,60 +449,8 @@ def process_tile_predictions(df, pred_thresh=0.5, patients=None):
 
     Adds `error`, `correct`, `incorrect`, `y_pred_bin` (and `patient`) to `df` IN PLACE and returns
     ``(df, pred_thresh)``; ``pred_thresh='detect'`` picks Youden's J on the tile ROC."""
-    with _open_table(df) as tab:
-        pred_thresh = _tile_stage(tab, df, pred_thresh, patients)
-    return df, pred_thresh
-
-
-# ----------------------------------------------------------------------------------------
-# group (slide / patient) level
-# ----------------------------------------------------------------------------------------
-
-def _factorize(keys: pd.Series):
-    codes, uniques = pd.factorize(keys, use_na_sentinel=True)   # first-appearance order, NaN -> -1
-    return codes.astype(np.int32, copy=False), uniques
-
-
-def _group_stage(tab: _DeviceTable, df, level, tile_uq_eff, pred_thresh, factorized=None):
-    """threshold.py:188-245 with the tile-UQ filter (threshold.py:298/412/426) applied on the
-    device.  Returns (group DataFrame, pred_thresh used)."""
-    if factorized is None and level == "slide":
-        factorized = getattr(tab, "slide_factorized", None)          # already factorised for the patient mapping
-    codes, uniques = factorized if factorized is not None else _factorize(df[level])
-    tab.set_groups(codes, len(uniques))
-    tab.set_filter(tile_uq_eff)
-    gp, gu, gt, cnt, first = tab.group_reduce()
-    alive = np.flatnonzero(cnt > 0)
-    order = alive[np.argsort(first[alive], kind="stable")]           # first appearance after filter
-    levels = [uniques[i] for i in order]                              # :190
-    return _group_table(tab.ctx, level, levels, gp[order], gu[order], gt[order].astype(np.uint8), pred_thresh)
-
-
-def _group_table(ctx, level, levels, yp, u, yt, pred_thresh):
-    """threshold.py:197-245 on the per-group means (already in first-appearance order, `yt` truncated to uint8,
-    :197-200): optional Youden detection on the group ROC, then the group DataFrame."""
-    if not len(yt):                                                   # :205-206
-        raise errors.ROCFailedError("Unable to generate ROC; preds are empty.")
-    if _is_detect(pred_thresh):                                       # :217-223
-        r = _roc(ctx, yp, yt)
-        if r.status != 0:
-            raise errors.ROCFailedError(f"Unable to generate {level}-level ROC")
-        pred_thresh = np.float64(r.threshold)
-        log.debug(f"Using detected prediction threshold: {pred_thresh:.4f}")
-    else:
-        log.debug(f"Using {level} prediction threshold: {pred_thresh:.4f}")   # :225
-    cols = _group_columns(ctx, yp, u, yt, pred_thresh, pred_thresh, _ffi.KEEP_ALL, 0.0)
-    l_df = pd.DataFrame({                                             # :235-244
-        level: pd.Series(levels),
-        "error": pd.Series(cols["error"]),
-        "uncertainty": pd.Series(u),
-        "correct": cols["correct"].view(np.bool_),
-        "incorrect": pd.Series(cols["incorrect"]).astype(int),
-        "y_true": pd.Series(yt),
-        "y_pred": pd.Series(yp),
-        "y_pred_bin": pd.Series(cols["y_pred_bin"].view(np.bool_)).astype(int),
-    })
-    return l_df, pred_thresh
+    with ResidentTable(df, tile_only=True) as table:
+        return df, table.tile_stage(pred_thresh, patients)
 
 
 def _group_columns(ctx, yp, u, yt, pred_thresh, strict_thresh, keep_mode, slide_uq_eff):
@@ -399,8 +481,8 @@ def process_group_predictions(df, pred_thresh, level):
     if len(df) == 0:
         df[level]                                                     # KeyError parity
         raise errors.ROCFailedError("Unable to generate ROC; preds are empty.")
-    with _open_table(df) as tab:
-        return _group_stage(tab, df, level, None, pred_thresh)
+    with ResidentTable(df) as table:
+        return table.group_table(level, None, pred_thresh)[:2]
 
 
 def _auc_included(ctx, s_yp, s_yt, include=None):
@@ -410,6 +492,16 @@ def _auc_included(ctx, s_yp, s_yt, include=None):
         log.warning("Unable to calculate ROC")
         return np.nan
     return float(r.auc)
+
+
+def _apply_preamble(df, tile_uq, keep, patients, level):
+    """threshold.py:281-287, before the table is opened."""
+    assert keep in ("high_confidence", "low_confidence")             # :281
+    assert not (level == "patient" and patients is None)             # :282
+    log.debug(f"Applying tile UQ threshold of {tile_uq:.5f}")         # :284 (TypeError on None)
+    if patients:                                                      # :285-286
+        df["patient"] = df["slide"].map(patients)
+    df[level]                                                         # :287 KeyError parity
 
 
 def apply(df, tile_uq, slide_uq, tile_pred=0.5, slide_pred=0.5, plot=False,
@@ -432,12 +524,7 @@ def apply(df, tile_uq, slide_uq, tile_pred=0.5, slide_pred=0.5, plot=False,
         (original integer index labels).  ({...None}, None) if no group-level ROC is possible."""
     if plot:
         log.warning("plot=True ignored: plotting is outside the scope of biscuit_b200")
-    assert keep in ("high_confidence", "low_confidence")             # :281
-    assert not (level == "patient" and patients is None)             # :282
-    log.debug(f"Applying tile UQ threshold of {tile_uq:.5f}")         # :284 (TypeError on None)
-    if patients:                                                      # :285-286
-        df["patient"] = df["slide"].map(patients)
-    df[level]                                                         # :287 KeyError parity
+    _apply_preamble(df, tile_uq, keep, patients, level)
     with ResidentTable(df) as table:
         return apply_resident(table, tile_uq, slide_uq, tile_pred=tile_pred, slide_pred=slide_pred, keep=keep,
                               patients=patients, level=level)
@@ -454,11 +541,9 @@ def apply_resident(table: ResidentTable, tile_uq, slide_uq, tile_pred=0.5, slide
         df["patient"] = df["slide"].map(patients)
     df[level]
     table.tile_stage(tile_pred, patients)                             # :290-294
-    codes, uniques = table.keys(level)
-    n_before = len(uniques) + int((codes < 0).any())                  # :295 (NaN counts as a key)
     tile_uq_eff = _cmp_scalar(tile_uq, table.dtype) if tile_uq else None   # :297-298
     try:
-        s_df, _ = table.groups(level, tile_uq_eff, slide_pred)        # :305
+        s_df, _, n_before = table.group_table(level, tile_uq_eff, slide_pred)   # :295, :305
     except errors.ROCFailedError:
         log.error("Unable to process slide predictions")
         return {k: None for k in _RESULT_KEYS}, None                  # :310-317
@@ -489,208 +574,19 @@ def _apply_group_level(ctx, s_df, slide_uq, slide_pred, keep, level, n_before):
     return results, s_df
 
 
-# ----------------------------------------------------------------------------------------
-# cohort sharded over GPUs (SURVEY.md 8e): one process per GPU, slide-aligned shards
-# ----------------------------------------------------------------------------------------
-_ERR_NONE, _ERR_NAN, _ERR_NONFINITE, _ERR_LABEL, _ERR_EMPTY = 0, 1, 2, 3, 4
-
-
-def _raise_shard_error(code):
-    """the same exception on every rank (a rank that raised alone would leave the others blocked in a collective)"""
-    if code == _ERR_NAN:
-        raise errors.PredsContainNaNError
-    if code == _ERR_NONFINITE:
-        raise ValueError("Input contains infinity or a value too large for dtype.")
-    if code == _ERR_LABEL:
-        raise ValueError("multiclass format is not supported")
-    if code == _ERR_EMPTY:
-        raise ValueError("Found array with 0 sample(s) while a minimum of 1 is required.")
-
-
-def _shard_local(df, level, patients, tile_pred, tile_uq_eff_fn):
-    """Local half of a sharded call: validation, tile processing (mutates the shard like the reference mutates the
-    table) and the reference-order per-slide reduction of THIS rank's slides.  Never raises: the error code travels
-    with the size exchange so that every rank fails together.  An empty shard (more ranks than slides) contributes
-    zero groups."""
-    out = {"err": _ERR_NONE, "n_rows": len(df), "names": [], "n_keys": 0, "msg": np.zeros((0, 6), np.float64),
-           "dtype": np.dtype(df["y_pred"].to_numpy().dtype) if "y_pred" in df.columns and len(df) else None,
-           "ctx": _ffi.default_context()}
-    if len(df) == 0:
-        return out
-    with _open_table(df) as tab:
-        out["ctx"], out["dtype"] = tab.ctx, tab.dtype
-        try:
-            _tile_stage(tab, df, tile_pred, patients)
-        except errors.PredsContainNaNError:
-            out["err"] = _ERR_NAN
-            return out
-        except ValueError as e:
-            out["err"] = _ERR_LABEL if "multiclass" in str(e) else _ERR_NONFINITE
-            return out
-        codes, uniques = _factorize(df[level])
-        out["n_keys"] = len(uniques) + int((codes < 0).any())
-        out["names"] = [str(u) for u in uniques]
-        tab.set_groups(codes, len(uniques))
-        tab.set_filter(tile_uq_eff_fn(tab.dtype))
-        gp, gu, gt, cnt, first = tab.group_reduce()
-    out["local"] = (gp, gu, gt, cnt, first)
-    return out
-
-
-def _exchange_groups(loc, group):
-    """meta all-gather (sizes + error codes) and ONE payload all-gather (per-slide aggregates + slide names as utf-8
-    tensors): -> (groups dict in global first-appearance order, all names, keys before the tile filter, dtype)."""
-    from . import dist as bdist
-    name_buf, name_len = bdist.pack_names(loc["names"])
-    L = len(loc["names"])
-    dcode = -1 if loc["dtype"] is None else (0 if loc["dtype"] == np.float32 else 1)
-    device = f"cuda:{loc['ctx'].device}"
-    meta = bdist.all_gather_meta([loc["n_rows"], L, loc["n_keys"], loc["err"], name_buf.shape[0], dcode],
-                                 group=group, device=device)
-    errs = meta[:, 3]
-    if errs.any():
-        _raise_shard_error(int(errs[errs != 0][0]))
-    if int(meta[:, 0].sum()) == 0:
-        _raise_shard_error(_ERR_EMPTY)
-    _, _, rank = bdist._dist_state(group)
-    code_off, row_off = int(meta[:rank, 1].sum()), int(meta[:rank, 0].sum())
-    if L:
-        gp, gu, gt, cnt, first = loc["local"]
-        msg = bdist.pack_groups(code_off, cnt, first, row_off, gp, gu, gt)
-    else:
-        msg = np.zeros((0, 6), np.float64)
-    payload = np.concatenate([msg.view(np.uint8).reshape(-1), name_len.view(np.uint8).reshape(-1), name_buf])
-    sizes = [int(m[1]) * 52 + int(m[4]) for m in meta]              # 48 B of aggregates + 4 B name length per slide
-    parts = bdist.all_gather_bytes(payload, sizes, group=group, device=device)
-    msgs, names = [], []
-    for m, part in zip(meta, parts):
-        Lr, nb = int(m[1]), int(m[4])
-        msgs.append(part[: Lr * 48].copy().view(np.float64).reshape(Lr, 6))
-        lens = part[Lr * 48: Lr * 52].copy().view(np.int32)
-        names += bdist.unpack_names(part[Lr * 52: Lr * 52 + nb], lens)
-    dcodes = meta[:, 5][meta[:, 5] >= 0]
-    dtype = np.dtype(np.float64 if (dcodes == 1).any() else np.float32)
-    g = bdist.unpack_groups(np.concatenate(msgs, axis=0), dtype)
-    return g, names, int(meta[:, 2].sum()), dtype
-
-
 def apply_sharded(df, tile_uq, slide_uq, tile_pred=0.5, slide_pred=0.5, keep="high_confidence",
                   patients=None, level="slide", group=None):
-    """`apply` for a cohort sharded over ranks (one process per GPU, torch.distributed initialised).
-
-    Every rank passes ITS contiguous, slide-aligned shard of the tile table (see `dist.shard_bounds`;
-    a slide / patient must not straddle ranks; a shard may be empty).  Tile processing and the
-    reference-order slide reduction run locally on each GPU; the per-slide aggregates (48 B per slide)
-    and the slide names (utf-8 tensors, no pickling) are all-gathered ONCE after a small size / error-code
-    exchange, and the group-level thresholding runs replicated, so every rank returns the same
-    (results, s_df) `apply` would return on the concatenated table -- and every rank raises the same
-    exception when any shard fails validation.  Thresholds must be numeric: 'detect' is resolved on the
-    whole cohort by `detect_sharded`."""
-    assert keep in ("high_confidence", "low_confidence")
-    assert not (level == "patient" and patients is None)
+    """`apply` for a cohort sharded over ranks: every rank passes ITS shard of the tile table (see
+    :class:`ShardedTable`) and returns the same (results, s_df) `apply` would return on the concatenated table, or
+    raises the same exception.  Thresholds must be numeric: 'detect' is resolved on the whole cohort by
+    `detect_sharded`."""
     if _is_detect(tile_pred) or _is_detect(slide_pred):
         raise ValueError("apply_sharded needs numeric prediction thresholds (a per-shard 'detect' would differ "
                          "between ranks): use detect_sharded / from_cv_sharded first")
-    log.debug(f"Applying tile UQ threshold of {tile_uq:.5f}")
-    if patients:
-        df["patient"] = df["slide"].map(patients)
-    df[level]
-    _check_columns(df)
-    loc = _shard_local(df, level, patients, tile_pred, lambda dt: _cmp_scalar(tile_uq, dt) if tile_uq else None)
-    g, names, n_before, _ = _exchange_groups(loc, group)
-    levels = [names[c] for c in g["code"]]
-    try:
-        s_df, _ = _group_table(loc["ctx"], level, levels, g["y_pred"], g["uncertainty"], g["y_true"], slide_pred)
-    except errors.ROCFailedError:
-        log.error("Unable to process slide predictions")
-        return {k: None for k in _RESULT_KEYS}, None
-    return _apply_group_level(loc["ctx"], s_df, slide_uq, slide_pred, keep, level, n_before)
-
-
-def detect_sharded(df, tile_uq="detect", slide_uq="detect", tile_pred="detect", slide_pred="detect",
-                   patients=None, group=None):
-    """`detect` for a table sharded over ranks (reference threshold.py:364-475 on the concatenated table).
-
-    The tile-level ROCs (`y_true ~ y_pred`, `incorrect ~ uncertainty`) run over ALL tiles of the cohort, so the
-    per-tile `(pred, unc, label)` triples (9 B per tile for float32 tables) are all-gathered -- the one real
-    exchange step of the path (SURVEY.md 8e) -- and the ROC kernels run on the gathered table on every GPU
-    (deterministic integer/fp64 kernels: replicated, identical thresholds, no broadcast needed).  The slide
-    reduction stays local and bit-exact (slide-aligned shards), its aggregates are all-gathered as in
-    `apply_sharded`, and the slide-level detection runs replicated.  Returns what `detect` returns, on every rank."""
-    from . import dist as bdist
-    none4 = {k: None for k in _THRESH_KEYS}
-    _check_columns(df)
-    ctx = _ffi.default_context()
-    device = f"cuda:{ctx.device}"
-    n_local = len(df)
-    yp_l = _float_col(df["y_pred"].to_numpy()) if n_local else np.zeros(0, np.float32)
-    un_l = _float_col(df["uncertainty"].to_numpy()) if n_local else np.zeros(0, np.float32)
-    if yp_l.dtype != un_l.dtype:
-        yp_l, un_l = yp_l.astype(np.float64), un_l.astype(np.float64)
-    need_tiles = _is_detect(tile_pred) or _is_detect(tile_uq)
-    if need_tiles:
-        # ---- exchange 1: sizes + column dtype, then the tile triples
-        meta = bdist.all_gather_meta([n_local, -1 if not n_local else int(yp_l.dtype == np.float64)], group=group, device=device)
-        wide = bool((meta[:, 1] == 1).any())
-        dt = np.dtype(np.float64 if wide else np.float32)
-        buf = bdist.pack_tiles(yp_l.astype(dt, copy=False), un_l.astype(dt, copy=False),
-                               _label_col(df["y_true"].to_numpy()) if n_local else np.zeros(0, np.uint8))
-        parts = bdist.all_gather_bytes(buf, [int(m[0]) * (2 * dt.itemsize + 1) for m in meta], group=group, device=device)
-        cols = [bdist.unpack_tiles(part, int(m[0]), dt) for m, part in zip(meta, parts)]
-        yp_g, un_g, yt_g = (np.concatenate([c[i] for c in cols]) for i in range(3))
-        with _DeviceTable(yp_g, un_g, yt_g, ctx=ctx) as tab:
-            n_nan, n_nonfinite, n_unc_nonfinite, n_badlabel = tab.validate()
-            if n_nan:
-                log.error("Tile-level predictions contain NaNs; unable to process.")
-                return none4, None
-            if n_nonfinite:
-                raise ValueError("Input contains infinity or a value too large for dtype.")
-            if n_badlabel:
-                raise ValueError("multiclass format is not supported")
-            if _is_detect(tile_pred):
-                r = tab.tile_roc(_ffi.SCORE_Y_PRED, _ffi.LABEL_Y_TRUE)
-                if r.status == 0:
-                    tile_pred = np.float64(r.threshold)
-                elif r.status == 1:
-                    tile_pred = 0.5
-                else:
-                    raise ValueError("Found array with 0 sample(s) while a minimum of 1 is required.")
-            tab.tile_process(_cmp_scalar(tile_pred, tab.dtype))
-            if _is_detect(tile_uq):
-                if n_unc_nonfinite:
-                    raise ValueError("Input contains NaN or infinity.")
-                tile_uq = _youden_or_raise(tab.tile_roc(_ffi.SCORE_UNCERTAINTY, _ffi.LABEL_INCORRECT))
-    if isinstance(tile_uq, _FLOAT_TYPES):
-        def tile_uq_eff_fn(dtype, t=tile_uq):
-            return _cmp_scalar(t, dtype) if not isinstance(t, np.float64) or True else float(t)
-    else:
-        if not _is_detect(tile_uq):
-            log.debug("Not performing tile-level uncertainty thresholding.")
-        tile_uq = None
-
-        def tile_uq_eff_fn(dtype):
-            return None
-    # ---- local tile processing + slide reduction, exchange 2: per-slide aggregates
-    loc = _shard_local(df, "slide", patients, tile_pred, tile_uq_eff_fn)
-    try:
-        g, names, _, _ = _exchange_groups(loc, group)
-    except errors.PredsContainNaNError:
-        log.error("Tile-level predictions contain NaNs; unable to process.")
-        return none4, None
-    levels = [names[c] for c in g["code"]]
-    try:
-        s_df, slide_pred = _group_table(loc["ctx"], "slide", levels, g["y_pred"], g["uncertainty"], g["y_true"], slide_pred)
-    except errors.ROCFailedError:
-        log.error("Unable to process slide predictions")
-        return none4, None
-    slide_uq, auc = _detect_group_level(loc["ctx"], s_df, slide_uq, slide_pred)
-    return {"tile_uq": tile_uq, "slide_uq": slide_uq, "tile_pred": tile_pred, "slide_pred": slide_pred}, auc
-
-
-def from_cv_sharded(dfs, group=None, **kwargs):
-    """`from_cv` with every fold table sharded over the ranks: `detect_sharded` per fold, same fold-skipping and
-    min / max / mean reduction over folds as the reference (threshold.py:478-557)."""
-    return _from_cv(dfs, lambda df, **kw: detect_sharded(df, group=group, **kw), kwargs, require_patient=False)
+    _apply_preamble(df, tile_uq, keep, patients, level)
+    with ShardedTable(df, group=group) as table:
+        return apply_resident(table, tile_uq, slide_uq, tile_pred=tile_pred, slide_pred=slide_pred, keep=keep,
+                              patients=patients, level=level)
 
 
 def detect(df, tile_uq="detect", slide_uq="detect", tile_pred="detect", slide_pred="detect",
@@ -709,9 +605,8 @@ def detect(df, tile_uq="detect", slide_uq="detect", tile_pred="detect", slide_pr
 
 def detect_resident(table: ResidentTable, tile_uq="detect", slide_uq="detect", tile_pred="detect", slide_pred="detect",
                     plot=False, patients=None):
-    """`detect` on a GPU-resident table (see :class:`ResidentTable`)."""
+    """`detect` on a GPU-resident table (see :class:`ResidentTable`) or on this rank's :class:`ShardedTable`."""
     none4 = {k: None for k in _THRESH_KEYS}
-    tab = table.tab
     try:
         found_tile_pred = table.tile_stage(tile_pred, patients)       # :398-402
     except errors.PredsContainNaNError:
@@ -720,19 +615,16 @@ def detect_resident(table: ResidentTable, tile_uq="detect", slide_uq="detect", t
     if _is_detect(tile_pred):                                         # :407-408
         tile_pred = found_tile_pred
     if isinstance(tile_uq, _FLOAT_TYPES):                             # :411-412
-        tile_uq_eff = _cmp_scalar(tile_uq, tab.dtype)
+        tile_uq_eff = _cmp_scalar(tile_uq, table.dtype)
     elif not _is_detect(tile_uq):                                     # :413-415
         log.debug("Not performing tile-level uncertainty thresholding.")
         tile_uq, tile_uq_eff = None, None
     else:                                                             # :416-426
-        if getattr(tab, "n_unc_nonfinite", 0):                         # roc_curve -> assert_all_finite (uncaught at :419)
-            raise ValueError("Input contains NaN or infinity.")
-        r = tab.tile_roc(_ffi.SCORE_UNCERTAINTY, _ffi.LABEL_INCORRECT)
-        tile_uq = _youden_or_raise(r)
+        tile_uq = table.tile_uq_threshold()
         log.debug(f"Tile-level optimal UQ threshold: {tile_uq:.4f}")
         tile_uq_eff = float(tile_uq)
     try:
-        s_df, slide_pred = table.groups("slide", tile_uq_eff, slide_pred)   # :433-438
+        s_df, slide_pred, _ = table.group_table("slide", tile_uq_eff, slide_pred)   # :433-438
     except errors.ROCFailedError:
         log.error("Unable to process slide predictions")
         return none4, None                                            # :439-441
@@ -761,6 +653,16 @@ def _detect_group_level(ctx, s_df, slide_uq, slide_pred):
     return slide_uq, _auc_included(ctx, yp, yt, include)              # :468
 
 
+def detect_sharded(df, tile_uq="detect", slide_uq="detect", tile_pred="detect", slide_pred="detect",
+                   patients=None, group=None):
+    """`detect` for a table sharded over ranks (see :class:`ShardedTable`): the reference's threshold.py:364-475 on the
+    concatenated table, with the tile-level ROCs over all tiles of the cohort.  Returns what `detect` returns, on every
+    rank."""
+    with ShardedTable(df, group=group) as table:
+        return detect_resident(table, tile_uq=tile_uq, slide_uq=slide_uq, tile_pred=tile_pred, slide_pred=slide_pred,
+                               patients=patients)
+
+
 def from_cv(dfs, **kwargs):
     """Optimal tile- and slide-level thresholds from a set of (nested) cross-validation folds
     (reference threshold.py:478-557): `detect` per fold, folds without a tile_uq / slide_uq are
@@ -773,6 +675,12 @@ def from_cv(dfs, **kwargs):
 
     Raises ValueError for missing columns and ThresholdError when no fold yields a threshold."""
     return _from_cv(dfs, detect, kwargs)
+
+
+def from_cv_sharded(dfs, group=None, **kwargs):
+    """`from_cv` with every fold table sharded over the ranks: `detect_sharded` per fold, same fold-skipping and
+    min / max / mean reduction over folds as the reference (threshold.py:478-557)."""
+    return _from_cv(dfs, lambda df, **kw: detect_sharded(df, group=group, **kw), kwargs, require_patient=False)
 
 
 class FoldSet:

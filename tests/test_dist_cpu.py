@@ -1,7 +1,7 @@
-"""CPU tier (gloo, world_size 2): the multi-GPU host logic of the path -- slide-aligned sharding and the single
-all-gather of per-slide aggregates -- reproduces the single-process group table exactly.  The per-shard
-aggregates are produced here by the oracle's pandas-order Kahan mean (the CUDA reduction is checked against
-the same oracle in the GPU tier)."""
+"""CPU tier (gloo, world_size 2): the multi-GPU host logic of the path -- slide-aligned sharding and the
+all-gather of per-slide aggregates and names that `threshold.ShardedTable` runs -- reproduces the single-process
+group table exactly.  The per-shard aggregates are produced here by the oracle's pandas-order Kahan mean (the
+CUDA reduction is checked against the same oracle in the GPU tier)."""
 import os
 import socket
 
@@ -40,19 +40,14 @@ def _worker(rank, world, port, out_dir):
     try:
         df = synth.tile_table(n_slides=11, tiles_per_slide=40, seed=21, ragged=True)
         counts = df.groupby("slide", sort=False).size().to_numpy()
-        bounds = bdist.shard_bounds(counts, world)
-        lo, hi = bounds[rank]
-        row_lo, row_hi = int(counts[:lo].sum()), int(counts[:hi].sum())
-        local = df.iloc[row_lo:row_hi].reset_index(drop=True)
-        names, gp, gu, gt, cnt, first = _local_groups(local)
-        meta = [None] * world
-        dist.all_gather_object(meta, (len(names), len(local)))
-        code_off = sum(m[0] for m in meta[:rank])
-        row_off = sum(m[1] for m in meta[:rank])
-        msg = bdist.pack_groups(code_off, cnt, first, row_off, gp, gu, gt)
-        allmsg = bdist.all_gather_groups(msg)
-        g = bdist.unpack_groups(allmsg, np.float32)
-        np.savez(os.path.join(out_dir, f"rank{rank}.npz"), **g, row_off=row_off, code_off=code_off)
+        lo, hi = bdist.shard_bounds(counts, world)[rank]
+        local = df.iloc[int(counts[:lo].sum()):int(counts[:hi].sum())].reset_index(drop=True)
+        # "split": slide-aligned shards; "empty": rank 0 holds the whole table and the last rank an EMPTY shard
+        for case, shard in (("split", local), ("empty", df if rank == 0 else df.iloc[0:0])):
+            names, gp, gu, gt, cnt, first = _local_groups(shard)
+            g, all_names, n_keys = bdist.all_gather_groups(names, (gp, gu, gt, cnt, first), len(shard), len(names),
+                                                           np.float32)
+            np.savez(os.path.join(out_dir, f"{case}{rank}.npz"), **g, names=np.array(all_names), n_keys=n_keys)
     finally:
         dist.destroy_process_group()
 
@@ -72,25 +67,28 @@ def test_shard_bounds_properties():
     assert bdist.shard_bounds([2000] * 1000, 8) == [(125 * r, 125 * (r + 1)) for r in range(8)]
 
 
-def test_all_gather_groups_world2(tmp_path):
+def test_all_gather_groups_exchange_world2(tmp_path):
     world = 2
     mp.spawn(_worker, args=(world, _free_port(), str(tmp_path)), nprocs=world, join=True)
     df = synth.tile_table(n_slides=11, tiles_per_slide=40, seed=21, ragged=True)
     names, gp, gu, gt, cnt, first = _local_groups(df)
-    for r in range(world):
-        g = np.load(tmp_path / f"rank{r}.npz")
-        assert np.array_equal(g["code"], np.arange(len(names)))
-        assert np.array_equal(g["count"], cnt)
-        assert g["y_pred"].tobytes() == gp.tobytes()                # bit-exact: slides never straddle ranks
-        assert g["uncertainty"].tobytes() == gu.tobytes()
-        assert np.array_equal(g["y_true"], gt.astype(np.uint8))
+    for case in ("split", "empty"):
+        for r in range(world):
+            g = np.load(tmp_path / f"{case}{r}.npz")
+            assert np.array_equal(g["code"], np.arange(len(names)))
+            assert np.array_equal(g["count"], cnt)
+            assert g["y_pred"].tobytes() == gp.tobytes()            # bit-exact: slides never straddle ranks
+            assert g["uncertainty"].tobytes() == gu.tobytes()
+            assert np.array_equal(g["y_true"], gt.astype(np.uint8))
+            assert list(g["names"]) == names and int(g["n_keys"]) == len(names)
 
 
-def test_single_process_passthrough():
-    msg = bdist.pack_groups(0, [3, 0, 2], [0, -1, 5], 0, np.float32([.1, np.nan, .3]), np.float32([.01, np.nan, .03]),
-                            [0.0, np.nan, 1.0])
-    out = bdist.unpack_groups(bdist.all_gather_groups(msg), np.float32)
-    assert list(out["code"]) == [0, 2] and list(out["y_true"]) == [0, 1]
+def test_all_gather_groups_single_process():
+    g, names, n_keys = bdist.all_gather_groups(
+        ["a", "b", "c"], (np.float32([.1, np.nan, .3]), np.float32([.01, np.nan, .03]), [0.0, np.nan, 1.0], [3, 0, 2],
+                          [0, -1, 5]), 6, 3, np.float32)
+    assert list(g["code"]) == [0, 2] and list(g["y_true"]) == [0, 1]
+    assert names == ["a", "b", "c"] and n_keys == 3
 
 
 # ----------------------------------------------------------------------------------------------------------------
