@@ -457,34 +457,38 @@ int build_plan(bq_model* m) {
   int H = s2, C = 64;
 
   int dw_rc = BQ_OK;
-  int n_dw = 0;
-  auto add_dw = [&](const bf16* in, bf16* out, int h, int c, int relu_in, const SepWeights& sw, int stage, int in_pitch = 0) {
+  // Every op carries a tag so that bq_model_debug_stage can stop behind it: block{b}_sub, block{b}_res,
+  // block{b}_sepconv{i}_dw (stand-alone depthwise), block{b}_sepconv{i} (SeparableConv after BN / ReLU), and block{b} for
+  // a block output (the last sepconv of blocks 5-12 with its residual, and block14_sepconv2).
+  auto add_dw = [&](const bf16* in, bf16* out, int h, int c, int relu_in, const SepWeights& sw, int stage, const std::string& tag,
+                    int in_pitch = 0) {
     Op op; op.kind = OP_DW; op.stage = stage; op.in = in; op.out = out; op.H = h; op.W = h; op.C = c;
     op.relu_in = relu_in; op.dw = (const float*)sw.dw.p;
     const int CC = (c % 64 != 0) ? 56 : 64;                            // 728 = 13 x 56
     int r = make_tmap_nhwc(ctx, &op.ta, in, (uint64_t)B, (uint64_t)h, (uint64_t)h, (uint64_t)c, bq::dwp::kHalo, bq::dwp::kHalo, CC,
                            false, false, (uint64_t)in_pitch);
     if (r && !dw_rc) dw_rc = r;
-    op.tag = "dw" + std::to_string(n_dw++);          // debug-stage name of the n-th stand-alone depthwise output
+    op.tag = tag;
     op.Ho = h; op.Wo = h; op.Cout = c;
     m->plan.push_back(op);
   };
   auto add_gemm = [&](const bf16* a, int rows, const PwWeights& w, bf16* out, int relu, const bf16* resid, int stage,
-                      const char* tag, int h, int cout) -> int {
+                      const std::string& tag, int h, int cout) -> int {
     Op op; op.stage = stage;
     int r = make_gemm(m, op, a, rows, w, out, relu, resid);
     if (r) return r;
-    if (tag) op.tag = tag;
+    op.tag = tag;
     op.Ho = h; op.Wo = h; op.Cout = cout;
     m->plan.push_back(op);
     return BQ_OK;
   };
-  // one SeparableConv2D (+BN, optional ReLU / residual): fused kernel for 728->728, otherwise depthwise + GEMM
+  // one SeparableConv2D `name` (+BN, optional ReLU / residual): fused entry-flow kernel for 64/128/256 -> 128/256,
+  // otherwise depthwise + GEMM; the output is tagged `tag`, or `name` when tag is null
   auto add_sep = [&](const bf16* in, bf16* dw_tmp, int h, int cin, int relu_in, const SepWeights& sw, bf16* out, int relu_out,
-                     const bf16* resid, int stage, const char* tag, int in_pitch = 0) -> int {
+                     const bf16* resid, int stage, const std::string& name, const char* tag, int in_pitch = 0) -> int {
     if (!in_pitch && !m->use_simt && !resid && cin % 64 == 0 && cin <= 256 && (sw.pw.cout == 128 || sw.pw.cout == 256)) {
       Op op; op.kind = OP_SEP2D; op.stage = stage;
-      if (tag) op.tag = tag;
+      op.tag = tag ? tag : name;
       op.in = in; op.out = out; op.H = h; op.W = h; op.C = cin; op.Ho = h; op.Wo = h; op.Cout = sw.pw.cout;
       op.s2.n_img = B; op.s2.H = h; op.s2.W = h; op.s2.K = cin; op.s2.N = sw.pw.cout;
       op.s2.relu_in = relu_in; op.s2.relu_out = relu_out;
@@ -497,8 +501,8 @@ int build_plan(bq_model* m) {
       m->plan.push_back(op);
       return BQ_OK;
     }
-    add_dw(in, dw_tmp, h, cin, relu_in, sw, stage, in_pitch);
-    return add_gemm(dw_tmp, h * h, sw.pw, out, relu_out, resid, stage, tag, h, sw.pw.cout);
+    add_dw(in, dw_tmp, h, cin, relu_in, sw, stage, name + "_dw", in_pitch);
+    return add_gemm(dw_tmp, h * h, sw.pw, out, relu_out, resid, stage, tag ? tag : name, h, sw.pw.cout);
   };
   // entry-style block with a strided 1x1 residual branch and a max-pool (blocks 2,3,4,13)
   // `padded_in` / `padded_out`: the block input / output lives in the zero-padded middle-flow layout (pitch 20), which
@@ -509,18 +513,20 @@ int build_plan(bq_model* m) {
     const int Ho = (H + 1) / 2;
     const bf16* xin = padded_in ? padded_in : A.p(X);
     const int in_pitch = padded_in ? bq::sepmid::kPitch : 0;
-    const SepWeights& s1w = *m->sep.at("block" + std::to_string(b) + "_sepconv1");
-    const SepWeights& s2w = *m->sep.at("block" + std::to_string(b) + "_sepconv2");
-    const PwWeights& rw = *m->res.at("block" + std::to_string(b) + "_res");
-    { Op op; op.kind = OP_SUBSAMPLE; op.stage = stage; op.in = xin; op.in_pitch = in_pitch; op.out = A.p(t[0]); op.H = H; op.W = H; op.Ho = Ho; op.Wo = Ho; op.C = C; m->plan.push_back(op); }
+    const std::string pre = "block" + std::to_string(b);
+    const SepWeights& s1w = *m->sep.at(pre + "_sepconv1");
+    const SepWeights& s2w = *m->sep.at(pre + "_sepconv2");
+    const PwWeights& rw = *m->res.at(pre + "_res");
+    { Op op; op.kind = OP_SUBSAMPLE; op.stage = stage; op.in = xin; op.in_pitch = in_pitch; op.out = A.p(t[0]); op.H = H; op.W = H; op.Ho = Ho; op.Wo = Ho; op.C = C;
+      op.Cout = C; op.tag = pre + "_sub"; m->plan.push_back(op); }
     int r;
-    if ((r = add_gemm(A.p(t[0]), Ho * Ho, rw, A.p(t[1]), 0, nullptr, stage, nullptr, Ho, cout2))) return r;   // res -> t1
-    if ((r = add_sep(xin, A.p(t[0]), H, C, relu_first, s1w, A.p(t[2]), 1, nullptr, stage, nullptr, in_pitch))) return r;
-    if ((r = add_sep(A.p(t[2]), A.p(t[0]), H, cout1, 0, s2w, A.p(t[3]), 0, nullptr, stage, nullptr))) return r;
+    if ((r = add_gemm(A.p(t[0]), Ho * Ho, rw, A.p(t[1]), 0, nullptr, stage, pre + "_res", Ho, cout2))) return r;   // res -> t1
+    if ((r = add_sep(xin, A.p(t[0]), H, C, relu_first, s1w, A.p(t[2]), 1, nullptr, stage, pre + "_sepconv1", nullptr, in_pitch))) return r;
+    if ((r = add_sep(A.p(t[2]), A.p(t[0]), H, cout1, 0, s2w, A.p(t[3]), 0, nullptr, stage, pre + "_sepconv2", nullptr))) return r;
     { Op op; op.kind = OP_POOLADD; op.stage = stage; op.in = A.p(t[3]); op.in2 = A.p(t[1]); op.out = padded_out ? padded_out : A.p(X);
       op.out_pitch = padded_out ? bq::sepmid::kPitch : 0; op.padded_out = padded_out != nullptr;
       op.H = H; op.W = H; op.Ho = Ho; op.Wo = Ho; op.C = cout2; op.Cout = cout2; op.pad_top = same_pad_before(H); op.pad_left = same_pad_before(H);
-      op.tag = "block" + std::to_string(b); m->plan.push_back(op); }
+      op.tag = pre; m->plan.push_back(op); }
     H = Ho; C = cout2;
     return BQ_OK;
   };
@@ -544,9 +550,9 @@ int build_plan(bq_model* m) {
   if (mid) {
     using namespace bq::sepmid;
     const uint64_t rows = (uint64_t)B * kImgRows + kSlackRows;
-    auto add_mid = [&](int src, int dst, int res, const SepWeights& sw, int relu_in, int relu_out, const char* tag) -> int {
+    auto add_mid = [&](int src, int dst, int res, const SepWeights& sw, int relu_in, int relu_out, const std::string& tag) -> int {
       Op op; op.kind = OP_SEPMID; op.stage = 3; op.padded_out = true;
-      if (tag) op.tag = tag;
+      op.tag = tag;
       op.in = P(src); op.out = P(dst); op.in2 = res >= 0 ? P(res) : nullptr;
       op.H = kMap; op.W = kMap; op.C = kC; op.Ho = kMap; op.Wo = kMap; op.Cout = kC; op.relu_in = relu_in;
       op.sm.n_rows = B * kImgRows; op.sm.relu_out = relu_out;
@@ -568,9 +574,9 @@ int build_plan(bq_model* m) {
       const SepWeights &w1 = *m->sep.at(pre + "1"), &w2 = *m->sep.at(pre + "2"), &w3 = *m->sep.at(pre + "3");
       const std::string tag = "block" + std::to_string(b);
       const int a = (x + 1) & 3, bb = (x + 2) & 3, c = (x + 3) & 3;
-      if ((rc = add_mid(x, a, -1, w1, 1, 1, nullptr))) return rc;
-      if ((rc = add_mid(a, bb, -1, w2, 0, 1, nullptr))) return rc;
-      if ((rc = add_mid(bb, c, x, w3, 0, 0, tag.c_str()))) return rc;
+      if ((rc = add_mid(x, a, -1, w1, 1, 1, pre + "1"))) return rc;
+      if ((rc = add_mid(a, bb, -1, w2, 0, 1, pre + "2"))) return rc;
+      if ((rc = add_mid(bb, c, x, w3, 0, 0, tag))) return rc;
       x = c;
     }
     mid_out = x;
@@ -581,9 +587,9 @@ int build_plan(bq_model* m) {
     const SepWeights &w1 = *m->sep.at(pre + "1"), &w2 = *m->sep.at(pre + "2"), &w3 = *m->sep.at(pre + "3");
     // (the unfused path ping-pongs t0 <-> t1; the fused kernel must not write its own input, so it uses t1 -> t3 -> t2)
     const std::string tag = "block" + std::to_string(b);
-    if ((rc = add_sep(A.p(X), A.p(t[0]), H, C, 1, w1, A.p(t[1]), 1, nullptr, 3, nullptr))) return rc;
-    if ((rc = add_sep(A.p(t[1]), A.p(t[0]), H, C, 0, w2, A.p(t[3]), 1, nullptr, 3, nullptr))) return rc;
-    if ((rc = add_sep(A.p(t[3]), A.p(t[0]), H, C, 0, w3, A.p(t[2]), 0, A.p(X), 3, tag.c_str()))) return rc;
+    if ((rc = add_sep(A.p(X), A.p(t[0]), H, C, 1, w1, A.p(t[1]), 1, nullptr, 3, pre + "1", nullptr))) return rc;
+    if ((rc = add_sep(A.p(t[1]), A.p(t[0]), H, C, 0, w2, A.p(t[3]), 1, nullptr, 3, pre + "2", nullptr))) return rc;
+    if ((rc = add_sep(A.p(t[3]), A.p(t[0]), H, C, 0, w3, A.p(t[2]), 0, A.p(X), 3, pre + "3", tag.c_str()))) return rc;
     X = t[2];
   }
   // ---- exit flow
@@ -591,9 +597,9 @@ int build_plan(bq_model* m) {
   {
     int t[4]; others(X, t);
     const SepWeights &w1 = *m->sep.at("block14_sepconv1"), &w2 = *m->sep.at("block14_sepconv2");
-    add_dw(A.p(X), A.p(t[0]), H, C, 0, w1, 4);
-    if ((rc = add_gemm(A.p(t[0]), H * H, w1.pw, A.p(t[1]), 1, nullptr, 4, nullptr, H, 1536))) return rc;
-    add_dw(A.p(t[1]), A.p(t[0]), H, 1536, 0, w2, 4);
+    add_dw(A.p(X), A.p(t[0]), H, C, 0, w1, 4, "block14_sepconv1_dw");
+    if ((rc = add_gemm(A.p(t[0]), H * H, w1.pw, A.p(t[1]), 1, nullptr, 4, "block14_sepconv1", H, 1536))) return rc;
+    add_dw(A.p(t[1]), A.p(t[0]), H, 1536, 0, w2, 4, "block14_sepconv2_dw");
     if ((rc = add_gemm(A.p(t[0]), H * H, w2.pw, A.p(t[2]), 1, nullptr, 4, "block14", H, kFeatures))) return rc;
     Op op; op.kind = OP_GAP; op.stage = 4; op.in = A.p(t[2]); op.H = H; op.W = H; op.C = kFeatures; m->plan.push_back(op);
   }
@@ -1235,6 +1241,35 @@ int bq_model_debug_stage(bq_model* m, const uint8_t* tiles, int64_t n, const cha
     src = dense;
   }
   bf16_to_f32_kernel<<<1024, 256, 0, ctx->stream>>>(src, (float*)scr, total);
+  BQ_LAUNCH_CHECK(ctx);
+  if ((rc = bq_from_device(ctx, out, scr, total * 4))) return rc;
+  BQ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return BQ_OK;
+}
+
+int bq_model_debug_tags(bq_model* m, char* out, int64_t capacity) {
+  if (!m) return BQ_ERR_ARG;
+  std::string all;
+  for (const Op& op : m->plan)
+    if (!op.tag.empty()) all += op.tag + "\n";
+  if (!out || (int64_t)all.size() + 1 > capacity)
+    return bq_fail(m->ctx, BQ_ERR_ARG, "bq_model_debug_tags: need %lld bytes", (long long)all.size() + 1);
+  memcpy(out, all.c_str(), all.size() + 1);
+  return BQ_OK;
+}
+
+int bq_model_debug_h1(bq_model* m, int64_t n, float* out) {
+  if (!m) return BQ_ERR_ARG;
+  bq_ctx* ctx = m->ctx;
+  if (!out || n < 1 || n > m->head_batch || !m->h_act[0].p || (m->sites & 1))
+    return bq_fail(ctx, BQ_ERR_ARG, "bq_model_debug_h1: needs a preceding predict of >= n tiles (n <= %d) with no dropout on the features",
+                   m->head_batch);
+  BQ_CUDA(ctx, cudaSetDevice(ctx->device));
+  const int64_t total = n * m->cfg.hidden_width;
+  void* scr = nullptr;
+  int rc;
+  if ((rc = bq_scratch(ctx, total * 4, &scr))) return rc;
+  bf16_to_f32_kernel<<<1024, 256, 0, ctx->stream>>>((const bf16*)m->h_act[0].p, (float*)scr, total);
   BQ_LAUNCH_CHECK(ctx);
   if ((rc = bq_from_device(ctx, out, scr, total * 4))) return rc;
   BQ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));

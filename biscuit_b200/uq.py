@@ -169,8 +169,12 @@ class UncertaintyInterface:
 
     # ------------------------------------------------------------------------------------
     def debug_stage(self, tiles: np.ndarray, stage: str) -> np.ndarray:
-        """Parity hook: NHWC float32 copy of a named backbone stage ('block1_conv1', 'block1_conv2',
-        'block2' ... 'block14')."""
+        """Parity hook: NHWC float32 copy of the output of one op of the backbone plan, run up to that op.
+        Tags: 'block1_conv1', 'block1_conv2'; 'block{b}_sub' (stride-2 subsample) and 'block{b}_res' (1x1 residual GEMM)
+        for b in 2, 3, 4, 13; 'block{b}_sepconv{i}_dw' (a depthwise output, where the depthwise runs as its own kernel);
+        'block{b}_sepconv{i}' (a SeparableConv after BatchNorm and ReLU); 'block{b}' for a block output: blocks 2-4 and 13
+        after max-pool + residual, blocks 5-12 after the third sepconv + residual (no separate 'block{b}_sepconv3' tag),
+        and 'block14' = block14_sepconv2 (no separate tag)."""
         n = int(tiles.shape[0])
         cap = n * 149 * 149 * 128
         out = np.empty(cap, np.float32)
@@ -181,6 +185,19 @@ class UncertaintyInterface:
                    "bq_model_debug_stage")
         s = tuple(int(x) for x in shape)
         return out[: int(np.prod(s))].reshape(s).copy()
+
+    def debug_h1(self, n: int) -> np.ndarray:
+        """Parity hook: hidden_0 output (bf16 as float32, [n, hidden_width]) of the first n tiles of the last `predict`
+        call (which must have held them in one head batch, with no dropout on the pooled features)."""
+        out = np.empty((int(n), self.config.hidden_layer_width), np.float32)
+        _ffi.check(self.ctx.handle, self.lib.bq_model_debug_h1(self.h, int(n), _ffi.ptr(out)), "bq_model_debug_h1")
+        return out
+
+    def debug_tags(self) -> list:
+        """the `debug_stage` tags of the execution plan, in execution order"""
+        buf = C.create_string_buffer(1 << 16)
+        _ffi.check(self.ctx.handle, self.lib.bq_model_debug_tags(self.h, buf, len(buf)), "bq_model_debug_tags")
+        return buf.value.decode().split()
 
     KERNEL_FAMILIES = ("tile_stats", "conv1", "gemm_conv2", "gemm_pointwise", "depthwise", "maxpool_add",
                        "subsample", "gap", "head_gemm", "mc_expand", "head_final", "head_fused", "sepconv_fused", "sepconv_mid")

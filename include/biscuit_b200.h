@@ -180,6 +180,11 @@ int bq_predict_uq_standardized(bq_model* m, const float* tiles, int64_t n, int32
  * float32 (NHWC).  Used by tests to localise a mismatch; not part of the reference surface. */
 int bq_model_debug_stage(bq_model* m, const uint8_t* tiles, int64_t n, const char* stage, float* out,
                          int64_t out_capacity, int64_t out_shape[4]);
+/* hidden_0 activations (bf16 as float32, [n, hidden_width]) of the first n tiles of the last bq_predict_uq call, when
+ * that call held them in one head batch and dropout on the pooled features is off. */
+int bq_model_debug_h1(bq_model* m, int64_t n, float* out);
+/* the debug_stage tags of the execution plan in execution order, one per line (NUL-terminated) */
+int bq_model_debug_tags(bq_model* m, char* out, int64_t capacity);
 
 /* per-stage device time of the last bq_predict_uq call, in ms: {stats+conv1, conv2, entry, middle,
  * exit, head} -- measured with CUDA events on the ctx stream when enabled */
