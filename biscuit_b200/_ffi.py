@@ -97,7 +97,19 @@ SIGNATURES = {
     "bq_debug_umma_probe": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "bq_model_kernel_profile": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double),
                                           C.POINTER(C.c_double), C.POINTER(C.c_int64)]),
+    "bq_jpeg_status_string": (C.c_char_p, [C.c_int32]),
+    "bq_jpeg_inspect": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p]),
+    "bq_jpeg_decode": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]),
+    "bq_jpeg_last_stats": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64)]),
+    "bq_predict_uq_jpeg": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_uint64, C.c_uint64,
+                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "bq_tfrecord_scan": (C.c_int, [C.c_void_p, C.c_int64, C.c_char_p, C.c_char_p, C.c_char_p, C.c_char_p, C.c_int64,
+                                   C.POINTER(C.c_int64), C.c_void_p, C.c_void_p, C.c_void_p, C.c_char_p, C.c_int64]),
+    "bq_crc32c": (C.c_uint32, [C.c_void_p, C.c_int64]),
+    "bq_crc32c_masked": (C.c_uint32, [C.c_void_p, C.c_int64]),
 }
+
+BQ_ERR_DATA = -6
 
 _lib = None
 _lock = threading.Lock()
@@ -131,11 +143,14 @@ def load_library():
 
 
 def check(ctx_handle, rc, what=""):
+    """raise on a failing return code: ValueError for malformed input data (BQ_ERR_DATA), else NativeLibraryError"""
     if rc == 0:
         return
     lib = load_library()
     msg = lib.bq_last_error(ctx_handle)
     msg = msg.decode() if msg else ""
+    if rc == BQ_ERR_DATA:
+        raise ValueError(msg)
     raise NativeLibraryError(f"{what or 'libbiscuit_b200 call'} failed (rc={rc}): {msg}")
 
 

@@ -66,6 +66,7 @@ void bq_destroy(bq_ctx* ctx) {
     cudaStreamDestroy(ctx->stream);
   }
   if (ctx->scratch) cudaFree(ctx->scratch);
+  bq_jpeg_state_destroy(ctx->jpeg);
   if (ctx->pinned) cudaFreeHost(ctx->pinned);
   delete ctx;
 }

@@ -263,6 +263,7 @@ struct bq_model {
   const uint8_t* tiles_src = nullptr;          // where stats / conv1 read the current micro-batch from
   cudaStream_t copy_stream = nullptr;          // H2D of micro-batch i+1 overlaps the backbone of micro-batch i
   cudaEvent_t copied[2] = {}, consumed[2] = {};
+  bq_jpeg_state* jpeg = nullptr;               // bq_predict_uq_jpeg: descriptors, compressed staging and decode scratch
   DevBuf mean, inv_std;                        // fp32 [max_batch]
   Arena arena;
   DevBuf feat, feat_bf16;                      // [max_batch, 2048]
@@ -966,6 +967,7 @@ void bq_model_destroy(bq_model* m) {
   for (auto& e : m->kev) cudaEventDestroy(e);
   if (m->copy_stream) { cudaStreamSynchronize(m->copy_stream); cudaStreamDestroy(m->copy_stream); }
   for (int i = 0; i < 2; ++i) { if (m->copied[i]) cudaEventDestroy(m->copied[i]); if (m->consumed[i]) cudaEventDestroy(m->consumed[i]); }
+  bq_jpeg_state_destroy(m->jpeg);
   delete m;
 }
 
@@ -1079,25 +1081,35 @@ int bq_model_load_weights(bq_model* m, const bq_named_tensor* tensors, int32_t n
   return BQ_OK;
 }
 
-static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, int64_t n, int32_t T, uint64_t seed,
-                        uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std, float* features);
+static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, const int64_t* jpeg_offsets, int64_t n,
+                        int32_t T, uint64_t seed, uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std,
+                        float* features);
 
 int bq_predict_uq(bq_model* m, const uint8_t* tiles, int64_t n, int32_t T, uint64_t seed, uint64_t tile_index_base,
                   const uint8_t* masks, float* mean, float* std, float* features) {
-  return predict_impl(m, tiles, false, n, T, seed, tile_index_base, masks, mean, std, features);
+  return predict_impl(m, tiles, false, nullptr, n, T, seed, tile_index_base, masks, mean, std, features);
+}
+
+int bq_predict_uq_jpeg(bq_model* m, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t T, uint64_t seed,
+                       uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std, float* features) {
+  if (!m) return BQ_ERR_ARG;
+  if (n > 0 && !offsets) return bq_fail(m->ctx, BQ_ERR_ARG, "bq_predict_uq_jpeg: offsets must not be NULL");
+  return predict_impl(m, data, false, offsets, n, T, seed, tile_index_base, masks, mean, std, features);
 }
 
 int bq_predict_uq_standardized(bq_model* m, const float* tiles, int64_t n, int32_t T, uint64_t seed, uint64_t tile_index_base,
                                const uint8_t* masks, float* mean, float* std, float* features) {
   if (!m) return BQ_ERR_ARG;
   m->input_f32 = true;
-  const int rc = predict_impl(m, (const uint8_t*)tiles, true, n, T, seed, tile_index_base, masks, mean, std, features);
+  const int rc = predict_impl(m, (const uint8_t*)tiles, true, nullptr, n, T, seed, tile_index_base, masks, mean, std,
+                              features);
   m->input_f32 = false;
   return rc;
 }
 
-static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, int64_t n, int32_t T, uint64_t seed,
-                        uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std, float* features) {
+static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, const int64_t* jpeg_offsets, int64_t n,
+                        int32_t T, uint64_t seed, uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std,
+                        float* features) {
   if (!m) return BQ_ERR_ARG;
   bq_ctx* ctx = m->ctx;
   if (!m->weights_loaded) return bq_fail(ctx, BQ_ERR_STATE, "bq_predict_uq: weights not loaded");
@@ -1118,8 +1130,15 @@ static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, int64
   if (m->profiling == 2)
     for (int k = 0; k < BQ_PROFILE_KINDS; ++k) { m->k_ms[k] = m->k_flops[k] = m->k_bytes[k] = 0; m->k_launches[k] = 0; }
   // Host tiles: double-buffered staging, the H2D copy of micro-batch i+1 runs on its own stream while the
-  // backbone of micro-batch i computes.  Device tiles are read in place.
-  const bool tiles_on_dev = bq_is_device_ptr(tiles);
+  // backbone of micro-batch i computes.  Device tiles are read in place.  JPEG tiles always take the staged route:
+  // micro-batch i + 1's descriptors (and its compressed bytes, unless they are device memory, which is read in place)
+  // go up on the copy stream, and micro-batch i is decoded on the ctx stream into tiles_dev.
+  const bool jpeg = jpeg_offsets != nullptr;
+  if (jpeg) {
+    const int rcj = bq_jpeg_prepare(ctx, m->jpeg, tiles, jpeg_offsets, n, m->px, B, nullptr);
+    if (rcj) return rcj;
+  }
+  const bool tiles_on_dev = !jpeg && bq_is_device_ptr(tiles);
   if (f32_input && !tiles_on_dev) {
     const int64_t cap = n < B ? n : B;                      // the interface is usually called tile by tile (results.py:249-257)
     for (auto& b : m->tiles_f32) { int rcf = bq_alloc(ctx, b, (size_t)cap * tile_bytes + 64); if (rcf) return rcf; }
@@ -1128,8 +1147,13 @@ static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, int64
   auto issue_copy = [&](int64_t i0c, int slot) -> int {
     const int nbc = (int)((n - i0c < B) ? (n - i0c) : B);
     BQ_CUDA(ctx, cudaStreamWaitEvent(m->copy_stream, m->consumed[slot], 0));   // previous reader of this slot done
-    BQ_CUDA(ctx, cudaMemcpyAsync(stage[slot], tiles + (size_t)i0c * tile_bytes, (size_t)nbc * tile_bytes,
-                                 cudaMemcpyHostToDevice, m->copy_stream));
+    if (jpeg) {
+      const int rcu = bq_jpeg_upload(ctx, m->jpeg, i0c / B, slot, m->copy_stream);
+      if (rcu) return rcu;
+    } else {
+      BQ_CUDA(ctx, cudaMemcpyAsync(stage[slot], tiles + (size_t)i0c * tile_bytes, (size_t)nbc * tile_bytes,
+                                   cudaMemcpyHostToDevice, m->copy_stream));
+    }
     BQ_CUDA(ctx, cudaEventRecord(m->copied[slot], m->copy_stream));
     return BQ_OK;
   };
@@ -1147,6 +1171,11 @@ static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, int64
     } else {
       BQ_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, m->copied[slot], 0));
       m->tiles_src = stage[slot];
+      if (jpeg) {
+        if ((rc = bq_jpeg_decode_group(ctx, m->jpeg, batch_idx, slot, (uint8_t*)m->tiles_dev.p))) return rc;
+        BQ_CUDA(ctx, cudaEventRecord(m->consumed[slot], ctx->stream));        // the compressed slot is free once decoded
+        m->tiles_src = (const uint8_t*)m->tiles_dev.p;
+      }
     }
     const uint8_t* mdev = nullptr;       // masks of the head batch (device)
     if (masks) {
@@ -1166,7 +1195,7 @@ static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, int64
     }
     if ((rc = run_backbone_graphed(m, nb))) return rc;
     if (!tiles_on_dev) {
-      BQ_CUDA(ctx, cudaEventRecord(m->consumed[slot], ctx->stream));
+      if (!jpeg) BQ_CUDA(ctx, cudaEventRecord(m->consumed[slot], ctx->stream));
       // The next micro-batch's copy is issued AFTER this one's backbone is queued: a copy from PAGEABLE memory blocks the
       // calling thread while the driver stages it, and that time must fall under queued GPU work (from pinned memory the
       // call returns at once and the order makes no difference).
@@ -1204,6 +1233,7 @@ static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, int64
     }
   }
   BQ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  if (jpeg) return bq_jpeg_finish(ctx, m->jpeg, nullptr);
   return BQ_OK;
 }
 

@@ -1,0 +1,123 @@
+"""JPEG tiles decoded on the GPU (csrc/jpeg.cu, csrc/jpeg_sm100.cuh).
+
+A `JpegBatch` holds n JPEG files back to back.  `decode(batch)` returns the uint8 tiles, byte for byte what
+`np.asarray(PIL.Image.open(io.BytesIO(b)).convert("RGB"))` gives (libjpeg-turbo's default decode: JDCT_ISLOW IDCT,
+fancy upsampling, jdcolor.c YCbCr->RGB), and `UncertaintyInterface.predict(batch)` runs MC-dropout inference on them
+with the decode in front of the backbone, micro-batch by micro-batch.
+
+Accepted: baseline / extended sequential Huffman JPEG, 8-bit, 3 components (YCbCr), sampling 4:4:4, 4:2:2 or 4:2:0,
+any quantisation / Huffman tables, restart intervals, APPn / COM segments, size tile_px x tile_px.  Everything else
+raises ValueError naming the tile before anything runs on the GPU; an entropy-coded segment that is truncated or holds
+an invalid code raises ValueError naming the tile after the batch.
+"""
+from __future__ import annotations
+
+import ctypes as C
+
+import numpy as np
+
+from . import _ffi
+from .hp import nature2022
+
+
+class JpegBatch:
+    """n JPEG files back to back: tile i is data[offsets[i]:offsets[i + 1]].
+
+    data: 1-D uint8 numpy array (host) or contiguous CUDA torch uint8 tensor (read in place on the GPU);
+    offsets: n + 1 non-decreasing int64 byte offsets (host)."""
+
+    def __init__(self, data, offsets):
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        if offsets.ndim != 1 or offsets.size < 1:
+            raise ValueError("offsets must be a 1-D array of n + 1 byte offsets")
+        if isinstance(data, (bytes, bytearray, memoryview)):
+            data = np.frombuffer(data, np.uint8)
+        if isinstance(data, np.ndarray):
+            data = np.ascontiguousarray(data.reshape(-1), dtype=np.uint8)
+        else:
+            if str(getattr(data, "dtype", "")) != "torch.uint8" or data.dim() != 1 or not data.is_contiguous():
+                raise TypeError("data must be a 1-D uint8 numpy array or a contiguous 1-D torch.uint8 tensor")
+        size = int(data.shape[0])
+        if offsets[0] < 0 or np.any(np.diff(offsets) < 0) or offsets[-1] > size:
+            raise ValueError("offsets must be non-decreasing and lie within data")
+        self.data = data
+        self.offsets = offsets
+
+    @classmethod
+    def from_bytes(cls, items) -> "JpegBatch":
+        """from a list of encoded files (bytes)"""
+        items = [bytes(b) for b in items]
+        offsets = np.zeros(len(items) + 1, np.int64)
+        offsets[1:] = np.cumsum([len(b) for b in items])
+        return cls(np.frombuffer(b"".join(items), np.uint8).copy(), offsets)
+
+    def __len__(self) -> int:
+        return int(self.offsets.size - 1)
+
+    @property
+    def nbytes(self) -> int:
+        return int(self.offsets[-1] - self.offsets[0])
+
+    @property
+    def on_device(self) -> bool:
+        return not isinstance(self.data, np.ndarray)
+
+    def tile(self, i: int) -> bytes:
+        a, b = int(self.offsets[i]), int(self.offsets[i + 1])
+        chunk = self.data[a:b]
+        return bytes(chunk.cpu().numpy()) if self.on_device else chunk.tobytes()
+
+    def cuda(self, device: int | None = None) -> "JpegBatch":
+        """the same batch with its bytes in device memory"""
+        import torch
+        return JpegBatch(torch.from_numpy(np.asarray(self.data)).cuda(device), self.offsets)
+
+
+def status_message(code: int) -> str:
+    return _ffi.load_library().bq_jpeg_status_string(int(code)).decode()
+
+
+def inspect(batch: JpegBatch, px: int = nature2022.tile_px) -> np.ndarray:
+    """Host marker parse of every tile, no GPU needed: int32 status per tile (0 = accepted, else a BQ_JPEG_* code,
+    see `status_message`)."""
+    if batch.on_device:
+        raise ValueError("inspect reads host bytes; the batch is in device memory")
+    lib = _ffi.load_library()
+    st = np.zeros(len(batch), np.int32)
+    rc = lib.bq_jpeg_inspect(_ffi.ptr(batch.data), _ffi.ptr(batch.offsets), len(batch), int(px), _ffi.ptr(st))
+    if rc != 0:
+        raise ValueError("bq_jpeg_inspect: bad argument")
+    return st
+
+
+def check(batch: JpegBatch, px: int = nature2022.tile_px) -> None:
+    """raise ValueError for the first tile `decode` would reject by its headers"""
+    st = inspect(batch, px)
+    bad = np.flatnonzero(st)
+    if bad.size:
+        raise ValueError(f"JPEG tile {int(bad[0])}: {status_message(int(st[bad[0]]))}")
+
+
+def decode(batch: JpegBatch, px: int = nature2022.tile_px, ctx: _ffi.Context | None = None, out=None):
+    """uint8 NHWC [n, px, px, 3] tiles decoded on the GPU.  `out` may be a preallocated numpy array or CUDA torch tensor
+    of that shape (device output stays on the device); default: a new numpy array."""
+    ctx = ctx or _ffi.default_context()
+    n = len(batch)
+    if out is None:
+        out = np.empty((n, px, px, 3), np.uint8)
+    if tuple(out.shape) != (n, px, px, 3) or str(out.dtype).replace("torch.", "") != "uint8":
+        raise ValueError(f"out must be uint8 of shape {(n, px, px, 3)}")
+    if isinstance(out, np.ndarray) and not out.flags.c_contiguous:
+        raise ValueError("out must be C-contiguous")
+    st = np.zeros(n, np.int32)
+    _ffi.check(ctx.handle, ctx.lib.bq_jpeg_decode(ctx.handle, _ffi.ptr(batch.data), _ffi.ptr(batch.offsets), n, int(px),
+                                                  _ffi.ptr(out), _ffi.ptr(st)), "bq_jpeg_decode")
+    return out
+
+
+def last_stats(ctx: _ffi.Context | None = None) -> dict:
+    """subsequence statistics of the last `decode` on ctx"""
+    ctx = ctx or _ffi.default_context()
+    s = (C.c_int64 * 4)()
+    _ffi.check(ctx.handle, ctx.lib.bq_jpeg_last_stats(ctx.handle, s), "bq_jpeg_last_stats")
+    return dict(tiles=int(s[0]), subsequences=int(s[1]), max_sync_rounds=int(s[2]), redecoded=int(s[3]))

@@ -33,7 +33,8 @@ enum {
   BQ_ERR_ARG = -2,       /* bad argument (null pointer, negative size, bad enum)  */
   BQ_ERR_STATE = -3,     /* call order violated (e.g. predict before weights)     */
   BQ_ERR_WEIGHTS = -4,   /* missing / mis-shaped weight tensor                    */
-  BQ_ERR_NOMEM = -5
+  BQ_ERR_NOMEM = -5,
+  BQ_ERR_DATA = -6       /* malformed input data (a JPEG tile or TFRecord file)   */
 };
 
 enum { BQ_F32 = 0, BQ_F64 = 1 };
@@ -252,6 +253,72 @@ int bq_stain_normalize(bq_ctx* ctx, int32_t kind, const uint8_t* tiles, int64_t 
                        float* lab_stats);
 /* Make bq_predict_uq normalise every tile first (kind = BQ_NORM_NONE switches it off again). */
 int bq_model_set_normalizer(bq_model* m, int32_t kind, const float target_means[3], const float target_stds[3]);
+
+/* ------------------------------------------------------------------------------------------------
+ * compressed tiles: baseline JPEG decode on the GPU and TFRecord reading
+ *   replaces the host side of Slideflow's evaluate route (TFRecord read + per-tile JPEG decode in front of
+ *   interface(batch)).  Decoded pixels equal libjpeg-turbo's default decompression byte for byte (JDCT_ISLOW,
+ *   fancy upsampling, jdcolor.c YCbCr->RGB), i.e. PIL.Image.open(...).convert("RGB").
+ *   Tiles are n JPEG files back to back: tile i = data[offsets[i], offsets[i + 1]); offsets is always host memory.
+ *   Accepted: SOF0 / SOF1 8-bit Huffman, one interleaved scan of 3 components (YCbCr), sampling 4:4:4, 4:2:2 or 4:2:0,
+ *   any DQT / DHT, restart intervals, APPn / COM segments (skipped), size px x px.
+ * ---------------------------------------------------------------------------------------------- */
+enum {
+  BQ_JPEG_OK = 0,
+  BQ_JPEG_NOT_JPEG = 1,            /* no SOI marker                                                  */
+  BQ_JPEG_TRUNCATED_HEADER = 2,    /* the file ends inside its headers                               */
+  BQ_JPEG_PROGRESSIVE = 3,
+  BQ_JPEG_ARITHMETIC = 4,
+  BQ_JPEG_LOSSLESS = 5,            /* lossless or hierarchical                                        */
+  BQ_JPEG_PRECISION = 6,           /* not 8-bit samples                                               */
+  BQ_JPEG_GRAYSCALE = 7,           /* 1 component                                                     */
+  BQ_JPEG_CMYK = 8,                /* 4 components                                                    */
+  BQ_JPEG_COMPONENTS = 9,          /* any other component count                                       */
+  BQ_JPEG_SIZE = 10,               /* width or height differs from px                                 */
+  BQ_JPEG_SAMPLING = 11,           /* sampling factors other than 4:4:4 / 4:2:2 / 4:2:0               */
+  BQ_JPEG_MISSING_DQT = 12,
+  BQ_JPEG_MISSING_DHT = 13,
+  BQ_JPEG_BAD_TABLE = 14,          /* malformed DQT / DHT                                             */
+  BQ_JPEG_BAD_HEADER = 15,         /* missing SOF / SOS / EOI, unexpected marker, bad scan parameters */
+  BQ_JPEG_COLORSPACE = 16,         /* 3 components that are not YCbCr (Adobe transform 0, RGB ids)    */
+  /* found on the device while decoding the entropy-coded segment */
+  BQ_JPEG_BAD_ENTROPY_MARKER = 20, /* a marker other than RSTn inside the scan, or wrong RSTn sequence  */
+  BQ_JPEG_INVALID_CODE = 21,       /* a Huffman code that is in no table                               */
+  BQ_JPEG_TRUNCATED_DATA = 22      /* the scan ends before its last MCU                                */
+};
+/* one line of text per status code above */
+const char* bq_jpeg_status_string(int32_t status);
+/* Host only, no device needed: the marker parse bq_jpeg_decode runs first.  status[i] = BQ_JPEG_* of tile i.
+ * data must be host memory.  Returns BQ_OK also when some tiles are rejected. */
+int bq_jpeg_inspect(const uint8_t* data, const int64_t* offsets, int64_t n, int32_t px, int32_t* status);
+/* Decode n tiles into out_u8 = uint8 NHWC [n, px, px, 3] (host or device); data host or device (device bytes are read
+ * in place).  status[i] (host, nullable) = BQ_JPEG_* of tile i.  A rejected header fails the call with BQ_ERR_DATA
+ * before anything is launched; an entropy-coded segment that runs out of bits or holds an invalid code fails it with
+ * BQ_ERR_DATA after the batch (the other tiles are decoded; the rejected tile's pixels are 0). */
+int bq_jpeg_decode(bq_ctx* ctx, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t px, uint8_t* out_u8,
+                   int32_t* status);
+/* Subsequence statistics of the last bq_jpeg_decode on ctx, summed over its tiles: {tiles, subsequences,
+ * synchronisation rounds (max over tiles), subsequences decoded again}. */
+int bq_jpeg_last_stats(bq_ctx* ctx, int64_t stats[4]);
+/* bq_predict_uq on JPEG tiles: same outputs, seeds and tile indices as bq_predict_uq on the decoded uint8 tiles.  The
+ * compressed bytes of micro-batch i + 1 are copied while micro-batch i runs; each is decoded on the GPU into the
+ * micro-batch buffer the uint8 path stages into. */
+int bq_predict_uq_jpeg(bq_model* m, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t T, uint64_t seed,
+                       uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std, float* features);
+
+/* TFRecord file (uncompressed) in a host buffer: record framing {u64 length, masked CRC32C of the length, payload,
+ * masked CRC32C of the payload}, both CRCs verified (SSE4.2 crc32 when the CPU has it), payload parsed as a
+ * tf.train.Example.  For each record r < capacity: image[2r..2r+1] = byte range [begin, end) of the first value of the
+ * bytes feature `image_key`, slide[2r..] = same for `slide_key` (-1, -1 when absent), loc[2r], loc[2r + 1] = first value
+ * of the int64 features `x_key`, `y_key` (INT64_MIN when absent).  *n_records = records in the buffer (may exceed
+ * capacity: call again with more room).  A bad CRC, a truncated record, a malformed Example, a record without
+ * `image_key` or a gzip / zlib-compressed file fail with BQ_ERR_DATA and a message in err (err_capacity bytes). */
+int bq_tfrecord_scan(const uint8_t* buf, int64_t len, const char* image_key, const char* slide_key, const char* x_key,
+                     const char* y_key, int64_t capacity, int64_t* n_records, int64_t* image, int64_t* slide,
+                     int64_t* loc, char* err, int64_t err_capacity);
+/* CRC32C (Castagnoli) of a host buffer, and TFRecord's masked form ((crc >> 15 | crc << 17) + 0xa282ead8) */
+uint32_t bq_crc32c(const uint8_t* buf, int64_t len);
+uint32_t bq_crc32c_masked(const uint8_t* buf, int64_t len);
 
 /* ------------------------------------------------------------------------------------------------
  * evaluation metrics next to the path
