@@ -103,6 +103,11 @@ SIGNATURES = {
     "bq_jpeg_last_stats": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64)]),
     "bq_predict_uq_jpeg": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_uint64, C.c_uint64,
                                      C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "bq_png_status_string": (C.c_char_p, [C.c_int32]),
+    "bq_png_inspect": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p]),
+    "bq_png_decode": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]),
+    "bq_predict_uq_png": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_uint64, C.c_uint64,
+                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "bq_tfrecord_scan": (C.c_int, [C.c_void_p, C.c_int64, C.c_char_p, C.c_char_p, C.c_char_p, C.c_char_p, C.c_int64,
                                    C.POINTER(C.c_int64), C.c_void_p, C.c_void_p, C.c_void_p, C.c_char_p, C.c_int64]),
     "bq_crc32c": (C.c_uint32, [C.c_void_p, C.c_int64]),

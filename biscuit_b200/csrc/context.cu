@@ -67,6 +67,7 @@ void bq_destroy(bq_ctx* ctx) {
   }
   if (ctx->scratch) cudaFree(ctx->scratch);
   bq_jpeg_state_destroy(ctx->jpeg);
+  bq_png_state_destroy(ctx->png);
   if (ctx->pinned) cudaFreeHost(ctx->pinned);
   delete ctx;
 }

@@ -261,9 +261,7 @@ int bq_jpeg_prepare(bq_ctx* ctx, bq_jpeg_state*& s, const uint8_t* data, const i
     if ((rc = bq_alloc(ctx, s->offs_dev, (size_t)(n + 1) * 8)) || (rc = bq_alloc(ctx, s->heads, (size_t)n * (kHead + 2))))
       return rc;
     BQ_CUDA(ctx, cudaMemcpyAsync(s->offs_dev.p, offsets, (size_t)(n + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
-    bq::jpeg::jpeg_gather_heads_kernel<<<(unsigned)n, 256, 0, ctx->stream>>>(data, (const int64_t*)s->offs_dev.p, kHead,
-                                                                             (uint8_t*)s->heads.p);
-    BQ_LAUNCH_CHECK(ctx);
+    if ((rc = bq_gather_heads(ctx, data, (const int64_t*)s->offs_dev.p, n, kHead, (uint8_t*)s->heads.p))) return rc;
     std::vector<uint8_t> heads((size_t)n * (kHead + 2)), whole;
     BQ_CUDA(ctx, cudaMemcpyAsync(heads.data(), s->heads.p, heads.size(), cudaMemcpyDeviceToHost, ctx->stream));
     BQ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
@@ -323,6 +321,12 @@ int bq_jpeg_prepare(bq_ctx* ctx, bq_jpeg_state*& s, const uint8_t* data, const i
 }
 
 int64_t bq_jpeg_group_count(const bq_jpeg_state* s) { return n_groups(s); }
+
+int bq_gather_heads(bq_ctx* ctx, const uint8_t* data, const int64_t* offsets_dev, int64_t n, int head, uint8_t* out) {
+  bq::jpeg::jpeg_gather_heads_kernel<<<(unsigned)n, 256, 0, ctx->stream>>>(data, offsets_dev, head, out);
+  BQ_LAUNCH_CHECK(ctx);
+  return BQ_OK;
+}
 
 // Copy group g's descriptors (and its bytes, when they are in host memory) into slot `slot` on `stream`.
 int bq_jpeg_upload(bq_ctx* ctx, bq_jpeg_state* s, int64_t g, int slot, cudaStream_t stream) {

@@ -264,6 +264,7 @@ struct bq_model {
   cudaStream_t copy_stream = nullptr;          // H2D of micro-batch i+1 overlaps the backbone of micro-batch i
   cudaEvent_t copied[2] = {}, consumed[2] = {};
   bq_jpeg_state* jpeg = nullptr;               // bq_predict_uq_jpeg: descriptors, compressed staging and decode scratch
+  bq_png_state* png = nullptr;                 // bq_predict_uq_png: likewise
   DevBuf mean, inv_std;                        // fp32 [max_batch]
   Arena arena;
   DevBuf feat, feat_bf16;                      // [max_batch, 2048]
@@ -968,6 +969,7 @@ void bq_model_destroy(bq_model* m) {
   if (m->copy_stream) { cudaStreamSynchronize(m->copy_stream); cudaStreamDestroy(m->copy_stream); }
   for (int i = 0; i < 2; ++i) { if (m->copied[i]) cudaEventDestroy(m->copied[i]); if (m->consumed[i]) cudaEventDestroy(m->consumed[i]); }
   bq_jpeg_state_destroy(m->jpeg);
+  bq_png_state_destroy(m->png);
   delete m;
 }
 
@@ -1081,35 +1083,46 @@ int bq_model_load_weights(bq_model* m, const bq_named_tensor* tensors, int32_t n
   return BQ_OK;
 }
 
-static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, const int64_t* jpeg_offsets, int64_t n,
-                        int32_t T, uint64_t seed, uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std,
-                        float* features);
+// Input of predict_impl: decoded pixels, or n compressed files back to back with n + 1 host byte offsets.
+enum class Encoding { kPixels, kJpeg, kPng };
+
+static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, Encoding enc, const int64_t* offsets,
+                        int64_t n, int32_t T, uint64_t seed, uint64_t tile_index_base, const uint8_t* masks, float* mean,
+                        float* std, float* features);
 
 int bq_predict_uq(bq_model* m, const uint8_t* tiles, int64_t n, int32_t T, uint64_t seed, uint64_t tile_index_base,
                   const uint8_t* masks, float* mean, float* std, float* features) {
-  return predict_impl(m, tiles, false, nullptr, n, T, seed, tile_index_base, masks, mean, std, features);
+  return predict_impl(m, tiles, false, Encoding::kPixels, nullptr, n, T, seed, tile_index_base, masks, mean, std,
+                      features);
 }
 
 int bq_predict_uq_jpeg(bq_model* m, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t T, uint64_t seed,
                        uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std, float* features) {
   if (!m) return BQ_ERR_ARG;
   if (n > 0 && !offsets) return bq_fail(m->ctx, BQ_ERR_ARG, "bq_predict_uq_jpeg: offsets must not be NULL");
-  return predict_impl(m, data, false, offsets, n, T, seed, tile_index_base, masks, mean, std, features);
+  return predict_impl(m, data, false, Encoding::kJpeg, offsets, n, T, seed, tile_index_base, masks, mean, std, features);
+}
+
+int bq_predict_uq_png(bq_model* m, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t T, uint64_t seed,
+                      uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std, float* features) {
+  if (!m) return BQ_ERR_ARG;
+  if (n > 0 && !offsets) return bq_fail(m->ctx, BQ_ERR_ARG, "bq_predict_uq_png: offsets must not be NULL");
+  return predict_impl(m, data, false, Encoding::kPng, offsets, n, T, seed, tile_index_base, masks, mean, std, features);
 }
 
 int bq_predict_uq_standardized(bq_model* m, const float* tiles, int64_t n, int32_t T, uint64_t seed, uint64_t tile_index_base,
                                const uint8_t* masks, float* mean, float* std, float* features) {
   if (!m) return BQ_ERR_ARG;
   m->input_f32 = true;
-  const int rc = predict_impl(m, (const uint8_t*)tiles, true, nullptr, n, T, seed, tile_index_base, masks, mean, std,
-                              features);
+  const int rc = predict_impl(m, (const uint8_t*)tiles, true, Encoding::kPixels, nullptr, n, T, seed, tile_index_base,
+                              masks, mean, std, features);
   m->input_f32 = false;
   return rc;
 }
 
-static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, const int64_t* jpeg_offsets, int64_t n,
-                        int32_t T, uint64_t seed, uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std,
-                        float* features) {
+static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, Encoding enc, const int64_t* offsets,
+                        int64_t n, int32_t T, uint64_t seed, uint64_t tile_index_base, const uint8_t* masks, float* mean,
+                        float* std, float* features) {
   if (!m) return BQ_ERR_ARG;
   bq_ctx* ctx = m->ctx;
   if (!m->weights_loaded) return bq_fail(ctx, BQ_ERR_STATE, "bq_predict_uq: weights not loaded");
@@ -1130,15 +1143,16 @@ static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, const
   if (m->profiling == 2)
     for (int k = 0; k < BQ_PROFILE_KINDS; ++k) { m->k_ms[k] = m->k_flops[k] = m->k_bytes[k] = 0; m->k_launches[k] = 0; }
   // Host tiles: double-buffered staging, the H2D copy of micro-batch i+1 runs on its own stream while the
-  // backbone of micro-batch i computes.  Device tiles are read in place.  JPEG tiles always take the staged route:
-  // micro-batch i + 1's descriptors (and its compressed bytes, unless they are device memory, which is read in place)
-  // go up on the copy stream, and micro-batch i is decoded on the ctx stream into tiles_dev.
-  const bool jpeg = jpeg_offsets != nullptr;
-  if (jpeg) {
-    const int rcj = bq_jpeg_prepare(ctx, m->jpeg, tiles, jpeg_offsets, n, m->px, B, nullptr);
+  // backbone of micro-batch i computes.  Device tiles are read in place.  Compressed (JPEG / PNG) tiles always take
+  // the staged route: micro-batch i + 1's descriptors (and its compressed bytes, unless they are device memory, which
+  // is read in place) go up on the copy stream, and micro-batch i is decoded on the ctx stream into tiles_dev.
+  const bool compressed = enc != Encoding::kPixels;
+  if (compressed) {
+    const int rcj = enc == Encoding::kJpeg ? bq_jpeg_prepare(ctx, m->jpeg, tiles, offsets, n, m->px, B, nullptr)
+                                           : bq_png_prepare(ctx, m->png, tiles, offsets, n, m->px, B, nullptr);
     if (rcj) return rcj;
   }
-  const bool tiles_on_dev = !jpeg && bq_is_device_ptr(tiles);
+  const bool tiles_on_dev = !compressed && bq_is_device_ptr(tiles);
   if (f32_input && !tiles_on_dev) {
     const int64_t cap = n < B ? n : B;                      // the interface is usually called tile by tile (results.py:249-257)
     for (auto& b : m->tiles_f32) { int rcf = bq_alloc(ctx, b, (size_t)cap * tile_bytes + 64); if (rcf) return rcf; }
@@ -1147,8 +1161,9 @@ static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, const
   auto issue_copy = [&](int64_t i0c, int slot) -> int {
     const int nbc = (int)((n - i0c < B) ? (n - i0c) : B);
     BQ_CUDA(ctx, cudaStreamWaitEvent(m->copy_stream, m->consumed[slot], 0));   // previous reader of this slot done
-    if (jpeg) {
-      const int rcu = bq_jpeg_upload(ctx, m->jpeg, i0c / B, slot, m->copy_stream);
+    if (compressed) {
+      const int rcu = enc == Encoding::kJpeg ? bq_jpeg_upload(ctx, m->jpeg, i0c / B, slot, m->copy_stream)
+                                             : bq_png_upload(ctx, m->png, i0c / B, slot, m->copy_stream);
       if (rcu) return rcu;
     } else {
       BQ_CUDA(ctx, cudaMemcpyAsync(stage[slot], tiles + (size_t)i0c * tile_bytes, (size_t)nbc * tile_bytes,
@@ -1171,8 +1186,10 @@ static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, const
     } else {
       BQ_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, m->copied[slot], 0));
       m->tiles_src = stage[slot];
-      if (jpeg) {
-        if ((rc = bq_jpeg_decode_group(ctx, m->jpeg, batch_idx, slot, (uint8_t*)m->tiles_dev.p))) return rc;
+      if (compressed) {
+        rc = enc == Encoding::kJpeg ? bq_jpeg_decode_group(ctx, m->jpeg, batch_idx, slot, (uint8_t*)m->tiles_dev.p)
+                                    : bq_png_decode_group(ctx, m->png, batch_idx, slot, (uint8_t*)m->tiles_dev.p);
+        if (rc) return rc;
         BQ_CUDA(ctx, cudaEventRecord(m->consumed[slot], ctx->stream));        // the compressed slot is free once decoded
         m->tiles_src = (const uint8_t*)m->tiles_dev.p;
       }
@@ -1195,7 +1212,7 @@ static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, const
     }
     if ((rc = run_backbone_graphed(m, nb))) return rc;
     if (!tiles_on_dev) {
-      if (!jpeg) BQ_CUDA(ctx, cudaEventRecord(m->consumed[slot], ctx->stream));
+      if (!compressed) BQ_CUDA(ctx, cudaEventRecord(m->consumed[slot], ctx->stream));
       // The next micro-batch's copy is issued AFTER this one's backbone is queued: a copy from PAGEABLE memory blocks the
       // calling thread while the driver stages it, and that time must fall under queued GPU work (from pinned memory the
       // call returns at once and the order makes no difference).
@@ -1233,7 +1250,7 @@ static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, const
     }
   }
   BQ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  if (jpeg) return bq_jpeg_finish(ctx, m->jpeg, nullptr);
+  if (compressed) return enc == Encoding::kJpeg ? bq_jpeg_finish(ctx, m->jpeg, nullptr) : bq_png_finish(ctx, m->png, nullptr);
   return BQ_OK;
 }
 

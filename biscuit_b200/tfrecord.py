@@ -1,9 +1,9 @@
 """Slideflow tile TFRecords read without TensorFlow (csrc/tfrecord.cu).
 
-Each record is a `tf.train.Example` holding one JPEG tile and where it came from.  `read(paths)` verifies both CRCs of
-every record and returns the tiles as one `jpeg.JpegBatch` (decoded on the GPU by `predict` / `jpeg.decode`) with the
-slide name and tile location of each.  The feature keys default to Slideflow's (`image_raw`, `slide`, `loc_x`,
-`loc_y`).  Compressed (gzip / zlib) record files are rejected: decompress them first.
+Each record is a `tf.train.Example` holding one JPEG or PNG tile and where it came from.  `read(paths)` verifies both
+CRCs of every record and returns the tiles as one `jpeg.JpegBatch` or `png.PngBatch` (decoded on the GPU by `predict` /
+`jpeg.decode` / `png.decode`) with the slide name and tile location of each.  The feature keys default to Slideflow's
+(`image_raw`, `slide`, `loc_x`, `loc_y`).  Compressed (gzip / zlib) record files are rejected: decompress them first.
 """
 from __future__ import annotations
 
@@ -14,6 +14,8 @@ import numpy as np
 
 from . import _ffi
 from .jpeg import JpegBatch
+from .png import SIGNATURE as PNG_SIGNATURE
+from .png import PngBatch
 
 LOC_MISSING = np.iinfo(np.int64).min
 
@@ -43,16 +45,27 @@ def scan(buf, image_key="image_raw", slide_key="slide", x_key="loc_x", y_key="lo
 
 
 def read(paths, image_key="image_raw", slide_key="slide", x_key="loc_x", y_key="loc_y"):
-    """(JpegBatch, slides, loc_x, loc_y) over the records of `paths` (one path or a list), in file order.
-    slides: list of str (UTF-8); loc_x / loc_y: int64 arrays."""
+    """(batch, slides, loc_x, loc_y) over the records of `paths` (one path or a list), in file order.
+    batch: a PngBatch when every image starts with the PNG signature, else a JpegBatch (whatever is not JPEG then fails
+    in the JPEG decoder, naming the tile).  A set that mixes PNG with other images raises ValueError naming the first
+    record (file, index in the file) whose format differs from record 0.  slides: list of str (UTF-8); loc_x / loc_y:
+    int64 arrays."""
     if isinstance(paths, (str, os.PathLike)):
         paths = [paths]
     parts, sizes, slides, locs = [], [], [], []
+    first_png = None
     for p in paths:
         with open(p, "rb") as f:
             buf = np.frombuffer(f.read(), np.uint8)
         image, slide, loc = scan(buf, image_key, slide_key, x_key, y_key)
-        for (a, b), (sa, sb) in zip(image, slide):
+        for r, ((a, b), (sa, sb)) in enumerate(zip(image, slide)):
+            is_png = buf[a:min(b, a + len(PNG_SIGNATURE))].tobytes() == PNG_SIGNATURE
+            if first_png is None:
+                first_png = is_png
+            elif is_png != first_png:
+                kinds = ("PNG", "not PNG") if first_png else ("not PNG", "PNG")
+                raise ValueError(f"{os.fspath(p)} record {r}: image is {kinds[1]} but the first record's is {kinds[0]}; "
+                                 "a record set must hold one image format")
             parts.append(buf[a:b])
             sizes.append(b - a)
             slides.append(buf[sa:sb].tobytes().decode("utf-8") if sa >= 0 else "")
@@ -61,7 +74,7 @@ def read(paths, image_key="image_raw", slide_key="slide", x_key="loc_x", y_key="
     offsets[1:] = np.cumsum(sizes)
     data = np.concatenate(parts) if parts else np.zeros(0, np.uint8)
     loc = np.concatenate(locs) if locs else np.zeros((0, 2), np.int64)
-    return JpegBatch(data, offsets), slides, loc[:, 0].copy(), loc[:, 1].copy()
+    return (PngBatch if first_png else JpegBatch)(data, offsets), slides, loc[:, 0].copy(), loc[:, 1].copy()
 
 
 def crc32c(b) -> int:

@@ -25,6 +25,7 @@ import pandas as pd
 from . import _ffi
 from .hp import ModelConfig, nature2022
 from .jpeg import JpegBatch
+from .png import PngBatch
 from .utils import uncertainty_header, y_pred_header, y_true_header
 
 FEATURES = 2048
@@ -124,17 +125,18 @@ class UncertaintyInterface:
                 masks=None, return_features: bool = False, out_mean=None, out_std=None):
         """tiles: NHWC [n, 299, 299, 3] -- uint8 raw RGB (decode + per-image standardisation fused into the first
         convolution), or float32 ALREADY passed through `tf.image.per_image_standardization` as the reference's call site
-        does (results.py:255-257); numpy, or a CUDA torch tensor used in place.  Or a `jpeg.JpegBatch` of JPEG tiles,
-        decoded on the GPU in front of the backbone: the results equal `predict` on the decoded uint8 tiles bit for bit.
+        does (results.py:255-257); numpy, or a CUDA torch tensor used in place.  Or a `jpeg.JpegBatch` / `png.PngBatch`
+        of JPEG / PNG tiles, decoded on the GPU in front of the backbone: the results equal `predict` on the decoded
+        uint8 tiles bit for bit.
         Returns (mean [n, C], std [n, C]) float32 -- population std over T dropout samples."""
         T = int(T or self.num_uq)
-        jpeg = isinstance(tiles, JpegBatch)
-        n = len(tiles) if jpeg else int(tiles.shape[0])
+        encoded = {JpegBatch: "jpeg", PngBatch: "png"}.get(type(tiles))
+        n = len(tiles) if encoded else int(tiles.shape[0])
         px = self.config.tile_px
-        if not jpeg and tuple(tiles.shape[1:]) != (px, px, 3):
+        if not encoded and tuple(tiles.shape[1:]) != (px, px, 3):
             raise ValueError(f"tiles must be [n, {px}, {px}, 3], got {tuple(tiles.shape)}")
-        dt = "jpeg" if jpeg else str(tiles.dtype).replace("torch.", "")
-        if dt not in ("uint8", "float32", "jpeg"):
+        dt = encoded or str(tiles.dtype).replace("torch.", "")
+        if dt not in ("uint8", "float32", "jpeg", "png"):
             raise TypeError("tiles must be uint8 (raw RGB) or float32 (already per-image standardised), got " + dt)
         if isinstance(tiles, np.ndarray):
             tiles = np.ascontiguousarray(tiles)
@@ -155,10 +157,10 @@ class UncertaintyInterface:
                 raise ValueError(f"masks must have shape {want}")
             if isinstance(masks, np.ndarray):
                 masks = np.ascontiguousarray(masks, dtype=np.uint8)
-        if jpeg:
-            rc = self.lib.bq_predict_uq_jpeg(self.h, _ffi.ptr(tiles.data), _ffi.ptr(tiles.offsets), n, T, C.c_uint64(seed),
-                                             C.c_uint64(tile_index_base), _ffi.ptr(masks), _ffi.ptr(mean), _ffi.ptr(std),
-                                             _ffi.ptr(feats))
+        if encoded:
+            entry = self.lib.bq_predict_uq_jpeg if encoded == "jpeg" else self.lib.bq_predict_uq_png
+            rc = entry(self.h, _ffi.ptr(tiles.data), _ffi.ptr(tiles.offsets), n, T, C.c_uint64(seed),
+                       C.c_uint64(tile_index_base), _ffi.ptr(masks), _ffi.ptr(mean), _ffi.ptr(std), _ffi.ptr(feats))
         else:
             entry = self.lib.bq_predict_uq if dt == "uint8" else self.lib.bq_predict_uq_standardized
             rc = entry(self.h, _ffi.ptr(tiles), n, T, C.c_uint64(seed), C.c_uint64(tile_index_base), _ffi.ptr(masks),
@@ -172,7 +174,7 @@ class UncertaintyInterface:
         """`logits, uncertainty = interface(batch)` (results.py:257): mean softmax [B, C] and the per-class std
         [B, C] over the dropout samples, so the reference's `uncertainty[0][0]` (results.py:258) reads the class-0 std --
         for two classes both stds agree up to rounding.  `batch` may be the standardised float32 batch the reference
-        passes, raw uint8 tiles, or a `jpeg.JpegBatch`."""
+        passes, raw uint8 tiles, a `jpeg.JpegBatch` or a `png.PngBatch`."""
         return self.predict(tiles, **kw)
 
     # ------------------------------------------------------------------------------------
@@ -248,8 +250,8 @@ def predict_table(interface: UncertaintyInterface, tiles, slides, y_true=None, o
 
 def predict_tfrecords(interface: UncertaintyInterface, paths, y_true=None, outcome="cohort", T: int | None = None,
                       seed: int = 0, renamed: bool = True, **keys):
-    """`predict_table` straight from Slideflow tile TFRecords: the records of `paths` in file order, JPEG tiles decoded
-    on the GPU.  Tile indices of the dropout streams run across files, so the table equals one `predict_table` over all
+    """`predict_table` straight from Slideflow tile TFRecords: the records of `paths` in file order, JPEG or PNG tiles
+    decoded on the GPU.  Tile indices of the dropout streams run across files, so the table equals one `predict_table` over all
     tiles.  y_true: per-tile labels, or a dict slide -> label.  Adds the `loc_x` / `loc_y` columns of each tile.
     `keys` overrides the feature names (`image_key`, `slide_key`, `x_key`, `y_key`; see `tfrecord.read`)."""
     from . import tfrecord

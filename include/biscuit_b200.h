@@ -34,7 +34,7 @@ enum {
   BQ_ERR_STATE = -3,     /* call order violated (e.g. predict before weights)     */
   BQ_ERR_WEIGHTS = -4,   /* missing / mis-shaped weight tensor                    */
   BQ_ERR_NOMEM = -5,
-  BQ_ERR_DATA = -6       /* malformed input data (a JPEG tile or TFRecord file)   */
+  BQ_ERR_DATA = -6       /* malformed input data (a JPEG / PNG tile, a TFRecord)  */
 };
 
 enum { BQ_F32 = 0, BQ_F64 = 1 };
@@ -305,6 +305,50 @@ int bq_jpeg_last_stats(bq_ctx* ctx, int64_t stats[4]);
  * micro-batch buffer the uint8 path stages into. */
 int bq_predict_uq_jpeg(bq_model* m, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t T, uint64_t seed,
                        uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std, float* features);
+
+/* PNG tiles, decoded on the GPU: the pixels equal PIL.Image.open(...).convert("RGB") (PNG is lossless, so also
+ * TensorFlow's decode_png).  Same layout as the JPEG entry points: tile i = data[offsets[i], offsets[i + 1]), offsets
+ * in host memory.  Accepted: 8-bit RGB (colour type 2), non-interlaced, px x px, any zlib level / strategy / window,
+ * IDAT split into chunks of any size, ancillary chunks and PLTE (skipped).  Every chunk before the first IDAT must pass
+ * its CRC; IDAT CRCs are not checked (the zlib Adler-32 is). */
+enum {
+  BQ_PNG_OK = 0,
+  BQ_PNG_NOT_PNG = 1,              /* no PNG signature                                                */
+  BQ_PNG_TRUNCATED_HEADER = 2,     /* the file ends before the first IDAT and the zlib header          */
+  BQ_PNG_BAD_CRC = 3,              /* a chunk before the first IDAT fails its CRC                       */
+  BQ_PNG_BAD_IHDR = 4,             /* IHDR missing / not first / length != 13 / invalid field / twice   */
+  BQ_PNG_SIZE = 5,                 /* width or height differs from px                                  */
+  BQ_PNG_BIT_DEPTH = 6,            /* not 8 bits per sample                                            */
+  BQ_PNG_COLOUR_TYPE = 7,          /* grayscale, palette or alpha                                      */
+  BQ_PNG_INTERLACED = 8,           /* Adam7                                                            */
+  BQ_PNG_UNKNOWN_CRITICAL = 9,     /* a critical chunk other than IHDR / PLTE / IDAT / IEND            */
+  BQ_PNG_NO_IDAT = 10,             /* IEND before any IDAT                                             */
+  BQ_PNG_BAD_ZLIB = 11,            /* zlib header: CM != 8, CINFO > 7 or bad FCHECK                    */
+  BQ_PNG_PRESET_DICT = 12,         /* zlib FDICT set                                                   */
+  /* found on the device */
+  BQ_PNG_TRUNCATED_DATA = 20,      /* the IDAT run or the DEFLATE stream ends early, or no Adler-32    */
+  BQ_PNG_BAD_BLOCK = 21,           /* BTYPE 3, or a stored block with LEN != ~NLEN                     */
+  BQ_PNG_BAD_HUFFMAN = 22,         /* over-subscribed / incomplete code, bad repeat, invalid symbol    */
+  BQ_PNG_BAD_DISTANCE = 23,        /* a match reaching before the start of the stream                  */
+  BQ_PNG_WRONG_SIZE = 24,          /* decompressed size != px * (1 + 3 px)                             */
+  BQ_PNG_ADLER = 25,               /* Adler-32 mismatch                                                */
+  BQ_PNG_BAD_FILTER = 26           /* a row filter type > 4                                            */
+};
+/* one line of text per status code above */
+const char* bq_png_status_string(int32_t status);
+/* Host only, no device needed: the chunk parse bq_png_decode runs first.  status[i] = BQ_PNG_* of tile i.  data must
+ * be host memory.  Returns BQ_OK also when some tiles are rejected. */
+int bq_png_inspect(const uint8_t* data, const int64_t* offsets, int64_t n, int32_t px, int32_t* status);
+/* Decode n tiles into out_u8 = uint8 NHWC [n, px, px, 3] (host or device); data host or device (device bytes are read
+ * in place).  status[i] (host, nullable) = BQ_PNG_* of tile i.  A rejected header fails the call with BQ_ERR_DATA
+ * before anything is launched; a tile rejected on the device fails it with BQ_ERR_DATA after the batch (the other
+ * tiles are decoded).  Stricter than Pillow on corrupt data: a missing Adler-32 and a stream that decompresses to
+ * more bytes than the image are rejected. */
+int bq_png_decode(bq_ctx* ctx, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t px, uint8_t* out_u8,
+                  int32_t* status);
+/* bq_predict_uq on PNG tiles: same outputs, seeds and tile indices as bq_predict_uq on the decoded uint8 tiles. */
+int bq_predict_uq_png(bq_model* m, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t T, uint64_t seed,
+                      uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std, float* features);
 
 /* TFRecord file (uncompressed) in a host buffer: record framing {u64 length, masked CRC32C of the length, payload,
  * masked CRC32C of the payload}, both CRCs verified (SSE4.2 crc32 when the CPU has it), payload parsed as a
