@@ -1,4 +1,5 @@
-// Shared host-side plumbing of libbiscuit_b200: context, error reporting, device buffers, staging.
+// Shared host-side plumbing of libbiscuit_b200: context, error reporting, device buffers, staging.  The compressed-tile
+// states a context keeps per format are declared in encoded.cuh.
 #pragma once
 
 #include <cuda_runtime.h>
@@ -12,8 +13,7 @@
 
 #include "../../include/biscuit_b200.h"
 
-struct bq_jpeg_state;   // jpeg.cu
-struct bq_png_state;    // png.cu
+struct bq_encoded;      // encoded.cuh
 
 struct bq_ctx {
   int device = 0;
@@ -27,35 +27,9 @@ struct bq_ctx {
   // small pinned mailbox for scalar results
   void* pinned = nullptr;
   size_t pinned_bytes = 0;
-  bq_jpeg_state* jpeg = nullptr;       // bq_jpeg_decode's descriptors and scratch (created on first use)
-  bq_png_state* png = nullptr;         // bq_png_decode's, likewise
+  bq_encoded* jpeg = nullptr;          // bq_jpeg_decode's descriptors and scratch (created on first use)
+  bq_encoded* png = nullptr;           // bq_png_decode's, likewise
 };
-
-// JPEG decode driver (jpeg.cu), shared by bq_jpeg_decode and bq_predict_uq_jpeg.  prepare parses every tile's headers
-// (failing with BQ_ERR_DATA before anything is launched) and splits the tiles into groups of `group`; upload copies a
-// group's descriptors (and its bytes, when they are host memory) into slot 0 / 1 on `stream`; decode_group runs the
-// four decode kernels on the ctx stream into `out` (device, uint8 NHWC); finish synchronises and fails with
-// BQ_ERR_DATA when a tile's entropy-coded data was rejected on the device.
-int bq_jpeg_prepare(bq_ctx* ctx, bq_jpeg_state*& s, const uint8_t* data, const int64_t* offsets, int64_t n, int px,
-                    int64_t group, int32_t* status_host);
-int64_t bq_jpeg_group_count(const bq_jpeg_state* s);
-int bq_jpeg_upload(bq_ctx* ctx, bq_jpeg_state* s, int64_t g, int slot, cudaStream_t stream);
-int bq_jpeg_decode_group(bq_ctx* ctx, bq_jpeg_state* s, int64_t g, int slot, uint8_t* out);
-int bq_jpeg_finish(bq_ctx* ctx, bq_jpeg_state* s, int32_t* status_host);
-void bq_jpeg_state_destroy(bq_jpeg_state* s);
-// Header bytes of n tiles resident on the device (offsets_dev: n + 1 device offsets): out[i * (head + 2) ...] = the first
-// `head` bytes of tile i (zero-padded), then its last two bytes.  Launched on the ctx stream.
-int bq_gather_heads(bq_ctx* ctx, const uint8_t* data, const int64_t* offsets_dev, int64_t n, int head, uint8_t* out);
-
-// PNG decode driver (png.cu), shared by bq_png_decode and bq_predict_uq_png, with the same four steps as the JPEG one;
-// decode_group runs the three PNG kernels.
-int bq_png_prepare(bq_ctx* ctx, bq_png_state*& s, const uint8_t* data, const int64_t* offsets, int64_t n, int px,
-                   int64_t group, int32_t* status_host);
-int64_t bq_png_group_count(const bq_png_state* s);
-int bq_png_upload(bq_ctx* ctx, bq_png_state* s, int64_t g, int slot, cudaStream_t stream);
-int bq_png_decode_group(bq_ctx* ctx, bq_png_state* s, int64_t g, int slot, uint8_t* out);
-int bq_png_finish(bq_ctx* ctx, bq_png_state* s, int32_t* status_host);
-void bq_png_state_destroy(bq_png_state* s);
 
 inline int bq_fail(bq_ctx* ctx, int code, const char* fmt, ...) {
   char buf[1024];

@@ -1,5 +1,5 @@
 // Context lifecycle of libbiscuit_b200 (one bq_ctx per GPU / host thread).
-#include "common.cuh"
+#include "encoded.cuh"
 
 static thread_local std::string g_create_error;
 
@@ -66,8 +66,8 @@ void bq_destroy(bq_ctx* ctx) {
     cudaStreamDestroy(ctx->stream);
   }
   if (ctx->scratch) cudaFree(ctx->scratch);
-  bq_jpeg_state_destroy(ctx->jpeg);
-  bq_png_state_destroy(ctx->png);
+  delete ctx->jpeg;
+  delete ctx->png;
   if (ctx->pinned) cudaFreeHost(ctx->pinned);
   delete ctx;
 }

@@ -1,12 +1,12 @@
-// Baseline-JPEG tiles on the GPU: host marker parse -> per-tile descriptors, staging, the four decode launches of
-// jpeg_sm100.cuh, and the bq_jpeg_* entry points.  bq_predict_uq_jpeg (model.cu) drives the same state per micro-batch.
+// Baseline-JPEG tiles on the GPU: the host marker parse into per-tile descriptors, the layout of their decode scratch
+// and the four decode launches of jpeg_sm100.cuh, driven by encoded.cu, and the bq_jpeg_* entry points.
 #include <cuda_runtime.h>
 
 #include <algorithm>
 #include <vector>
 
 #include "../../include/biscuit_b200.h"
-#include "common.cuh"
+#include "encoded.cuh"
 #include "jpeg_sm100.cuh"
 
 using bq::jpeg::Tile;
@@ -18,16 +18,14 @@ const uint8_t kNaturalHost[64] = {0,  1,  8,  16, 9,  2,  3,  10, 17, 24, 32, 25
                                   35, 42, 49, 56, 57, 50, 43, 36, 29, 22, 15, 23, 30, 37, 44, 51,
                                   58, 59, 52, 45, 38, 31, 39, 46, 53, 60, 61, 54, 47, 55, 62, 63};
 
-constexpr int kNeedMore = -1;
-
 // Marker parse of one file b[0, len) of which the first `avail` bytes are at hand (tail2 = its last two bytes).
-// Returns BQ_JPEG_* (t filled on BQ_JPEG_OK; t.seg_off relative to the file start) or kNeedMore.
+// Returns BQ_JPEG_* (t filled on BQ_JPEG_OK; t.seg_off relative to the file start) or bq_encoded::kNeedMore.
 int parse_tile(const uint8_t* b, int64_t len, int64_t avail, const uint8_t* tail2, int px, Tile& t) {
   memset(&t, 0, sizeof(t));
 #define NEED(k)                                        \
   do {                                                 \
     if ((int64_t)(k) > len) return BQ_JPEG_TRUNCATED_HEADER; \
-    if ((int64_t)(k) > avail) return kNeedMore;        \
+    if ((int64_t)(k) > avail) return bq_encoded::kNeedMore; \
   } while (0)
   NEED(2);
   if (b[0] != 0xFF || b[1] != 0xD8) return BQ_JPEG_NOT_JPEG;
@@ -198,244 +196,121 @@ const char* status_string(int32_t s) {
   }
 }
 
-}  // namespace
 
-// Decode state of one caller (the ctx's bq_jpeg_decode, or one model's bq_predict_uq_jpeg): descriptors of all tiles,
-// split into groups of at most `group` tiles that are staged and decoded one at a time; device scratch sized for the
-// largest group (grown on demand, never shrunk).
-struct bq_jpeg_state {
-  const uint8_t* data = nullptr;
-  bool on_dev = false;
-  int px = 0;
-  int64_t n = 0, group = 0;
-  std::vector<int64_t> offs;
-  Tile* desc_host = nullptr;           // pinned [n]
-  size_t desc_host_cap = 0;
-  DevBuf stage[2], desc[2];            // compressed bytes / descriptors of a group (double-buffered)
-  DevBuf ub, intv, ichunk, chunks, coef, planes, status, stats, heads, offs_dev;
-  size_t max_bytes = 0;
+// Decode state of one caller: the driver's, plus the JPEG decode scratch sized for the largest group.
+struct Jpeg final : bq_encoded {
+  DevBuf ub, intv, ichunk, chunks, coef, planes, stats;
   int64_t max_int = 0, max_chunks = 0, max_blocks = 0, max_tile_blocks = 0;
   int64_t last_stats[4] = {};
-  ~bq_jpeg_state() { if (desc_host) cudaFreeHost(desc_host); }
+
+  const char* name() const override { return "JPEG"; }
+  size_t desc_bytes() const override { return sizeof(Tile); }
+  int head_bytes() const override { return 2048; }
+  bool px_ok(int px) const override { return px >= 16 && px <= 4096; }
+  int parse(const uint8_t* b, int64_t len, int64_t avail, const uint8_t* tail2, int px, void* desc) const override {
+    return parse_tile(b, len, avail, tail2, px, *(Tile*)desc);
+  }
+  const char* status_string(int32_t code) const override { return ::status_string(code); }
+
+  // every base is relative to the group
+  int layout(bq_ctx* ctx) override {
+    Tile* tiles = (Tile*)desc_host;
+    max_int = max_chunks = max_blocks = max_tile_blocks = 0;
+    for (int64_t g = 0; g < n_groups(); ++g) {
+      const int64_t i0 = g * group, i1 = group_end(g);
+      int64_t ni = 0, nc = 0, nbk = 0;
+      for (int64_t i = i0; i < i1; ++i) {
+        Tile& t = tiles[i];
+        t.seg_off += offs[i] - offs[i0];
+        t.int_base = (int32_t)ni;
+        t.chunk_base = (int32_t)nc;
+        t.coef_base = nbk;
+        const int64_t blocks = (int64_t)t.mcux * t.mcuy * t.bpm;
+        ni += t.n_int + 1;
+        nc += t.chunk_cap;
+        nbk += blocks;
+        max_tile_blocks = std::max(max_tile_blocks, blocks);
+      }
+      if (nc > INT32_MAX || ni > INT32_MAX) return bq_fail(ctx, BQ_ERR_ARG, "bq_jpeg: group too large");
+      max_int = std::max(max_int, ni);
+      max_chunks = std::max(max_chunks, nc);
+      max_blocks = std::max(max_blocks, nbk);
+    }
+    const size_t pitch = bq_align_up((size_t)px, 16);
+    const int64_t gmax = std::min(n, group);
+    int rc;
+    if ((rc = bq_alloc(ctx, ub, max_bytes + 16)) || (rc = bq_alloc(ctx, intv, (size_t)max_int * 4)) ||
+        (rc = bq_alloc(ctx, ichunk, (size_t)max_int * 4)) ||
+        (rc = bq_alloc(ctx, chunks, (size_t)max_chunks * sizeof(bq::jpeg::Chunk))) ||
+        (rc = bq_alloc(ctx, coef, (size_t)max_blocks * 128)) ||
+        (rc = bq_alloc(ctx, planes, (size_t)gmax * 3 * pitch * pitch)) ||
+        (rc = bq_alloc(ctx, stats, (size_t)std::max<int64_t>(n, 1) * 12)))
+      return rc;
+    return BQ_OK;
+  }
+
+  int launch(bq_ctx* ctx, int64_t i0, int nb, const uint8_t* src, const void* desc_dev, int32_t* status,
+             uint8_t* out) override {
+    namespace J = bq::jpeg;
+    const int pitch = (int)bq_align_up((size_t)px, 16);
+    const Tile* d = (const Tile*)desc_dev;
+    const Tile* tiles = (const Tile*)desc_host;
+    int32_t* st = (int32_t*)stats.p + 3 * i0;
+    int64_t blocks = 0;
+    for (int64_t i = i0; i < i0 + nb; ++i) blocks += (int64_t)tiles[i].mcux * tiles[i].mcuy * tiles[i].bpm;
+    BQ_CUDA(ctx, cudaMemsetAsync(st, 0, (size_t)nb * 12, ctx->stream));
+    BQ_CUDA(ctx, cudaMemsetAsync(coef.p, 0, (size_t)blocks * 128, ctx->stream));
+    J::jpeg_unstuff_kernel<<<nb, J::kUnstuffThreads, 0, ctx->stream>>>(d, src, (uint8_t*)ub.p, (int32_t*)intv.p, status);
+    BQ_LAUNCH_CHECK(ctx);
+    J::jpeg_huffman_kernel<<<nb, J::kHuffThreads, 0, ctx->stream>>>(d, (const uint8_t*)ub.p, (const int32_t*)intv.p,
+                                                                    (int32_t*)ichunk.p, (J::Chunk*)chunks.p,
+                                                                    (int16_t*)coef.p, status, st);
+    BQ_LAUNCH_CHECK(ctx);
+    const dim3 gi((unsigned)((max_tile_blocks + J::kIdctBlocks - 1) / J::kIdctBlocks), (unsigned)nb);
+    J::jpeg_idct_kernel<<<gi, J::kIdctThreads, 0, ctx->stream>>>(d, (const int16_t*)coef.p, status, (uint8_t*)planes.p,
+                                                                 pitch);
+    BQ_LAUNCH_CHECK(ctx);
+    const dim3 gc((unsigned)((px * px + 255) / 256), (unsigned)nb);
+    J::jpeg_color_kernel<<<gc, 256, 0, ctx->stream>>>(d, (const uint8_t*)planes.p, status, pitch, px, out);
+    BQ_LAUNCH_CHECK(ctx);
+    return BQ_OK;
+  }
+
+  // subsequence statistics of the whole call, for bq_jpeg_last_stats
+  int finished(bq_ctx* ctx) override {
+    std::vector<int32_t> s((size_t)n * 3);
+    BQ_CUDA(ctx, cudaMemcpy(s.data(), stats.p, s.size() * 4, cudaMemcpyDeviceToHost));
+    last_stats[0] = n;
+    last_stats[1] = last_stats[2] = last_stats[3] = 0;
+    for (int64_t i = 0; i < n; ++i) {
+      last_stats[1] += s[3 * i];
+      last_stats[2] = std::max<int64_t>(last_stats[2], s[3 * i + 1]);
+      last_stats[3] += s[3 * i + 2];
+    }
+    return BQ_OK;
+  }
 };
 
-void bq_jpeg_state_destroy(bq_jpeg_state* s) { delete s; }
+}  // namespace
 
-static int64_t n_groups(const bq_jpeg_state* s) { return (s->n + s->group - 1) / s->group; }
-
-// Parse every tile (nothing is launched when one is rejected), lay out the groups and size the scratch.
-int bq_jpeg_prepare(bq_ctx* ctx, bq_jpeg_state*& s, const uint8_t* data, const int64_t* offsets, int64_t n, int px,
-                    int64_t group, int32_t* status_host) {
-  if (!s) s = new bq_jpeg_state();
-  if (n < 0 || px < 16 || px > 4096 || group < 1 || (n > 0 && (!data || !offsets)))
-    return bq_fail(ctx, BQ_ERR_ARG, "bq_jpeg: bad argument");
-  for (int64_t i = 0; i < n; ++i)
-    if (offsets[i] < 0 || offsets[i + 1] < offsets[i])
-      return bq_fail(ctx, BQ_ERR_ARG, "bq_jpeg: offsets must be non-negative and non-decreasing (tile %lld)", (long long)i);
-  s->data = data;
-  s->on_dev = n > 0 && bq_is_device_ptr(data);
-  s->px = px;
-  s->n = n;
-  s->group = group;
-  s->offs.assign(offsets, offsets + n + 1);
-  if ((size_t)n > s->desc_host_cap) {
-    if (s->desc_host) cudaFreeHost(s->desc_host);
-    s->desc_host = nullptr;
-    s->desc_host_cap = 0;
-    BQ_CUDA(ctx, cudaHostAlloc((void**)&s->desc_host, (size_t)n * sizeof(Tile), cudaHostAllocDefault));
-    s->desc_host_cap = (size_t)n;
-  }
-  std::vector<int32_t> st((size_t)n, 0);
-  if (!s->on_dev) {
-    for (int64_t i = 0; i < n; ++i) {
-      const int64_t len = offsets[i + 1] - offsets[i];
-      const uint8_t* b = data + offsets[i];
-      const uint8_t tail[2] = {len >= 2 ? b[len - 2] : (uint8_t)0, len >= 1 ? b[len - 1] : (uint8_t)0};
-      st[i] = parse_tile(b, len, len, tail, px, s->desc_host[i]);
-    }
-  } else if (n > 0) {
-    // device bytes: fetch each tile's first kHead bytes and last two; parse again from the whole tile when the headers
-    // run past kHead (large APPn segments)
-    constexpr int kHead = 2048;
-    int rc;
-    if ((rc = bq_alloc(ctx, s->offs_dev, (size_t)(n + 1) * 8)) || (rc = bq_alloc(ctx, s->heads, (size_t)n * (kHead + 2))))
-      return rc;
-    BQ_CUDA(ctx, cudaMemcpyAsync(s->offs_dev.p, offsets, (size_t)(n + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
-    if ((rc = bq_gather_heads(ctx, data, (const int64_t*)s->offs_dev.p, n, kHead, (uint8_t*)s->heads.p))) return rc;
-    std::vector<uint8_t> heads((size_t)n * (kHead + 2)), whole;
-    BQ_CUDA(ctx, cudaMemcpyAsync(heads.data(), s->heads.p, heads.size(), cudaMemcpyDeviceToHost, ctx->stream));
-    BQ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    for (int64_t i = 0; i < n; ++i) {
-      const int64_t len = offsets[i + 1] - offsets[i];
-      const uint8_t* h = heads.data() + (size_t)i * (kHead + 2);
-      st[i] = parse_tile(h, len, std::min<int64_t>(len, kHead), h + kHead, px, s->desc_host[i]);
-      if (st[i] == kNeedMore) {
-        whole.resize((size_t)len);
-        BQ_CUDA(ctx, cudaMemcpy(whole.data(), data + offsets[i], (size_t)len, cudaMemcpyDeviceToHost));
-        st[i] = parse_tile(whole.data(), len, len, h + kHead, px, s->desc_host[i]);
-      }
-    }
-  }
-  if (status_host) memcpy(status_host, st.data(), (size_t)n * 4);
-  for (int64_t i = 0; i < n; ++i)
-    if (st[i] != BQ_JPEG_OK)
-      return bq_fail(ctx, BQ_ERR_DATA, "JPEG tile %lld: %s", (long long)i, status_string(st[i]));
-  // group layout: every base is relative to the group
-  s->max_bytes = 0;
-  s->max_int = s->max_chunks = s->max_blocks = s->max_tile_blocks = 0;
-  for (int64_t g = 0; g < n_groups(s); ++g) {
-    const int64_t i0 = g * group, i1 = std::min(n, i0 + group);
-    int64_t ni = 0, nc = 0, nbk = 0;
-    for (int64_t i = i0; i < i1; ++i) {
-      Tile& t = s->desc_host[i];
-      t.seg_off += offsets[i] - offsets[i0];
-      t.int_base = (int32_t)ni;
-      t.chunk_base = (int32_t)nc;
-      t.coef_base = nbk;
-      const int64_t blocks = (int64_t)t.mcux * t.mcuy * t.bpm;
-      ni += t.n_int + 1;
-      nc += t.chunk_cap;
-      nbk += blocks;
-      s->max_tile_blocks = std::max(s->max_tile_blocks, blocks);
-    }
-    if (nc > INT32_MAX || ni > INT32_MAX) return bq_fail(ctx, BQ_ERR_ARG, "bq_jpeg: group too large");
-    s->max_bytes = std::max(s->max_bytes, (size_t)(offsets[i1] - offsets[i0]));
-    s->max_int = std::max(s->max_int, ni);
-    s->max_chunks = std::max(s->max_chunks, nc);
-    s->max_blocks = std::max(s->max_blocks, nbk);
-  }
-  const size_t pitch = bq_align_up((size_t)px, 16);
-  const int64_t gmax = std::min(n, group);
-  int rc;
-  if ((!s->on_dev && ((rc = bq_alloc(ctx, s->stage[0], s->max_bytes + 16)) || (rc = bq_alloc(ctx, s->stage[1], s->max_bytes + 16)))) ||
-      (rc = bq_alloc(ctx, s->desc[0], (size_t)gmax * sizeof(Tile))) || (rc = bq_alloc(ctx, s->desc[1], (size_t)gmax * sizeof(Tile))) ||
-      (rc = bq_alloc(ctx, s->ub, s->max_bytes + 16)) || (rc = bq_alloc(ctx, s->intv, (size_t)s->max_int * 4)) ||
-      (rc = bq_alloc(ctx, s->ichunk, (size_t)s->max_int * 4)) ||
-      (rc = bq_alloc(ctx, s->chunks, (size_t)s->max_chunks * sizeof(bq::jpeg::Chunk))) ||
-      (rc = bq_alloc(ctx, s->coef, (size_t)s->max_blocks * 128)) ||
-      (rc = bq_alloc(ctx, s->planes, (size_t)gmax * 3 * pitch * pitch)) ||
-      (rc = bq_alloc(ctx, s->status, (size_t)std::max<int64_t>(n, 1) * 4)) ||
-      (rc = bq_alloc(ctx, s->stats, (size_t)std::max<int64_t>(n, 1) * 12)))
-    return rc;
-  return BQ_OK;
-}
-
-int64_t bq_jpeg_group_count(const bq_jpeg_state* s) { return n_groups(s); }
-
-int bq_gather_heads(bq_ctx* ctx, const uint8_t* data, const int64_t* offsets_dev, int64_t n, int head, uint8_t* out) {
-  bq::jpeg::jpeg_gather_heads_kernel<<<(unsigned)n, 256, 0, ctx->stream>>>(data, offsets_dev, head, out);
-  BQ_LAUNCH_CHECK(ctx);
-  return BQ_OK;
-}
-
-// Copy group g's descriptors (and its bytes, when they are in host memory) into slot `slot` on `stream`.
-int bq_jpeg_upload(bq_ctx* ctx, bq_jpeg_state* s, int64_t g, int slot, cudaStream_t stream) {
-  const int64_t i0 = g * s->group, i1 = std::min(s->n, i0 + s->group);
-  BQ_CUDA(ctx, cudaMemcpyAsync(s->desc[slot].p, s->desc_host + i0, (size_t)(i1 - i0) * sizeof(Tile),
-                               cudaMemcpyHostToDevice, stream));
-  if (!s->on_dev)
-    BQ_CUDA(ctx, cudaMemcpyAsync(s->stage[slot].p, s->data + s->offs[i0], (size_t)(s->offs[i1] - s->offs[i0]),
-                                 cudaMemcpyHostToDevice, stream));
-  return BQ_OK;
-}
-
-// Decode group g (uploaded into `slot`) on the ctx stream into out = uint8 NHWC [group tiles, px, px, 3] (device).
-int bq_jpeg_decode_group(bq_ctx* ctx, bq_jpeg_state* s, int64_t g, int slot, uint8_t* out) {
-  namespace J = bq::jpeg;
-  const int64_t i0 = g * s->group, i1 = std::min(s->n, i0 + s->group);
-  const int nb = (int)(i1 - i0);
-  const int px = s->px, pitch = (int)bq_align_up((size_t)px, 16);
-  const uint8_t* src = s->on_dev ? s->data + s->offs[i0] : (const uint8_t*)s->stage[slot].p;
-  const Tile* d = (const Tile*)s->desc[slot].p;
-  int32_t* status = (int32_t*)s->status.p + i0;
-  int32_t* stats = (int32_t*)s->stats.p + 3 * i0;
-  int64_t blocks = 0;
-  for (int64_t i = i0; i < i1; ++i) blocks += (int64_t)s->desc_host[i].mcux * s->desc_host[i].mcuy * s->desc_host[i].bpm;
-  BQ_CUDA(ctx, cudaMemsetAsync(status, 0, (size_t)nb * 4, ctx->stream));
-  BQ_CUDA(ctx, cudaMemsetAsync(stats, 0, (size_t)nb * 12, ctx->stream));
-  BQ_CUDA(ctx, cudaMemsetAsync(s->coef.p, 0, (size_t)blocks * 128, ctx->stream));
-  J::jpeg_unstuff_kernel<<<nb, J::kUnstuffThreads, 0, ctx->stream>>>(d, src, (uint8_t*)s->ub.p, (int32_t*)s->intv.p, status);
-  BQ_LAUNCH_CHECK(ctx);
-  J::jpeg_huffman_kernel<<<nb, J::kHuffThreads, 0, ctx->stream>>>(d, (const uint8_t*)s->ub.p, (const int32_t*)s->intv.p,
-                                                                  (int32_t*)s->ichunk.p, (J::Chunk*)s->chunks.p,
-                                                                  (int16_t*)s->coef.p, status, stats);
-  BQ_LAUNCH_CHECK(ctx);
-  const dim3 gi((unsigned)((s->max_tile_blocks + J::kIdctBlocks - 1) / J::kIdctBlocks), (unsigned)nb);
-  J::jpeg_idct_kernel<<<gi, J::kIdctThreads, 0, ctx->stream>>>(d, (const int16_t*)s->coef.p, status, (uint8_t*)s->planes.p,
-                                                               pitch);
-  BQ_LAUNCH_CHECK(ctx);
-  const dim3 gc((unsigned)((px * px + 255) / 256), (unsigned)nb);
-  J::jpeg_color_kernel<<<gc, 256, 0, ctx->stream>>>(d, (const uint8_t*)s->planes.p, status, pitch, px, out);
-  BQ_LAUNCH_CHECK(ctx);
-  return BQ_OK;
-}
-
-// After the last group: wait, fetch the per-tile status, and fail with the first rejected tile.
-int bq_jpeg_finish(bq_ctx* ctx, bq_jpeg_state* s, int32_t* status_host) {
-  BQ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  if (s->n == 0) return BQ_OK;
-  std::vector<int32_t> st((size_t)s->n), stats((size_t)s->n * 3);
-  BQ_CUDA(ctx, cudaMemcpy(st.data(), s->status.p, st.size() * 4, cudaMemcpyDeviceToHost));
-  BQ_CUDA(ctx, cudaMemcpy(stats.data(), s->stats.p, stats.size() * 4, cudaMemcpyDeviceToHost));
-  s->last_stats[0] = s->n;
-  s->last_stats[1] = s->last_stats[2] = s->last_stats[3] = 0;
-  for (int64_t i = 0; i < s->n; ++i) {
-    s->last_stats[1] += stats[3 * i];
-    s->last_stats[2] = std::max<int64_t>(s->last_stats[2], stats[3 * i + 1]);
-    s->last_stats[3] += stats[3 * i + 2];
-  }
-  if (status_host) memcpy(status_host, st.data(), st.size() * 4);
-  for (int64_t i = 0; i < s->n; ++i)
-    if (st[i] != BQ_JPEG_OK)
-      return bq_fail(ctx, BQ_ERR_DATA, "JPEG tile %lld: %s", (long long)i, status_string(st[i]));
-  return BQ_OK;
-}
+bq_encoded* bq_jpeg_state(bq_encoded*& slot) { return slot ? slot : (slot = new Jpeg()); }
 
 extern "C" {
 
 const char* bq_jpeg_status_string(int32_t status) { return status_string(status); }
 
 int bq_jpeg_inspect(const uint8_t* data, const int64_t* offsets, int64_t n, int32_t px, int32_t* status) {
-  if (n < 0 || !status || (n > 0 && (!data || !offsets))) return BQ_ERR_ARG;
-  for (int64_t i = 0; i < n; ++i) {
-    const int64_t len = offsets[i + 1] - offsets[i];
-    if (offsets[i] < 0 || len < 0) return BQ_ERR_ARG;
-    const uint8_t* b = data + offsets[i];
-    const uint8_t tail[2] = {len >= 2 ? b[len - 2] : (uint8_t)0, len >= 1 ? b[len - 1] : (uint8_t)0};
-    Tile t;
-    status[i] = parse_tile(b, len, len, tail, px, t);
-  }
-  return BQ_OK;
+  return bq_encoded_inspect(Jpeg(), data, offsets, n, px, status);
 }
 
 int bq_jpeg_decode(bq_ctx* ctx, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t px, uint8_t* out_u8,
                    int32_t* status) {
-  if (!ctx) return BQ_ERR_ARG;
-  if (n > 0 && !out_u8) return bq_fail(ctx, BQ_ERR_ARG, "bq_jpeg_decode: bad argument");
-  BQ_CUDA(ctx, cudaSetDevice(ctx->device));
-  constexpr int64_t kGroup = 512;
-  int rc = bq_jpeg_prepare(ctx, ctx->jpeg, data, offsets, n, px, kGroup, status);
-  if (rc) return rc;
-  bq_jpeg_state* s = ctx->jpeg;
-  const size_t tile_bytes = (size_t)px * px * 3;
-  const bool out_dev = bq_is_device_ptr(out_u8);
-  DevBuf tmp;
-  if (!out_dev && n > 0 && (rc = bq_alloc(ctx, tmp, (size_t)std::min(n, kGroup) * tile_bytes))) return rc;
-  for (int64_t g = 0; g < n_groups(s); ++g) {
-    const int64_t i0 = g * kGroup, nb = std::min(n - i0, kGroup);
-    uint8_t* dst = out_dev ? out_u8 + (size_t)i0 * tile_bytes : (uint8_t*)tmp.p;
-    if ((rc = bq_jpeg_upload(ctx, s, g, 0, ctx->stream)) || (rc = bq_jpeg_decode_group(ctx, s, g, 0, dst))) return rc;
-    if (!out_dev) BQ_CUDA(ctx, cudaMemcpyAsync(out_u8 + (size_t)i0 * tile_bytes, dst, (size_t)nb * tile_bytes,
-                                               cudaMemcpyDeviceToHost, ctx->stream));
-  }
-  rc = bq_jpeg_finish(ctx, s, status);
-  if (!out_dev) BQ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // tmp is released below
-  return rc;
+  return ctx ? bq_encoded_decode(ctx, bq_jpeg_state(ctx->jpeg), data, offsets, n, px, out_u8, status) : BQ_ERR_ARG;
 }
 
 int bq_jpeg_last_stats(bq_ctx* ctx, int64_t stats[4]) {
   if (!ctx || !stats) return BQ_ERR_ARG;
-  for (int k = 0; k < 4; ++k) stats[k] = ctx->jpeg ? ctx->jpeg->last_stats[k] : 0;
+  for (int k = 0; k < 4; ++k) stats[k] = ctx->jpeg ? static_cast<const Jpeg*>(ctx->jpeg)->last_stats[k] : 0;
   return BQ_OK;
 }
 

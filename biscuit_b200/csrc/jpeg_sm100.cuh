@@ -566,20 +566,5 @@ __global__ void __launch_bounds__(256) jpeg_color_kernel(const Tile* __restrict_
   o[2] = (uint8_t)min(max(B, 0), 255);
 }
 
-// Header bytes of tiles resident on the device, for the host marker parse: the first `head` bytes of every tile
-// (zero-padded) followed by its last two bytes.
-__global__ void jpeg_gather_heads_kernel(const uint8_t* __restrict__ data, const int64_t* __restrict__ offsets, int head,
-                                         uint8_t* __restrict__ out) {
-  const int64_t i = blockIdx.x;
-  const int64_t off = offsets[i], len = offsets[i + 1] - offsets[i];
-  uint8_t* o = out + i * (head + 2);
-  for (int j = threadIdx.x; j < head + 2; j += blockDim.x) {
-    uint8_t v = 0;
-    if (j < head) v = j < len ? data[off + j] : 0;
-    else if (len >= 2) v = data[off + len - 2 + (j - head)];
-    o[j] = v;
-  }
-}
-
 }  // namespace jpeg
 }  // namespace bq

@@ -12,7 +12,7 @@
 #include <map>
 #include <memory>
 
-#include "common.cuh"
+#include "encoded.cuh"
 #include "gemm_sm100.cuh"
 #include "layers.cuh"
 #include "head_sm100.cuh"
@@ -263,8 +263,8 @@ struct bq_model {
   const uint8_t* tiles_src = nullptr;          // where stats / conv1 read the current micro-batch from
   cudaStream_t copy_stream = nullptr;          // H2D of micro-batch i+1 overlaps the backbone of micro-batch i
   cudaEvent_t copied[2] = {}, consumed[2] = {};
-  bq_jpeg_state* jpeg = nullptr;               // bq_predict_uq_jpeg: descriptors, compressed staging and decode scratch
-  bq_png_state* png = nullptr;                 // bq_predict_uq_png: likewise
+  bq_encoded* jpeg = nullptr;                  // bq_predict_uq_jpeg: descriptors, compressed staging and decode scratch
+  bq_encoded* png = nullptr;                   // bq_predict_uq_png: likewise
   DevBuf mean, inv_std;                        // fp32 [max_batch]
   Arena arena;
   DevBuf feat, feat_bf16;                      // [max_batch, 2048]
@@ -968,8 +968,8 @@ void bq_model_destroy(bq_model* m) {
   for (auto& e : m->kev) cudaEventDestroy(e);
   if (m->copy_stream) { cudaStreamSynchronize(m->copy_stream); cudaStreamDestroy(m->copy_stream); }
   for (int i = 0; i < 2; ++i) { if (m->copied[i]) cudaEventDestroy(m->copied[i]); if (m->consumed[i]) cudaEventDestroy(m->consumed[i]); }
-  bq_jpeg_state_destroy(m->jpeg);
-  bq_png_state_destroy(m->png);
+  delete m->jpeg;
+  delete m->png;
   delete m;
 }
 
@@ -1083,48 +1083,46 @@ int bq_model_load_weights(bq_model* m, const bq_named_tensor* tensors, int32_t n
   return BQ_OK;
 }
 
-// Input of predict_impl: decoded pixels, or n compressed files back to back with n + 1 host byte offsets.
-enum class Encoding { kPixels, kJpeg, kPng };
-
-static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, Encoding enc, const int64_t* offsets,
+// Input of predict_impl: decoded pixels (enc == NULL), or n compressed files back to back with n + 1 host byte offsets,
+// decoded through the format state `enc`.
+static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, bq_encoded* enc, const int64_t* offsets,
                         int64_t n, int32_t T, uint64_t seed, uint64_t tile_index_base, const uint8_t* masks, float* mean,
                         float* std, float* features);
 
 int bq_predict_uq(bq_model* m, const uint8_t* tiles, int64_t n, int32_t T, uint64_t seed, uint64_t tile_index_base,
                   const uint8_t* masks, float* mean, float* std, float* features) {
-  return predict_impl(m, tiles, false, Encoding::kPixels, nullptr, n, T, seed, tile_index_base, masks, mean, std,
-                      features);
+  return predict_impl(m, tiles, false, nullptr, nullptr, n, T, seed, tile_index_base, masks, mean, std, features);
 }
 
 int bq_predict_uq_jpeg(bq_model* m, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t T, uint64_t seed,
                        uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std, float* features) {
-  if (!m) return BQ_ERR_ARG;
-  if (n > 0 && !offsets) return bq_fail(m->ctx, BQ_ERR_ARG, "bq_predict_uq_jpeg: offsets must not be NULL");
-  return predict_impl(m, data, false, Encoding::kJpeg, offsets, n, T, seed, tile_index_base, masks, mean, std, features);
+  return predict_impl(m, data, false, m ? bq_jpeg_state(m->jpeg) : nullptr, offsets, n, T, seed, tile_index_base, masks,
+                      mean, std, features);
 }
 
 int bq_predict_uq_png(bq_model* m, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t T, uint64_t seed,
                       uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std, float* features) {
-  if (!m) return BQ_ERR_ARG;
-  if (n > 0 && !offsets) return bq_fail(m->ctx, BQ_ERR_ARG, "bq_predict_uq_png: offsets must not be NULL");
-  return predict_impl(m, data, false, Encoding::kPng, offsets, n, T, seed, tile_index_base, masks, mean, std, features);
+  return predict_impl(m, data, false, m ? bq_png_state(m->png) : nullptr, offsets, n, T, seed, tile_index_base, masks,
+                      mean, std, features);
 }
 
 int bq_predict_uq_standardized(bq_model* m, const float* tiles, int64_t n, int32_t T, uint64_t seed, uint64_t tile_index_base,
                                const uint8_t* masks, float* mean, float* std, float* features) {
   if (!m) return BQ_ERR_ARG;
   m->input_f32 = true;
-  const int rc = predict_impl(m, (const uint8_t*)tiles, true, Encoding::kPixels, nullptr, n, T, seed, tile_index_base,
+  const int rc = predict_impl(m, (const uint8_t*)tiles, true, nullptr, nullptr, n, T, seed, tile_index_base,
                               masks, mean, std, features);
   m->input_f32 = false;
   return rc;
 }
 
-static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, Encoding enc, const int64_t* offsets,
+static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, bq_encoded* enc, const int64_t* offsets,
                         int64_t n, int32_t T, uint64_t seed, uint64_t tile_index_base, const uint8_t* masks, float* mean,
                         float* std, float* features) {
   if (!m) return BQ_ERR_ARG;
   bq_ctx* ctx = m->ctx;
+  if (enc && n > 0 && !offsets)
+    return bq_fail(ctx, BQ_ERR_ARG, "bq_predict_uq_%s: offsets must not be NULL", enc->api().c_str());
   if (!m->weights_loaded) return bq_fail(ctx, BQ_ERR_STATE, "bq_predict_uq: weights not loaded");
   if (n < 0 || T < 1 || T > 4096 || (n > 0 && (!tiles || !mean || !std)))
     return bq_fail(ctx, BQ_ERR_ARG, "bq_predict_uq: bad argument");
@@ -1146,10 +1144,9 @@ static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, Encod
   // backbone of micro-batch i computes.  Device tiles are read in place.  Compressed (JPEG / PNG) tiles always take
   // the staged route: micro-batch i + 1's descriptors (and its compressed bytes, unless they are device memory, which
   // is read in place) go up on the copy stream, and micro-batch i is decoded on the ctx stream into tiles_dev.
-  const bool compressed = enc != Encoding::kPixels;
+  const bool compressed = enc != nullptr;
   if (compressed) {
-    const int rcj = enc == Encoding::kJpeg ? bq_jpeg_prepare(ctx, m->jpeg, tiles, offsets, n, m->px, B, nullptr)
-                                           : bq_png_prepare(ctx, m->png, tiles, offsets, n, m->px, B, nullptr);
+    const int rcj = enc->prepare(ctx, tiles, offsets, n, m->px, B, nullptr);
     if (rcj) return rcj;
   }
   const bool tiles_on_dev = !compressed && bq_is_device_ptr(tiles);
@@ -1162,8 +1159,7 @@ static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, Encod
     const int nbc = (int)((n - i0c < B) ? (n - i0c) : B);
     BQ_CUDA(ctx, cudaStreamWaitEvent(m->copy_stream, m->consumed[slot], 0));   // previous reader of this slot done
     if (compressed) {
-      const int rcu = enc == Encoding::kJpeg ? bq_jpeg_upload(ctx, m->jpeg, i0c / B, slot, m->copy_stream)
-                                             : bq_png_upload(ctx, m->png, i0c / B, slot, m->copy_stream);
+      const int rcu = enc->upload(ctx, i0c / B, slot, m->copy_stream);
       if (rcu) return rcu;
     } else {
       BQ_CUDA(ctx, cudaMemcpyAsync(stage[slot], tiles + (size_t)i0c * tile_bytes, (size_t)nbc * tile_bytes,
@@ -1187,9 +1183,7 @@ static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, Encod
       BQ_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, m->copied[slot], 0));
       m->tiles_src = stage[slot];
       if (compressed) {
-        rc = enc == Encoding::kJpeg ? bq_jpeg_decode_group(ctx, m->jpeg, batch_idx, slot, (uint8_t*)m->tiles_dev.p)
-                                    : bq_png_decode_group(ctx, m->png, batch_idx, slot, (uint8_t*)m->tiles_dev.p);
-        if (rc) return rc;
+        if ((rc = enc->decode_group(ctx, batch_idx, slot, (uint8_t*)m->tiles_dev.p))) return rc;
         BQ_CUDA(ctx, cudaEventRecord(m->consumed[slot], ctx->stream));        // the compressed slot is free once decoded
         m->tiles_src = (const uint8_t*)m->tiles_dev.p;
       }
@@ -1250,7 +1244,7 @@ static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, Encod
     }
   }
   BQ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  if (compressed) return enc == Encoding::kJpeg ? bq_jpeg_finish(ctx, m->jpeg, nullptr) : bq_png_finish(ctx, m->png, nullptr);
+  if (compressed) return enc->finish(ctx, nullptr);
   return BQ_OK;
 }
 

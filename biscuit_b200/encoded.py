@@ -1,8 +1,11 @@
-"""Byte container shared by the compressed-tile formats (`jpeg.JpegBatch`, `png.PngBatch`): n files back to back in
-one host or device buffer plus n + 1 host byte offsets.  The subclass names the format the bytes are decoded as."""
+"""Compressed tiles of any format (`jpeg.JpegBatch`, `png.PngBatch`): the byte container -- n files back to back in one
+host or device buffer plus n + 1 host byte offsets -- and the calls into the library's `bq_{fmt}_*` entry points that
+`jpeg` and `png` expose.  The subclass names the format the bytes are decoded as (`FORMAT`)."""
 from __future__ import annotations
 
 import numpy as np
+
+from . import _ffi
 
 
 class EncodedBatch:
@@ -10,6 +13,8 @@ class EncodedBatch:
 
     data: 1-D uint8 numpy array (host) or contiguous CUDA torch uint8 tensor (read in place on the GPU);
     offsets: n + 1 non-decreasing int64 byte offsets (host)."""
+
+    FORMAT: str          # "jpeg" / "png": the `bq_{FORMAT}_*` entry points that decode it
 
     def __init__(self, data, offsets):
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
@@ -56,3 +61,41 @@ class EncodedBatch:
         """the same batch (same class) with its bytes in device memory"""
         import torch
         return type(self)(torch.from_numpy(np.asarray(self.data)).cuda(device), self.offsets)
+
+
+def status_message(fmt: str, code: int) -> str:
+    return getattr(_ffi.load_library(), f"bq_{fmt}_status_string")(int(code)).decode()
+
+
+def inspect(fmt: str, batch: EncodedBatch, px: int) -> np.ndarray:
+    if batch.on_device:
+        raise ValueError("inspect reads host bytes; the batch is in device memory")
+    entry = getattr(_ffi.load_library(), f"bq_{fmt}_inspect")
+    st = np.zeros(len(batch), np.int32)
+    rc = entry(_ffi.ptr(batch.data), _ffi.ptr(batch.offsets), len(batch), int(px), _ffi.ptr(st))
+    if rc != 0:
+        raise ValueError(f"bq_{fmt}_inspect: bad argument")
+    return st
+
+
+def check(fmt: str, batch: EncodedBatch, px: int) -> None:
+    st = inspect(fmt, batch, px)
+    bad = np.flatnonzero(st)
+    if bad.size:
+        raise ValueError(f"{fmt.upper()} tile {int(bad[0])}: {status_message(fmt, int(st[bad[0]]))}")
+
+
+def decode(fmt: str, batch: EncodedBatch, px: int, ctx: _ffi.Context | None, out):
+    ctx = ctx or _ffi.default_context()
+    n = len(batch)
+    if out is None:
+        out = np.empty((n, px, px, 3), np.uint8)
+    if tuple(out.shape) != (n, px, px, 3) or str(out.dtype).replace("torch.", "") != "uint8":
+        raise ValueError(f"out must be uint8 of shape {(n, px, px, 3)}")
+    if isinstance(out, np.ndarray) and not out.flags.c_contiguous:
+        raise ValueError("out must be C-contiguous")
+    st = np.zeros(n, np.int32)
+    entry = getattr(ctx.lib, f"bq_{fmt}_decode")
+    _ffi.check(ctx.handle, entry(ctx.handle, _ffi.ptr(batch.data), _ffi.ptr(batch.offsets), n, int(px), _ffi.ptr(out),
+                                 _ffi.ptr(st)), f"bq_{fmt}_decode")
+    return out

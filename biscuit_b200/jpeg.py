@@ -16,7 +16,7 @@ import ctypes as C
 
 import numpy as np
 
-from . import _ffi
+from . import _ffi, encoded
 from .encoded import EncodedBatch
 from .hp import nature2022
 
@@ -27,47 +27,28 @@ class JpegBatch(EncodedBatch):
     data: 1-D uint8 numpy array (host) or contiguous CUDA torch uint8 tensor (read in place on the GPU);
     offsets: n + 1 non-decreasing int64 byte offsets (host)."""
 
+    FORMAT = "jpeg"
+
 
 def status_message(code: int) -> str:
-    return _ffi.load_library().bq_jpeg_status_string(int(code)).decode()
+    return encoded.status_message("jpeg", code)
 
 
 def inspect(batch: JpegBatch, px: int = nature2022.tile_px) -> np.ndarray:
     """Host marker parse of every tile, no GPU needed: int32 status per tile (0 = accepted, else a BQ_JPEG_* code,
     see `status_message`)."""
-    if batch.on_device:
-        raise ValueError("inspect reads host bytes; the batch is in device memory")
-    lib = _ffi.load_library()
-    st = np.zeros(len(batch), np.int32)
-    rc = lib.bq_jpeg_inspect(_ffi.ptr(batch.data), _ffi.ptr(batch.offsets), len(batch), int(px), _ffi.ptr(st))
-    if rc != 0:
-        raise ValueError("bq_jpeg_inspect: bad argument")
-    return st
+    return encoded.inspect("jpeg", batch, px)
 
 
 def check(batch: JpegBatch, px: int = nature2022.tile_px) -> None:
     """raise ValueError for the first tile `decode` would reject by its headers"""
-    st = inspect(batch, px)
-    bad = np.flatnonzero(st)
-    if bad.size:
-        raise ValueError(f"JPEG tile {int(bad[0])}: {status_message(int(st[bad[0]]))}")
+    return encoded.check("jpeg", batch, px)
 
 
 def decode(batch: JpegBatch, px: int = nature2022.tile_px, ctx: _ffi.Context | None = None, out=None):
     """uint8 NHWC [n, px, px, 3] tiles decoded on the GPU.  `out` may be a preallocated numpy array or CUDA torch tensor
     of that shape (device output stays on the device); default: a new numpy array."""
-    ctx = ctx or _ffi.default_context()
-    n = len(batch)
-    if out is None:
-        out = np.empty((n, px, px, 3), np.uint8)
-    if tuple(out.shape) != (n, px, px, 3) or str(out.dtype).replace("torch.", "") != "uint8":
-        raise ValueError(f"out must be uint8 of shape {(n, px, px, 3)}")
-    if isinstance(out, np.ndarray) and not out.flags.c_contiguous:
-        raise ValueError("out must be C-contiguous")
-    st = np.zeros(n, np.int32)
-    _ffi.check(ctx.handle, ctx.lib.bq_jpeg_decode(ctx.handle, _ffi.ptr(batch.data), _ffi.ptr(batch.offsets), n, int(px),
-                                                  _ffi.ptr(out), _ffi.ptr(st)), "bq_jpeg_decode")
-    return out
+    return encoded.decode("jpeg", batch, px, ctx, out)
 
 
 def last_stats(ctx: _ffi.Context | None = None) -> dict:

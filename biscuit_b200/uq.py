@@ -24,8 +24,7 @@ import pandas as pd
 
 from . import _ffi
 from .hp import ModelConfig, nature2022
-from .jpeg import JpegBatch
-from .png import PngBatch
+from .encoded import EncodedBatch
 from .utils import uncertainty_header, y_pred_header, y_true_header
 
 FEATURES = 2048
@@ -130,7 +129,7 @@ class UncertaintyInterface:
         uint8 tiles bit for bit.
         Returns (mean [n, C], std [n, C]) float32 -- population std over T dropout samples."""
         T = int(T or self.num_uq)
-        encoded = {JpegBatch: "jpeg", PngBatch: "png"}.get(type(tiles))
+        encoded = tiles.FORMAT if isinstance(tiles, EncodedBatch) else None
         n = len(tiles) if encoded else int(tiles.shape[0])
         px = self.config.tile_px
         if not encoded and tuple(tiles.shape[1:]) != (px, px, 3):
@@ -158,7 +157,7 @@ class UncertaintyInterface:
             if isinstance(masks, np.ndarray):
                 masks = np.ascontiguousarray(masks, dtype=np.uint8)
         if encoded:
-            entry = self.lib.bq_predict_uq_jpeg if encoded == "jpeg" else self.lib.bq_predict_uq_png
+            entry = getattr(self.lib, f"bq_predict_uq_{encoded}")
             rc = entry(self.h, _ffi.ptr(tiles.data), _ffi.ptr(tiles.offsets), n, T, C.c_uint64(seed),
                        C.c_uint64(tile_index_base), _ffi.ptr(masks), _ffi.ptr(mean), _ffi.ptr(std), _ffi.ptr(feats))
         else:
