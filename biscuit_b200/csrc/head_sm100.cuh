@@ -43,6 +43,7 @@ struct HeadParams {
   int n, T, W, C;
   int n_sites, slot1, slot2; // enabled sites in the mask tensor; slot < 0: that site has no dropout (keep everything)
   int mask_w;               // row pitch of the injected masks (2048 when the feature site is enabled, else W)
+  int w2_box;               // rows of one W2 TMA box: 256, or W itself when W < 256 (bn_box_for in model.cu)
   int h1_per_sample;        // 1: h1 is [n * T, W] (dropout on the pooled features made hidden_0 sample dependent)
   float inv_keep1, inv_keep2;   // 1/(1-p) behind an enabled site, 1 otherwise
   float inv_keep;
@@ -77,7 +78,7 @@ __device__ __forceinline__ uint32_t keep8(const HeadParams& p, uint64_t tile, in
 }
 
 __global__ void __launch_bounds__(kHThreads, 1)
-mc_head_fused_kernel(const __grid_constant__ CUtensorMap tmap_w2 /*[W(out), W(in)] bf16, box [256 x 64]*/,
+mc_head_fused_kernel(const __grid_constant__ CUtensorMap tmap_w2 /*[W(out), W(in)] bf16, box [w2_box x 64]*/,
                      const HeadParams p) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -144,13 +145,16 @@ mc_head_fused_kernel(const __grid_constant__ CUtensorMap tmap_w2 /*[W(out), W(in
         const int hw = min(512, W - h * 512);                  // output units of this half
         if (warp == 0) {
           // ---------------- W2 k-blocks by TMA ----------------
+          // A box is 256 rows, or all W rows when W < 256 (then one box covers the half): either way box nb lands at
+          // row nb * 256 of the stage, where the MMA below reads it.  Rows past W arrive zero-filled and count in full.
           if (lane == 0) {
+            const int box = p.w2_box;
             for (int kb = 0; kb < num_kb; ++kb) {
               mbar_wait(empty_bar(s), ph ^ 1u);
-              mbar_expect_tx(full_bar(s), (uint32_t)((hw + 255) / 256) * 256u * 64u * 2u);
+              mbar_expect_tx(full_bar(s), (uint32_t)((hw + box - 1) / box) * (uint32_t)box * 64u * 2u);
               const uint32_t b_dst = smem_base + s * kHStageBytes + kHABytes;
-              for (int nb = 0; nb * 256 < hw; ++nb)
-                tma_load_2d(b_dst + nb * 256 * 128, &tmap_w2, full_bar(s), kb * 64, h * 512 + nb * 256);
+              for (int nb = 0; nb * box < hw; ++nb)
+                tma_load_2d(b_dst + nb * box * 128, &tmap_w2, full_bar(s), kb * 64, h * 512 + nb * box);
               if (++s == kHStages) { s = 0; ph ^= 1u; }
             }
           }

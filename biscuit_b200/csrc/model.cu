@@ -878,6 +878,7 @@ int run_head(bq_model* m, int nb, int T, uint64_t seed, uint64_t tile_base, cons
   hp.n = nb; hp.T = T; hp.W = Wd; hp.C = NC;
   hp.n_sites = m->n_sites; hp.slot1 = m->slot[1]; hp.slot2 = m->slot[2];
   hp.mask_w = m->mask_w;
+  hp.w2_box = m->head_gemms[1].gp.bn_box;          // the box rows the W2 tensor map was built with
   hp.h1_per_sample = (m->sites & 1) ? 1 : 0;
   hp.inv_keep = 1.0f / (1.0f - m->cfg.dropout);
   hp.inv_keep1 = (m->sites & 2) ? hp.inv_keep : 1.0f;
@@ -910,6 +911,7 @@ int bq_model_create(bq_ctx* ctx, const bq_model_config* cfg, bq_model** out) {
   if (cfg->tile_px != 299) return bq_fail(ctx, BQ_ERR_ARG, "tile_px must be 299 (hp.py:5), got %d", cfg->tile_px);
   if (cfg->hidden_layers != 2) return bq_fail(ctx, BQ_ERR_ARG, "hidden_layers must be 2 (hp.py:21), got %d", cfg->hidden_layers);
   if (cfg->hidden_width <= 0 || cfg->hidden_width % 64) return bq_fail(ctx, BQ_ERR_ARG, "hidden_width must be a positive multiple of 64");
+  if (cfg->hidden_width > bq::head::kHMaxW) return bq_fail(ctx, BQ_ERR_ARG, "the fused MC-dropout head needs 2 hidden layers of width <= 1024 (hp.py:13,21)");
   if (cfg->n_classes < 2 || cfg->n_classes > bq::kMaxClasses) return bq_fail(ctx, BQ_ERR_ARG, "n_classes must be in [2,8]");
   if (!(cfg->dropout >= 0.f && cfg->dropout < 1.f)) return bq_fail(ctx, BQ_ERR_ARG, "dropout must be in [0,1)");
   if (cfg->max_batch < 1 || cfg->max_batch > 512) return bq_fail(ctx, BQ_ERR_ARG, "max_batch must be in [1,512]");
@@ -1302,11 +1304,12 @@ int bq_model_debug_tags(bq_model* m, char* out, int64_t capacity) {
 int bq_model_debug_h1(bq_model* m, int64_t n, float* out) {
   if (!m) return BQ_ERR_ARG;
   bq_ctx* ctx = m->ctx;
-  if (!out || n < 1 || n > m->head_batch || !m->h_act[0].p || (m->sites & 1))
-    return bq_fail(ctx, BQ_ERR_ARG, "bq_model_debug_h1: needs a preceding predict of >= n tiles (n <= %d) with no dropout on the features",
-                   m->head_batch);
+  if (!out || n < 1 || n > m->head_batch || !m->h_act[0].p || m->head_T < 1)
+    return bq_fail(ctx, BQ_ERR_ARG, "bq_model_debug_h1: needs a preceding predict of >= n tiles (n <= %d)", m->head_batch);
   BQ_CUDA(ctx, cudaSetDevice(ctx->device));
-  const int64_t total = n * m->cfg.hidden_width;
+  // with dropout on the pooled features hidden_0 is per sample: [n * T, W] rows in (tile, sample) order
+  const int64_t rows = (m->sites & 1) ? n * m->head_T : n;
+  const int64_t total = rows * m->cfg.hidden_width;
   void* scr = nullptr;
   int rc;
   if ((rc = bq_scratch(ctx, total * 4, &scr))) return rc;

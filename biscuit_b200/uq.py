@@ -69,11 +69,14 @@ class UncertaintyInterface:
                  device: int | None = None, ctx: _ffi.Context | None = None, normalizer=None):
         if config.model != "xception" or config.pooling != "avg" or config.include_top:
             raise ValueError("only the reference configuration (xception, avg pooling, include_top=False) is built")
+        if not config.uq:
+            raise ValueError("UncertaintyInterface runs MC-dropout inference: config.uq must be True")
         self.config = config
         self.ctx = ctx or _ffi.default_context(device)
         self.lib = self.ctx.lib
         self.num_uq = config.uq_samples
         self.max_batch = int(max_batch)
+        self._head_T = None
         self.wsi_normalizer = None     # attribute the reference call site probes (results.py:251)
         cfg = _ffi.ModelConfig(tile_px=config.tile_px, hidden_width=config.hidden_layer_width,
                                hidden_layers=config.hidden_layers, n_classes=config.n_classes,
@@ -165,6 +168,8 @@ class UncertaintyInterface:
             rc = entry(self.h, _ffi.ptr(tiles), n, T, C.c_uint64(seed), C.c_uint64(tile_index_base), _ffi.ptr(masks),
                        _ffi.ptr(mean), _ffi.ptr(std), _ffi.ptr(feats))
         _ffi.check(self.ctx.handle, rc, "bq_predict_uq")
+        if n > 0:
+            self._head_T = T             # the head buffers now hold this call's T (debug_h1)
         if return_features:
             return mean, std, feats
         return mean, std
@@ -196,9 +201,14 @@ class UncertaintyInterface:
         return out[: int(np.prod(s))].reshape(s).copy()
 
     def debug_h1(self, n: int) -> np.ndarray:
-        """Parity hook: hidden_0 output (bf16 as float32, [n, hidden_width]) of the first n tiles of the last `predict`
-        call (which must have held them in one head batch, with no dropout on the pooled features)."""
-        out = np.empty((int(n), self.config.hidden_layer_width), np.float32)
+        """Parity hook: hidden_0 output (bf16 as float32) of the first n tiles of the last `predict` call, which must
+        have held them in one head batch: [n, hidden_width], or [n, T, hidden_width] with dropout on the pooled features
+        (hidden_0 is then per sample, T = that call's sample count)."""
+        width = self.config.hidden_layer_width
+        if self._head_T is None:
+            raise ValueError("debug_h1 needs a preceding predict")
+        shape = (int(n), self._head_T, width) if self.config.dropout_sites[0] else (int(n), width)
+        out = np.empty(shape, np.float32)
         _ffi.check(self.ctx.handle, self.lib.bq_model_debug_h1(self.h, int(n), _ffi.ptr(out)), "bq_model_debug_h1")
         return out
 

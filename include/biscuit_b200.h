@@ -133,15 +133,16 @@ int bq_group_apply(bq_ctx* ctx, int64_t n_groups, int dtype, const void* g_pred,
 
 typedef struct bq_model_config {
   int32_t tile_px;        /* 299  (hp.py:5)                    */
-  int32_t hidden_width;   /* 1024 (hp.py:13)                   */
+  int32_t hidden_width;   /* 1024 (hp.py:13); a multiple of 64, at most 1024 (the fused head's limit) */
   int32_t hidden_layers;  /* 2    (hp.py:21)                   */
-  int32_t n_classes;      /* 2                                 */
+  int32_t n_classes;      /* 2; 2..8                           */
   float dropout;          /* 0.1  (hp.py:11)                   */
   int32_t max_batch;      /* tiles per backbone micro-batch    */
   /* MC-dropout placement, bit i = a Dropout(rate) active at inference after site i:
    *   bit 0: the pooled 2048-d features (Slideflow's `post_convolution`), bit 1: hidden_0, bit 2: hidden_1.
-   * 0 selects the default 0b110 (after each hidden layer).  Which placement a saved model has depends on the
-   * Slideflow version that built it (hp.py:11-12 only fix the rate and `uq`); INTEGRATION.md lists both. */
+   * 0 selects the default 0b110 (after each hidden layer), so a model without any dropout site cannot be built: the
+   * Python `ModelConfig` rejects an all-False placement instead of passing 0.  Which placement a saved model has
+   * depends on the Slideflow version that built it (hp.py:11-12 only fix the rate and `uq`); INTEGRATION.md lists both. */
   int32_t dropout_sites;
   int32_t reserved[7];
 } bq_model_config;
@@ -181,8 +182,9 @@ int bq_predict_uq_standardized(bq_model* m, const float* tiles, int64_t n, int32
  * float32 (NHWC).  Used by tests to localise a mismatch; not part of the reference surface. */
 int bq_model_debug_stage(bq_model* m, const uint8_t* tiles, int64_t n, const char* stage, float* out,
                          int64_t out_capacity, int64_t out_shape[4]);
-/* hidden_0 activations (bf16 as float32, [n, hidden_width]) of the first n tiles of the last bq_predict_uq call, when
- * that call held them in one head batch and dropout on the pooled features is off. */
+/* hidden_0 activations (bf16 as float32) of the first n tiles of the last bq_predict_uq call, when that call held them
+ * in one head batch: [n, hidden_width], or [n, T, hidden_width] (one row per sample, T of that call) when dropout on
+ * the pooled features is on.  `out` must hold that many floats. */
 int bq_model_debug_h1(bq_model* m, int64_t n, float* out);
 /* the debug_stage tags of the execution plan in execution order, one per line (NUL-terminated) */
 int bq_model_debug_tags(bq_model* m, char* out, int64_t capacity);

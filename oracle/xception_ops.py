@@ -21,7 +21,8 @@ Rounding points are taken from the kernels, not from oracle/xception_uq.py:
     with the per-tile constants g = scale / sd and h = shift - (m - m0) * sum(W) * g.
   * global average pool (layers.cuh): an n-term fp32 sum and one division.
   * MC-dropout head (gemm hidden_0 + head_sm100.cuh): intervals through the two bf16 activations h1, h2 and the fp32
-    prelogits, softmax evaluated at the interval ends (it is monotone in the logit difference).
+    prelogits, the softmax bounded through its monotonicity in each logit, then the fp32 allowances of the per-chunk
+    statistics and their Chan merge (head_slack), for every class count, width, dropout placement and rate.
 
 All functions take torch tensors (float32 holding bf16 values, NHWC) and work on the tensors' device.
 """
@@ -87,6 +88,16 @@ class OpWeights:
                 p = np.asarray(weights[f"{name}/pointwise_kernel"], np.float32)[0, 0]
                 self.pw[name] = t(_bf16_np(p.T))
                 self.affine[name] = tuple(t(a) for a in bn_affine(weights, f"{name}_bn"))
+        HeadWeights.__init__(self, weights, device)
+
+
+class HeadWeights:
+    """The head's kernel-side weights alone: `hidden[i]` = (bf16 [out, in], fp32 bias) of hidden_0 / hidden_1,
+    `w3` fp32 [W, C] and `b3` fp32 [C] of the prelogits"""
+
+    def __init__(self, weights: dict, device="cpu"):
+        self.device = device
+        t = lambda a: a.to(device)                                           # noqa: E731
         self.hidden = [(t(_bf16_np(np.asarray(weights[f"hidden_{i}/kernel"]).T)),
                         t(torch.from_numpy(np.asarray(weights[f"hidden_{i}/bias"], np.float32))))
                        for i in range(2)]
@@ -367,9 +378,23 @@ def describe(rep):
 MMA_K = 16            # K of one tcgen05.mma (bf16): the head's hidden_1 accumulates 1024 / 16 of them in k order
 
 
-def hidden0_ref(features: torch.Tensor, ow: OpWeights):
-    """hidden_0 on bf16(features): GEMM epilogue RN(acc * 1) + b1, ReLU, bf16 -> (z, E)"""
-    return gemm_ref(rn_bf16(features), ow.hidden[0][0], None, ow.hidden[0][1])
+def inv_keep(rate: float) -> float:
+    """the kernels' fp32 1/(1-p)"""
+    return float(np.float32(1.0) / (np.float32(1.0) - np.float32(rate)))
+
+
+def hidden0_ref(features: torch.Tensor, ow: OpWeights, k0=None, rate: float = 0.0):
+    """hidden_0 on bf16(features) [n, 2048]: GEMM epilogue RN(acc * alpha) + b1, ReLU, bf16 -> (z, E) [n, W].
+    With dropout on the pooled features (site 0), k0 = the site-0 keep-masks [n, T, 2048]: mc_expand_kernel writes one
+    row bf16(features) * keep0 per (tile, sample) (an exact selection) and the GEMM runs on those n * T rows with
+    alpha = 1/(1-p) (prepare_head) -> (z, E) [n, T, W]."""
+    a = rn_bf16(features)
+    W1, b1 = ow.hidden[0]
+    if k0 is None:
+        return gemm_ref(a, W1, None, b1)                                  # alpha = 1: RN(acc * 1) is exact
+    k0 = torch.as_tensor(k0).to(a.device, torch.float32)
+    alpha = torch.tensor(inv_keep(rate), dtype=torch.float64, device=a.device)
+    return gemm_ref(a[:, None, :] * k0, W1, alpha, b1)
 
 
 def mma_chain_bound(a: torch.Tensor, w: torch.Tensor):
@@ -389,13 +414,13 @@ def mma_chain_bound(a: torch.Tensor, w: torch.Tensor):
     return z, E * (1 + 2 * g * 17 * UA)                                 # the accumulator's own error, carried along
 
 
-def _fma_chain_interval(lo, hi, w):
-    """sequential fp32 fma over units j (ascending) of x_j * w[j, c], x in [lo, hi] (>= 0) -> (lo, hi) of the result"""
+def _fma_chain_error(lo, hi, w):
+    """bound on the rounding error of the sequential fp32 fma chain over units j (ascending) of x_j * w[j, c], for any x
+    in [lo, hi] (>= 0): one rounding of each partial sum, u * sum_j max |partial sum j| -> [n, C]"""
     wp, wn = torch.clamp_min(w, 0.0), torch.clamp_max(w, 0.0)
     tlo, thi = lo[:, :, None] * wp + hi[:, :, None] * wn, hi[:, :, None] * wp + lo[:, :, None] * wn   # [n, units, C]
     plo, phi = torch.cumsum(tlo, 1), torch.cumsum(thi, 1)
-    err = U * torch.maximum(plo.abs(), phi.abs()).sum(1) + TINY * w.shape[0]   # one rounding per fma
-    return plo[:, -1] - err, phi[:, -1] + err
+    return U * torch.maximum(plo.abs(), phi.abs()).sum(1) + TINY * w.shape[0], plo[:, -1], phi[:, -1]
 
 
 def _round_interval(lo, hi, mul, add):
@@ -406,48 +431,170 @@ def _round_interval(lo, hi, mul, add):
     return lo - U * lo.abs() - TINY, hi + U * hi.abs() + TINY
 
 
-def head_ref(h1: torch.Tensor, masks: np.ndarray, ow: OpWeights, rate=0.1):
-    """Fused head (head_sm100.cuh) from the GPU's own hidden_0 output h1 (bf16 [n, 1024]) and injected masks uint8
-    [n, T, 2, 1024] (sites 1, 2).  -> dict(mean_lo, mean_hi, std_z, std_w, slack) [n, 2]: the GPU mean must lie in
-    [mean_lo, mean_hi] +- slack and the GPU std within std_w + slack of std_z."""
+def logit_diff_interval(h2lo, h2hi, w3, b3, ik2):
+    """Interval of the fp32 logit differences z_j - z_c, z = RN(RN(l * ik2) + b3) with l the fp32 fma chain over the
+    bf16 activations h2 in [h2lo, h2hi] (>= 0) -> (dlo, dhi) [n, c, j].
+
+    Every logit is a function of the same h2, so the difference is bounded through the weights w3[:, j] - w3[:, c]
+    (bounding each logit alone and subtracting the ends would count each h2 unit's uncertainty twice): its exact part
+    lies in ik2 * [sum_k min, sum_k max of h2_k (w3[k, j] - w3[k, c])] + b3_j - b3_c.  Each logit adds its own fp32
+    error: the fma chain's (_fma_chain_error), scaled by ik2, then u |l ik2| and u |z| of the two roundings."""
+    C = w3.shape[1]
+    err, llo, lhi = _fma_chain_error(h2lo, h2hi, w3)
+    a = ik2 * (torch.maximum(llo.abs(), lhi.abs()) + err)                    # >= |RN(l) * ik2|
+    eps = ik2 * err + U * a + U * (a * (1 + U) + b3.abs()) + 3 * TINY         # [n, C]: |z~ - (ik2 l + b3)|
+    dw = (w3[:, None, :] - w3[:, :, None]).reshape(w3.shape[0], C * C)       # [units, (c, j)]
+    dp, dn = torch.clamp_min(dw, 0.0), torch.clamp_max(dw, 0.0)
+    dlo = (h2lo @ dp + h2hi @ dn).reshape(-1, C, C)
+    dhi = (h2hi @ dp + h2lo @ dn).reshape(-1, C, C)
+    db = b3[None, :] - b3[:, None]                                           # [c, j]: b3_j - b3_c
+    e = eps[:, None, :] + eps[:, :, None]
+    return ik2 * dlo + db - e, ik2 * dhi + db + e
+
+
+def softmax_interval(dlo, dhi):
+    """softmax p_c = 1 / (1 + sum_{j != c} exp(z_j - z_c)) falls with every difference d[c, j] = z_j - z_c, so for
+    differences in [dlo, dhi] ([..., c, j]): p_c in [1 / (1 + sum_{j != c} exp(dhi[c, j])), 1 / (1 + sum_{j != c}
+    exp(dlo[c, j]))] (C = 2: the sigmoid of the logit difference at its two ends)"""
+    C = dlo.shape[-1]
+    off = ~torch.eye(C, dtype=torch.bool, device=dlo.device)
+    return 1.0 / (1.0 + (torch.exp(dhi) * off).sum(-1)), 1.0 / (1.0 + (torch.exp(dlo) * off).sum(-1))
+
+
+CHUNK = 32            # samples per chunk of the head kernel's statistics (one per lane of a row warp)
+
+
+def head_slack(T: int, C: int):
+    """-> (dp, e_mean, eta): the fp32 rounding allowances of the head's softmax and statistics (head_sm100.cuh), for T
+    samples in K = ceil(T / 32) chunks and C classes; u = 2^-24, probabilities are <= 1.
+
+      * softmax (per sample): t_c = RN(z_c - max) is off by u |t_c|, which exp turns into a relative error u |t_c| on
+        e_c; expf adds <= 2 ulp (4u relative); the C-term fp32 sum of the denominator (>= 1: its largest term is
+        exp(0)) adds (C - 1) u; the division u.  With p_c |t_c| <= e^-|t_c| |t_c| <= 1/e and sum_j p_j |t_j| <= (C-1)/e,
+        |RN(p_c) - p_c| <= u (1/e + 4 + 4 + (C-1) + (C-1)/e + 1) + O(u^2) <= dp = (12 + 2 C) u.
+      * chunk mean: a 5-level shuffle butterfly over 32 lanes (invalid lanes add 0) and one division: |cm~ - cm| <=
+        gamma_6 max|p| <= 6u (+ O(u^2)).
+      * Chan merge k of r_mean: delta = RN(cm - r_mean), RN(delta * cn), RN(/ tot), RN(r_mean + .): the new exact mean
+        is a convex combination of the old one and cm, so the carried error stays <= max(E_{k-1}, 6u), and the three
+        roundings of the increment (|delta| <= 1) plus the one of the sum (|r_mean| <= 1) add 4u:
+        E_mean <= e_mean = (6 + 4 (K - 1)) u.
+      * M2: the chunk M2 uses d = RN(p - cm~) with cm~ = cm + eps: sum (d_j - eps)^2 = M2_chunk + cn eps^2 exactly (the
+        d_j of the exact chunk mean sum to 0), then the square and the butterfly: a relative gamma_7 on nonnegative
+        terms.  The merge term RN(RN(RN(delta^2) * r_n) * cn) / tot) has delta off by eta_k <= E_{k-1} + 6u + u R
+        (R: the range of the tile's probabilities, which bounds |delta|), so it moves by <= min(na, nb) (2 R eta_k +
+        eta_k^2) with min(na, nb) <= cn_k; its four roundings and the two additions into r_m2 are relative errors on
+        nonnegative terms, gamma_(2K + 12) overall with the final RN(r_m2 / r_n).
+      * std = sqrtf(var): |sqrt(a) - sqrt(b)| <= min(sqrt(|a - b|), |a - b| / sqrt(b)), and sqrtf's own rounding u.
+    Returns dp, e_mean and eta [K - 1] (eta_k, k = 1..K-1), each with a 2^-10 relative margin for the O(u^2) terms."""
+    K = (T + CHUNK - 1) // CHUNK
+    g = 1 + 2.0 ** -10
+    dp = (12 + 2 * C) * U * g
+    e_mean = (6 + 4 * (K - 1)) * U * g
+    eta = np.array([(13 + 4 * (k - 1)) * U * g for k in range(1, K)])
+    return dp, e_mean, eta
+
+
+def head_ref(h1: torch.Tensor, masks, ow, rate: float = 0.1, sites=(False, True, True), rows_per_block: int = 4096):
+    """Fused MC-dropout head (head_sm100.cuh) from the GPU's own hidden_0 output and injected keep-masks.
+
+    h1: bf16 values [n, W], or [n, T, W] when site 0 is on (hidden_0 is then per sample); masks: uint8 [n, T, n_sites,
+    mask_w] with the enabled sites in ascending order (mask_w = 2048 with site 0 on, else W); W and C are read from the
+    weights (`ow.hidden[1]`, `ow.w3`, `ow.b3`).  A disabled site has no mask and a scale of 1, as in the kernel
+    (`slot < 0`, `inv_keep1` / `inv_keep2`).
+
+    Per sample: the masked operand (exact), hidden_1 as the kernel's chain of K = 16 MMAs (mma_chain_bound), RN(* 1/(1-p)
+    or 1), RN(+ b2), ReLU and bf16 at both interval ends, the site-2 mask, the fp32 fma chain into the C prelogits,
+    RN(* 1/(1-p) or 1), RN(+ b3) bounded as logit differences (logit_diff_interval), then the softmax bound
+    (softmax_interval).  The statistics are then checked with the
+    fp32 allowances of head_slack.
+    -> dict with, per [n, C]: mean_lo / mean_hi (the GPU mean must lie inside), std_z / std_allow (|std - std_z| <=
+    std_allow); plo / phi [n, T, C] per sample, and T, K, the slack terms."""
     dev = ow.device
     f64 = torch.float64
-    inv_keep = float(np.float32(1.0) / (np.float32(1.0) - np.float32(rate)))
     W2, b2 = ow.hidden[1][0], ow.hidden[1][1].to(f64)
     W3, b3 = ow.w3.to(f64), ow.b3.to(f64)
-    h1 = h1.to(dev).to(f64)
-    m = torch.from_numpy(masks).to(dev).to(f64)
+    W, C = W2.shape[0], W3.shape[1]
+    masks = torch.as_tensor(masks).to(dev)
     n, T = masks.shape[:2]
-    plo_t, phi_t = [], []
-    for t in range(T):
-        a = h1 * m[:, t, 0, :h1.shape[1]]                                 # the masked operand: an exact selection
-        z2, E2 = mma_chain_bound(a, W2)
-        h2lo, h2hi = _round_interval(z2 - E2, z2 + E2, inv_keep, b2)
-        k2 = m[:, t, 1, :W2.shape[0]]
-        h2lo = rn_bf16(torch.clamp_min(h2lo, 0.0).to(torch.float32)).to(f64) * k2
-        h2hi = rn_bf16(torch.clamp_min(h2hi, 0.0).to(torch.float32)).to(f64) * k2
-        llo, lhi = _fma_chain_interval(h2lo, h2hi, W3)
-        zlo, zhi = _round_interval(llo, lhi, inv_keep, b3)
-        # 2 classes: p1 = sigmoid(z1 - z0) is monotone in the logit difference
-        dlo, dhi = zlo[:, 1] - zhi[:, 0], zhi[:, 1] - zlo[:, 0]
-        p1lo, p1hi = torch.sigmoid(dlo), torch.sigmoid(dhi)
-        plo_t.append(torch.stack([1 - p1hi, p1lo], 1))
-        phi_t.append(torch.stack([1 - p1lo, p1hi], 1))
-    plo, phi = torch.stack(plo_t), torch.stack(phi_t)                   # [T, n, 2]
+    slot, k = {}, 0
+    for i, on in enumerate(sites):
+        if on:
+            slot[i], k = k, k + 1
+    assert masks.shape[2] == k, (tuple(masks.shape), sites)
+    ik = inv_keep(rate)
+    ik1, ik2 = (ik if sites[1] else 1.0), (ik if sites[2] else 1.0)
+    h1 = torch.as_tensor(h1).to(dev, f64)
+    per_sample = h1.dim() == 3
+    assert per_sample == bool(sites[0]), "hidden_0 is per sample exactly when site 0 is on"
+    tb = max(1, rows_per_block // n)
+    plo_b, phi_b = [], []
+    for t0 in range(0, T, tb):
+        t1 = min(T, t0 + tb)
+        a = h1[:, t0:t1] if per_sample else h1[:, None, :].expand(n, t1 - t0, W)
+        if 1 in slot:
+            a = a * masks[:, t0:t1, slot[1], :W].to(f64)                  # the masked operand: an exact selection
+        z2, E2 = mma_chain_bound(a.reshape(-1, W), W2)
+        h2lo, h2hi = _round_interval(z2 - E2, z2 + E2, ik1, b2)
+        h2lo = rn_bf16(torch.clamp_min(h2lo, 0.0).to(torch.float32)).to(f64)
+        h2hi = rn_bf16(torch.clamp_min(h2hi, 0.0).to(torch.float32)).to(f64)
+        if 2 in slot:
+            k2 = masks[:, t0:t1, slot[2], :W].reshape(-1, W).to(f64)
+            h2lo, h2hi = h2lo * k2, h2hi * k2
+        plo, phi = softmax_interval(*logit_diff_interval(h2lo, h2hi, W3, b3, ik2))
+        plo_b.append(plo.reshape(n, t1 - t0, C))
+        phi_b.append(phi.reshape(n, t1 - t0, C))
+    plo, phi = torch.cat(plo_b, 1), torch.cat(phi_b, 1)                  # [n, T, C]
+    dp, e_mean, eta = head_slack(T, C)
+    K = (T + CHUNK - 1) // CHUNK
     pz = 0.5 * (plo + phi)
-    # fp32 softmax (expf: <= 2 ulp, a subtraction, a sum and a division) on probabilities <= 1, then the shuffle sums,
-    # one division and one sqrt; T > 32 adds Chan's merge of 32-sample chunks
-    slack = 2.0 ** -18 * (2 if T > 32 else 1)
-    # population std moves by at most the largest change of one sample
-    return dict(mean_lo=plo.mean(0), mean_hi=phi.mean(0), std_z=pz.std(0, unbiased=False),
-                std_w=torch.maximum(phi - pz, pz - plo).amax(0), slack=slack)
+    std_z = pz.std(1, unbiased=False)
+    # population std is 1-Lipschitz in the max norm: it moves by at most the largest change of one sample
+    lip = torch.maximum(phi - pz, pz - plo).amax(1) + dp
+    R = phi.amax(1) - plo.amin(1) + 2 * dp
+    cn = [min(CHUNK, T - CHUNK * k) for k in range(1, K)]
+    d_m2 = T * (7 * U) ** 2 + sum(c * (2 * R * e + e * e) for c, e in zip(cn, eta)) * (1 + 8 * U)
+    s_hi = std_z + lip
+    s_lo = torch.clamp_min(std_z - lip, 0.0)
+    d_var = d_m2 / T + s_hi ** 2 * (2 * K + 12) * U * (1 + 2.0 ** -10)
+    d_std = torch.minimum(torch.sqrt(d_var), d_var / s_lo) + 2 * U * s_hi + TINY
+    return dict(mean_lo=plo.mean(1) - dp - e_mean, mean_hi=phi.mean(1) + dp + e_mean, std_z=std_z,
+                std_allow=lip + d_std, plo=plo, phi=phi, T=T, K=K, dp=dp, e_mean=e_mean)
+
+
+def head_report(mean, std, h):
+    """GPU mean / std [n, C] against head_ref's result -> report dict: n_fail_mean, n_fail_std, width (the widest mean
+    interval), ratio_mean (max |mean - mid| / half-width), ratio_std (max |std - std_z| / allowed), and on a failure the
+    first failing (tile, class) with their intervals"""
+    dev = h["mean_lo"].device
+    mean = torch.as_tensor(np.asarray(mean)).to(dev, torch.float64)
+    std = torch.as_tensor(np.asarray(std)).to(dev, torch.float64)
+    lo, hi = h["mean_lo"], h["mean_hi"]
+    mid, half = 0.5 * (lo + hi), 0.5 * (hi - lo)
+    bad_m = (mean < lo) | (mean > hi) | torch.isnan(mean)
+    ds = (std - h["std_z"]).abs()
+    bad_s = (ds > h["std_allow"]) | torch.isnan(std)
+    rep = dict(n=int(mean.numel()), n_fail_mean=int(bad_m.sum()), n_fail_std=int(bad_s.sum()),
+               width=float((hi - lo).max()), ratio_mean=float(((mean - mid).abs() / half).max()),
+               ratio_std=float((ds / h["std_allow"]).max()), T=h["T"], K=h["K"], first=[])
+    for i, c in torch.nonzero(bad_m | bad_s)[:8].tolist():
+        rep["first"].append(dict(tile=i, cls=c, group=i // 4, quadrant=i % 4, mean=float(mean[i, c]),
+                                 mean_interval=(float(lo[i, c]), float(hi[i, c])), std=float(std[i, c]),
+                                 std_z=float(h["std_z"][i, c]), std_allow=float(h["std_allow"][i, c])))
+    return rep
 
 
 def check_head(mean, std, h):
-    """-> (n_fail_mean, n_fail_std, max |d std| / allowed)"""
-    mean = torch.as_tensor(mean).to(h["mean_lo"].device, torch.float64)
-    std = torch.as_tensor(std).to(h["mean_lo"].device, torch.float64)
-    bad_m = (mean < h["mean_lo"] - h["slack"]) | (mean > h["mean_hi"] + h["slack"])
-    allowed = h["std_w"] + h["slack"]
-    bad_s = (std - h["std_z"]).abs() > allowed
-    return int(bad_m.sum()), int(bad_s.sum()), float(((std - h["std_z"]).abs() / allowed).max())
+    """-> (n_fail_mean, n_fail_std, max |d std| / allowed); head_report has the details"""
+    rep = head_report(mean, std, h)
+    return rep["n_fail_mean"], rep["n_fail_std"], rep["ratio_std"]
+
+
+def describe_head(tag, rep):
+    """one line per failing (tile, class): the tile's four-tile group and TMEM quadrant, the value and its interval"""
+    s = (f"{tag}: {rep['n_fail_mean']} means and {rep['n_fail_std']} stds of {rep['n']} outside the bound "
+         f"(T = {rep['T']}, {rep['K']} sample chunks of 32)")
+    for f in rep["first"]:
+        s += (f"\n    tile {f['tile']} (group {f['group']}, quadrant {f['quadrant']}) class {f['cls']}: mean {f['mean']:.7f}"
+              f" in [{f['mean_interval'][0]:.7f}, {f['mean_interval'][1]:.7f}]?  std {f['std']:.7f} vs {f['std_z']:.7f}"
+              f" +- {f['std_allow']:.2e}")
+    return s

@@ -1,4 +1,4 @@
-"""Shared test helpers: golden decoding and bit-exact DataFrame / scalar comparison."""
+"""Shared test helpers: golden decoding, bit-exact DataFrame / scalar comparison, degenerate tiles."""
 import hashlib
 import json
 import os
@@ -63,3 +63,13 @@ def assert_same_results(a, b, what=""):
     assert set(a) == set(b), what
     for k in a:
         assert same_scalar(a[k], b[k]), f"{what}: {k}: {a[k]!r} ({type(a[k]).__name__}) vs {b[k]!r} ({type(b[k]).__name__})"
+
+
+def degenerate_tiles():
+    """4 tiles with large uniform regions (all-zero channels deep in the net)"""
+    t = np.zeros((4, 299, 299, 3), np.uint8)
+    t[0] = 255                                                          # white background
+    t[1] = 237                                                          # constant, odd value
+    t[2] = 200; t[2, 150, 150, 1] = 201                                 # a single pixel differs
+    t[3] = (np.indices((299, 299)).sum(0) % 2 * 255).astype(np.uint8)[..., None]   # checkerboard 0 / 255
+    return t

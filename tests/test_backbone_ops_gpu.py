@@ -16,20 +16,12 @@ import numpy as np
 import pytest
 import torch
 
+from helpers import degenerate_tiles
 from oracle import synth, xception_ops as XO, xception_uq as X
 
 pytestmark = pytest.mark.gpu
 
 PLANS = {"sepmid": XO.plan(True), "unfused": XO.plan(False)}
-
-
-def degenerate_tiles():
-    t = np.zeros((4, 299, 299, 3), np.uint8)
-    t[0] = 255                                                          # white background
-    t[1] = 237                                                          # constant, odd value
-    t[2] = 200; t[2, 150, 150, 1] = 201                                 # a single pixel differs
-    t[3] = (np.indices((299, 299)).sum(0) % 2 * 255).astype(np.uint8)[..., None]   # checkerboard 0 / 255
-    return t
 
 
 @pytest.fixture(scope="module")
