@@ -100,9 +100,13 @@ SIGNATURES = {
     "bq_jpeg_status_string": (C.c_char_p, [C.c_int32]),
     "bq_jpeg_inspect": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p]),
     "bq_jpeg_decode": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]),
+    "bq_jpeg_decode_ex": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p,
+                                    C.c_void_p]),
     "bq_jpeg_last_stats": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64)]),
     "bq_predict_uq_jpeg": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_uint64, C.c_uint64,
                                      C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "bq_predict_uq_jpeg_ex": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_uint64,
+                                        C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "bq_png_status_string": (C.c_char_p, [C.c_int32]),
     "bq_png_inspect": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p]),
     "bq_png_decode": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]),
@@ -115,6 +119,7 @@ SIGNATURES = {
 }
 
 BQ_ERR_DATA = -6
+BQ_JPEG_IDCT_IFAST, BQ_JPEG_REPLICATE_CHROMA = 1, 2
 
 _lib = None
 _lock = threading.Lock()

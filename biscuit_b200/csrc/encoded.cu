@@ -50,9 +50,12 @@ int bq_encoded::report(bq_ctx* ctx, const std::vector<int32_t>& st, int32_t* sta
 }
 
 int bq_encoded::prepare(bq_ctx* ctx, const uint8_t* data_, const int64_t* offsets, int64_t n_, int px_, int64_t group_,
-                        int32_t* status_host) {
+                        int32_t flags_, int32_t* status_host) {
   if (n_ < 0 || !px_ok(px_) || group_ < 1 || (n_ > 0 && (!data_ || !offsets)))
     return bq_fail(ctx, BQ_ERR_ARG, "bq_%s: bad argument", api().c_str());
+  if (flags_ & ~known_flags())
+    return bq_fail(ctx, BQ_ERR_ARG, "bq_%s: unknown decode flag bits 0x%x (known: 0x%x)", api().c_str(),
+                   (unsigned)(flags_ & ~known_flags()), (unsigned)known_flags());
   const int64_t cap = max_tile_bytes();
   for (int64_t i = 0; i < n_; ++i)
     if (offsets[i] < 0 || offsets[i + 1] < offsets[i] || offsets[i + 1] - offsets[i] > cap)
@@ -61,6 +64,7 @@ int bq_encoded::prepare(bq_ctx* ctx, const uint8_t* data_, const int64_t* offset
   data = data_;
   on_dev = n_ > 0 && bq_is_device_ptr(data_);
   px = px_;
+  flags = flags_;
   n = n_;
   group = group_;
   offs.assign(offsets, offsets + n + 1);
@@ -157,11 +161,11 @@ int bq_encoded_inspect(const bq_encoded& f, const uint8_t* data, const int64_t* 
 }
 
 int bq_encoded_decode(bq_ctx* ctx, bq_encoded* s, const uint8_t* data, const int64_t* offsets, int64_t n, int px,
-                      uint8_t* out_u8, int32_t* status) {
+                      int32_t flags, uint8_t* out_u8, int32_t* status) {
   if (n > 0 && !out_u8) return bq_fail(ctx, BQ_ERR_ARG, "bq_%s_decode: bad argument", s->api().c_str());
   BQ_CUDA(ctx, cudaSetDevice(ctx->device));
   constexpr int64_t kGroup = 512;
-  int rc = s->prepare(ctx, data, offsets, n, px, kGroup, status);
+  int rc = s->prepare(ctx, data, offsets, n, px, kGroup, flags, status);
   if (rc) return rc;
   const size_t tile_bytes = (size_t)px * px * 3;
   const bool out_dev = bq_is_device_ptr(out_u8);

@@ -24,6 +24,8 @@ struct bq_encoded {
   virtual bool px_ok(int px) const = 0;                        // tile sizes the kernels decode
   // Longest file the descriptor addresses; INT32_MAX when it holds a length in 32 bits ("tiles < 2 GB").
   virtual int64_t max_tile_bytes() const { return INT64_MAX; }
+  // Decode-option bits the format accepts in a call's `flags` (JPEG: BQ_JPEG_IDCT_IFAST | BQ_JPEG_REPLICATE_CHROMA).
+  virtual int32_t known_flags() const { return 0; }
   // Header parse of one file b[0, len) of which the first `avail` bytes are at hand (tail2 = its last two bytes):
   // fills the descriptor `desc` and returns the format's status code (0 = accepted), or kNeedMore.
   virtual int parse(const uint8_t* b, int64_t len, int64_t avail, const uint8_t* tail2, int px, void* desc) const = 0;
@@ -38,9 +40,10 @@ struct bq_encoded {
   virtual int finished(bq_ctx*) { return BQ_OK; }
 
   // ---- the driver (encoded.cu)
-  // Parse every tile (nothing is launched when one is rejected), lay out the groups and size the scratch.
+  // Parse every tile (nothing is launched when one is rejected), lay out the groups and size the scratch.  `flags` are
+  // the call's decode options; every call sets them, so none carries over to the next call on the same state.
   int prepare(bq_ctx* ctx, const uint8_t* data, const int64_t* offsets, int64_t n, int px, int64_t group,
-              int32_t* status_host);
+              int32_t flags, int32_t* status_host);
   // Copy group g's descriptors (and its bytes, when they are in host memory) into slot `slot` on `stream`.
   int upload(bq_ctx* ctx, int64_t g, int slot, cudaStream_t stream);
   // Decode group g (uploaded into `slot`) on the ctx stream into out = uint8 NHWC [group tiles, px, px, 3] (device).
@@ -56,6 +59,7 @@ struct bq_encoded {
   const uint8_t* data = nullptr;
   bool on_dev = false;
   int px = 0;
+  int32_t flags = 0;
   int64_t n = 0, group = 0;
   std::vector<int64_t> offs;
   void* desc_host = nullptr;           // pinned [n] descriptors
@@ -72,7 +76,7 @@ struct bq_encoded {
 int bq_encoded_inspect(const bq_encoded& f, const uint8_t* data, const int64_t* offsets, int64_t n, int px,
                        int32_t* status);
 int bq_encoded_decode(bq_ctx* ctx, bq_encoded* s, const uint8_t* data, const int64_t* offsets, int64_t n, int px,
-                      uint8_t* out_u8, int32_t* status);
+                      int32_t flags, uint8_t* out_u8, int32_t* status);
 
 // The JPEG (jpeg.cu) / PNG (png.cu) state kept in `slot`, created on first use.
 bq_encoded* bq_jpeg_state(bq_encoded*& slot);

@@ -204,6 +204,7 @@ struct Jpeg final : bq_encoded {
   int64_t last_stats[4] = {};
 
   const char* name() const override { return "JPEG"; }
+  int32_t known_flags() const override { return BQ_JPEG_IDCT_IFAST | BQ_JPEG_REPLICATE_CHROMA; }
   size_t desc_bytes() const override { return sizeof(Tile); }
   int head_bytes() const override { return 2048; }
   bool px_ok(int px) const override { return px >= 16 && px <= 4096; }
@@ -266,12 +267,16 @@ struct Jpeg final : bq_encoded {
                                                                     (int32_t*)ichunk.p, (J::Chunk*)chunks.p,
                                                                     (int16_t*)coef.p, status, st);
     BQ_LAUNCH_CHECK(ctx);
+    // this call's decode options (prepare sets them on every call) pick the instantiation; the grids do not depend on them
     const dim3 gi((unsigned)((max_tile_blocks + J::kIdctBlocks - 1) / J::kIdctBlocks), (unsigned)nb);
-    J::jpeg_idct_kernel<<<gi, J::kIdctThreads, 0, ctx->stream>>>(d, (const int16_t*)coef.p, status, (uint8_t*)planes.p,
-                                                                 pitch);
+    const auto idct = flags & BQ_JPEG_IDCT_IFAST ? J::jpeg_idct_kernel<J::Idct::kIfast>
+                                                 : J::jpeg_idct_kernel<J::Idct::kIslow>;
+    idct<<<gi, J::kIdctThreads, 0, ctx->stream>>>(d, (const int16_t*)coef.p, status, (uint8_t*)planes.p, pitch);
     BQ_LAUNCH_CHECK(ctx);
     const dim3 gc((unsigned)((px * px + 255) / 256), (unsigned)nb);
-    J::jpeg_color_kernel<<<gc, 256, 0, ctx->stream>>>(d, (const uint8_t*)planes.p, status, pitch, px, out);
+    const auto color = flags & BQ_JPEG_REPLICATE_CHROMA ? J::jpeg_color_kernel<J::Upsample::kReplicate>
+                                                        : J::jpeg_color_kernel<J::Upsample::kFancy>;
+    color<<<gc, 256, 0, ctx->stream>>>(d, (const uint8_t*)planes.p, status, pitch, px, out);
     BQ_LAUNCH_CHECK(ctx);
     return BQ_OK;
   }
@@ -305,7 +310,13 @@ int bq_jpeg_inspect(const uint8_t* data, const int64_t* offsets, int64_t n, int3
 
 int bq_jpeg_decode(bq_ctx* ctx, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t px, uint8_t* out_u8,
                    int32_t* status) {
-  return ctx ? bq_encoded_decode(ctx, bq_jpeg_state(ctx->jpeg), data, offsets, n, px, out_u8, status) : BQ_ERR_ARG;
+  return bq_jpeg_decode_ex(ctx, data, offsets, n, px, 0, out_u8, status);
+}
+
+int bq_jpeg_decode_ex(bq_ctx* ctx, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t px, int32_t flags,
+                      uint8_t* out_u8, int32_t* status) {
+  return ctx ? bq_encoded_decode(ctx, bq_jpeg_state(ctx->jpeg), data, offsets, n, px, flags, out_u8, status)
+             : BQ_ERR_ARG;
 }
 
 int bq_jpeg_last_stats(bq_ctx* ctx, int64_t stats[4]) {

@@ -1,11 +1,13 @@
-// Baseline-JPEG decode kernels (sm_100a), bit-exact with libjpeg-turbo's default decompression (JDCT_ISLOW, fancy
-// upsampling, jdcolor.c tables).  Included by jpeg.cu only.  Four launches per batch of tiles, one CTA per tile for the
-// first two:
+// Baseline-JPEG decode kernels (sm_100a), bit-exact with libjpeg-turbo's decompression (jdcolor.c tables) under the two
+// options TensorFlow's decode_jpeg exposes: the IDCT (JDCT_ISLOW, libjpeg-turbo's default, or JDCT_IFAST) and fancy or
+// replicated (merged) chroma upsampling.  Included by jpeg.cu only.  Four launches per batch of tiles, one CTA per tile
+// for the first two:
 //   (a) jpeg_unstuff_kernel   removes FF00 stuffing and RSTn markers, records where each restart interval starts;
 //   (b) jpeg_huffman_kernel   parallel Huffman decode by self-synchronising subsequences (Weissenberger & Schmidt,
 //                             ICPP 2018), then the DC prediction per component per restart interval;
-//   (c) jpeg_idct_kernel      dequantisation + ISLOW IDCT -> component planes;
-//   (d) jpeg_color_kernel     fancy upsampling + YCbCr->RGB + crop, NHWC uint8 into the caller's tile buffer.
+//   (c) jpeg_idct_kernel      dequantisation + ISLOW or IFAST IDCT -> component planes;
+//   (d) jpeg_color_kernel     fancy or replicated upsampling + YCbCr->RGB + crop, NHWC uint8 into the caller's tile
+//                             buffer.
 #pragma once
 
 #include <cub/block/block_scan.cuh>
@@ -450,11 +452,20 @@ __global__ void __launch_bounds__(kHuffThreads) jpeg_huffman_kernel(const Tile* 
 }
 
 // ------------------------------------------------------------------------------------------------------------------
-// (c) dequantisation + jidctint.c jpeg_idct_islow.  Eight threads per block: thread r transforms column r, then row r.
-// All arithmetic is exact integer; the range limit is the saturating one of libjpeg-turbo's SIMD IDCT, equal to the C
-// table lookup wherever |value| < 512.
+// (c) dequantisation + jidctint.c jpeg_idct_islow or jidctfst.c jpeg_idct_ifast.  Eight threads per block: thread r
+// transforms column r, then row r.  All arithmetic is exact integer; the range limit is the saturating one of
+// libjpeg-turbo's SIMD IDCT, equal to the C table lookup wherever |value| < 512.
 // ------------------------------------------------------------------------------------------------------------------
 constexpr int kIdctThreads = 256, kIdctBlocks = kIdctThreads / 8;
+
+enum class Idct { kIslow, kIfast };
+
+// jddctmgr.c aanscales (natural order): 16384 * s(row) * s(col), s(0) = 1, s(k) = sqrt(2) cos(k pi / 16)
+__constant__ int32_t kAanScales[64] = {
+    16384, 22725, 21407, 19266, 16384, 12873, 8867,  4520,  22725, 31521, 29692, 26722, 22725, 17855, 12299, 6270,
+    21407, 29692, 27969, 25172, 21407, 16819, 11585, 5906,  19266, 26722, 25172, 22654, 19266, 15137, 10426, 5315,
+    16384, 22725, 21407, 19266, 16384, 12873, 8867,  4520,  12873, 17855, 16819, 15137, 12873, 10114, 6967,  3552,
+    8867,  12299, 11585, 10426, 8867,  6967,  4799,  2446,  4520,  6270,  5906,  5315,  4520,  3552,  2446,  1247};
 
 __device__ __forceinline__ void islow_1d(int32_t i0, int32_t i1, int32_t i2, int32_t i3, int32_t i4, int32_t i5,
                                          int32_t i6, int32_t i7, int shift, int32_t* o) {
@@ -483,6 +494,40 @@ __device__ __forceinline__ void islow_1d(int32_t i0, int32_t i1, int32_t i2, int
   o[4] = (t13 - tmp0 + r) >> shift;
 }
 
+// jidctfst.c: CONST_BITS 8 multiplies that truncate (no USE_ACCURATE_ROUNDING); the product is taken in 64 bits as
+// libjpeg-turbo's JLONG is
+__device__ __forceinline__ int32_t ifast_mul(int32_t v, int32_t c) { return (int32_t)(((int64_t)v * c) >> 8); }
+
+// One jpeg_idct_ifast pass.  It keeps the scale of its input: the caller shifts the row pass right by PASS1_BITS + 3.
+__device__ __forceinline__ void ifast_1d(int32_t i0, int32_t i1, int32_t i2, int32_t i3, int32_t i4, int32_t i5,
+                                         int32_t i6, int32_t i7, int32_t* o) {
+  const int32_t t10 = i0 + i4, t11 = i0 - i4, t13 = i2 + i6;
+  const int32_t t12 = ifast_mul(i2 - i6, 362) - t13;
+  const int32_t e0 = t10 + t13, e3 = t10 - t13, e1 = t11 + t12, e2 = t11 - t12;
+  const int32_t z13 = i5 + i3, z10 = i5 - i3, z11 = i1 + i7, z12 = i1 - i7;
+  const int32_t o7 = z11 + z13;
+  const int32_t o11 = ifast_mul(z11 - z13, 362);
+  const int32_t z5 = ifast_mul(z10 + z12, 473);
+  const int32_t o10 = ifast_mul(z12, 277) - z5;
+  const int32_t o12 = ifast_mul(z10, -669) + z5;
+  const int32_t o6 = o12 - o7, o5 = o11 - o6, o4 = o10 + o5;
+  o[0] = e0 + o7;
+  o[7] = e0 - o7;
+  o[1] = e1 + o6;
+  o[6] = e1 - o6;
+  o[2] = e2 + o5;
+  o[5] = e2 - o5;
+  o[3] = e3 - o4;
+  o[4] = e3 + o4;
+}
+
+// jddctmgr.c: the IFAST multiplier of quantisation table entry i (natural order), DESCALE by 12 bits and the
+// IFAST_MULT_TYPE (short) cast.  q * aan < 2^31 for every 16-bit q.
+__device__ __forceinline__ int32_t ifast_multiplier(uint32_t q, int i) {
+  return (int16_t)((q * (uint32_t)kAanScales[i] + 2048u) >> 12);
+}
+
+template <Idct kMethod>
 __global__ void __launch_bounds__(kIdctThreads) jpeg_idct_kernel(const Tile* __restrict__ tiles,
                                                                   const int16_t* __restrict__ coef,
                                                                   const int32_t* __restrict__ status,
@@ -503,14 +548,27 @@ __global__ void __launch_bounds__(kIdctThreads) jpeg_idct_kernel(const Tile* __r
   const int16_t* cb = coef + ((size_t)t.coef_base + b) * 64;
   const uint16_t* q = t.qt[comp];
   int32_t in[8], out[8];
+  if constexpr (kMethod == Idct::kIslow) {
 #pragma unroll
-  for (int k = 0; k < 8; ++k) in[k] = (int32_t)cb[k * 8 + r] * (int32_t)q[k * 8 + r];
-  islow_1d(in[0], in[1], in[2], in[3], in[4], in[5], in[6], in[7], 11, out);
+    for (int k = 0; k < 8; ++k) in[k] = (int32_t)cb[k * 8 + r] * (int32_t)q[k * 8 + r];
+    islow_1d(in[0], in[1], in[2], in[3], in[4], in[5], in[6], in[7], 11, out);
+  } else {
+#pragma unroll
+    for (int k = 0; k < 8; ++k) in[k] = (int32_t)cb[k * 8 + r] * ifast_multiplier(q[k * 8 + r], k * 8 + r);
+    ifast_1d(in[0], in[1], in[2], in[3], in[4], in[5], in[6], in[7], out);
+  }
 #pragma unroll
   for (int k = 0; k < 8; ++k) ws[g][k][r] = out[k];
   __syncwarp(gmask);
-  islow_1d(ws[g][r][0], ws[g][r][1], ws[g][r][2], ws[g][r][3], ws[g][r][4], ws[g][r][5], ws[g][r][6], ws[g][r][7], 18,
-           out);
+  if constexpr (kMethod == Idct::kIslow) {
+    islow_1d(ws[g][r][0], ws[g][r][1], ws[g][r][2], ws[g][r][3], ws[g][r][4], ws[g][r][5], ws[g][r][6], ws[g][r][7],
+             18, out);
+  } else {
+    ifast_1d(ws[g][r][0], ws[g][r][1], ws[g][r][2], ws[g][r][3], ws[g][r][4], ws[g][r][5], ws[g][r][6], ws[g][r][7],
+             out);
+#pragma unroll
+    for (int k = 0; k < 8; ++k) out[k] >>= 5;           // PASS1_BITS + 3, truncating
+  }
   uint32_t lo = 0, hi = 0;
 #pragma unroll
   for (int k = 0; k < 4; ++k) {
@@ -522,11 +580,16 @@ __global__ void __launch_bounds__(kIdctThreads) jpeg_idct_kernel(const Tile* __r
 }
 
 // ------------------------------------------------------------------------------------------------------------------
-// (d) jdsample.c fancy upsampling (h2v1 / h2v2, edge samples replicated, odd widths cut at the downsampled width) and
-// jdcolor.c ycc_rgb_convert, one thread per output pixel.
+// (d) jdsample.c fancy upsampling (h2v1 / h2v2, edge samples replicated, odd widths cut at the downsampled width) or,
+// without fancy upsampling, jdmerge.c's replicated chroma (each chroma sample covers its 2x1 / 2x2 output pixels), and
+// jdcolor.c ycc_rgb_convert (jdmerge.c uses the same tables), one thread per output pixel.
 // ------------------------------------------------------------------------------------------------------------------
+enum class Upsample { kFancy, kReplicate };
+
+template <Upsample kUp>
 __device__ __forceinline__ int chroma(const uint8_t* p, int pitch, int mode, int y, int x, int dw, int dh) {
   if (mode == 0) return p[y * pitch + x];
+  if constexpr (kUp == Upsample::kReplicate) return p[(mode == 1 ? y : y >> 1) * pitch + (x >> 1)];
   const int i = x >> 1, odd = x & 1;
   const int ni = odd ? min(i + 1, dw - 1) : max(i - 1, 0);
   if (mode == 1) {
@@ -542,6 +605,7 @@ __device__ __forceinline__ int chroma(const uint8_t* p, int pitch, int mode, int
   return (3 * cs + cn + 8 - odd) >> 4;
 }
 
+template <Upsample kUp>
 __global__ void __launch_bounds__(256) jpeg_color_kernel(const Tile* __restrict__ tiles, const uint8_t* __restrict__ planes,
                                                          const int32_t* __restrict__ status, int pitch, int px,
                                                          uint8_t* __restrict__ out) {
@@ -556,8 +620,8 @@ __global__ void __launch_bounds__(256) jpeg_color_kernel(const Tile* __restrict_
   const int dw = (px + t.hmax - 1) / t.hmax, dh = (px + t.vmax - 1) / t.vmax;
   const uint8_t* p0 = planes + (size_t)tile * 3 * pitch * pitch;
   const int Y = p0[y * pitch + x];
-  const int cb = chroma(p0 + (size_t)pitch * pitch, pitch, mode, y, x, dw, dh) - 128;
-  const int cr = chroma(p0 + (size_t)2 * pitch * pitch, pitch, mode, y, x, dw, dh) - 128;
+  const int cb = chroma<kUp>(p0 + (size_t)pitch * pitch, pitch, mode, y, x, dw, dh) - 128;
+  const int cr = chroma<kUp>(p0 + (size_t)2 * pitch * pitch, pitch, mode, y, x, dw, dh) - 128;
   const int R = Y + ((91881 * cr + 32768) >> 16);
   const int G = Y + ((-46802 * cr - 22554 * cb + 32768) >> 16);
   const int B = Y + ((116130 * cb + 32768) >> 16);

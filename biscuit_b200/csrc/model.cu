@@ -1086,41 +1086,47 @@ int bq_model_load_weights(bq_model* m, const bq_named_tensor* tensors, int32_t n
 }
 
 // Input of predict_impl: decoded pixels (enc == NULL), or n compressed files back to back with n + 1 host byte offsets,
-// decoded through the format state `enc`.
+// decoded through the format state `enc` with the decode options `enc_flags`.
 static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, bq_encoded* enc, const int64_t* offsets,
-                        int64_t n, int32_t T, uint64_t seed, uint64_t tile_index_base, const uint8_t* masks, float* mean,
-                        float* std, float* features);
+                        int32_t enc_flags, int64_t n, int32_t T, uint64_t seed, uint64_t tile_index_base,
+                        const uint8_t* masks, float* mean, float* std, float* features);
 
 int bq_predict_uq(bq_model* m, const uint8_t* tiles, int64_t n, int32_t T, uint64_t seed, uint64_t tile_index_base,
                   const uint8_t* masks, float* mean, float* std, float* features) {
-  return predict_impl(m, tiles, false, nullptr, nullptr, n, T, seed, tile_index_base, masks, mean, std, features);
+  return predict_impl(m, tiles, false, nullptr, nullptr, 0, n, T, seed, tile_index_base, masks, mean, std, features);
 }
 
 int bq_predict_uq_jpeg(bq_model* m, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t T, uint64_t seed,
                        uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std, float* features) {
-  return predict_impl(m, data, false, m ? bq_jpeg_state(m->jpeg) : nullptr, offsets, n, T, seed, tile_index_base, masks,
-                      mean, std, features);
+  return bq_predict_uq_jpeg_ex(m, data, offsets, n, 0, T, seed, tile_index_base, masks, mean, std, features);
+}
+
+int bq_predict_uq_jpeg_ex(bq_model* m, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t flags, int32_t T,
+                          uint64_t seed, uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std,
+                          float* features) {
+  return predict_impl(m, data, false, m ? bq_jpeg_state(m->jpeg) : nullptr, offsets, flags, n, T, seed, tile_index_base,
+                      masks, mean, std, features);
 }
 
 int bq_predict_uq_png(bq_model* m, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t T, uint64_t seed,
                       uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std, float* features) {
-  return predict_impl(m, data, false, m ? bq_png_state(m->png) : nullptr, offsets, n, T, seed, tile_index_base, masks,
-                      mean, std, features);
+  return predict_impl(m, data, false, m ? bq_png_state(m->png) : nullptr, offsets, 0, n, T, seed, tile_index_base,
+                      masks, mean, std, features);
 }
 
 int bq_predict_uq_standardized(bq_model* m, const float* tiles, int64_t n, int32_t T, uint64_t seed, uint64_t tile_index_base,
                                const uint8_t* masks, float* mean, float* std, float* features) {
   if (!m) return BQ_ERR_ARG;
   m->input_f32 = true;
-  const int rc = predict_impl(m, (const uint8_t*)tiles, true, nullptr, nullptr, n, T, seed, tile_index_base,
+  const int rc = predict_impl(m, (const uint8_t*)tiles, true, nullptr, nullptr, 0, n, T, seed, tile_index_base,
                               masks, mean, std, features);
   m->input_f32 = false;
   return rc;
 }
 
 static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, bq_encoded* enc, const int64_t* offsets,
-                        int64_t n, int32_t T, uint64_t seed, uint64_t tile_index_base, const uint8_t* masks, float* mean,
-                        float* std, float* features) {
+                        int32_t enc_flags, int64_t n, int32_t T, uint64_t seed, uint64_t tile_index_base,
+                        const uint8_t* masks, float* mean, float* std, float* features) {
   if (!m) return BQ_ERR_ARG;
   bq_ctx* ctx = m->ctx;
   if (enc && n > 0 && !offsets)
@@ -1148,7 +1154,7 @@ static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, bq_en
   // is read in place) go up on the copy stream, and micro-batch i is decoded on the ctx stream into tiles_dev.
   const bool compressed = enc != nullptr;
   if (compressed) {
-    const int rcj = enc->prepare(ctx, tiles, offsets, n, m->px, B, nullptr);
+    const int rcj = enc->prepare(ctx, tiles, offsets, n, m->px, B, enc_flags, nullptr);
     if (rcj) return rcj;
   }
   const bool tiles_on_dev = !compressed && bq_is_device_ptr(tiles);

@@ -188,7 +188,7 @@ int bq_png_inspect(const uint8_t* data, const int64_t* offsets, int64_t n, int32
 
 int bq_png_decode(bq_ctx* ctx, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t px, uint8_t* out_u8,
                   int32_t* status) {
-  return ctx ? bq_encoded_decode(ctx, bq_png_state(ctx->png), data, offsets, n, px, out_u8, status) : BQ_ERR_ARG;
+  return ctx ? bq_encoded_decode(ctx, bq_png_state(ctx->png), data, offsets, n, px, 0, out_u8, status) : BQ_ERR_ARG;
 }
 
 }  // extern "C"

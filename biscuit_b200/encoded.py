@@ -15,6 +15,8 @@ class EncodedBatch:
     offsets: n + 1 non-decreasing int64 byte offsets (host)."""
 
     FORMAT: str          # "jpeg" / "png": the `bq_{FORMAT}_*` entry points that decode it
+    # decode options as the `flags` of the `bq_{FORMAT}_*_ex` entry points; None: the format has none
+    flags: int | None = None
 
     def __init__(self, data, offsets):
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
@@ -34,12 +36,16 @@ class EncodedBatch:
         self.offsets = offsets
 
     @classmethod
-    def from_bytes(cls, items):
-        """from a list of encoded files (bytes)"""
+    def from_bytes(cls, items, **options):
+        """from a list of encoded files (bytes); `options` are the subclass's decode options"""
         items = [bytes(b) for b in items]
         offsets = np.zeros(len(items) + 1, np.int64)
         offsets[1:] = np.cumsum([len(b) for b in items])
-        return cls(np.frombuffer(b"".join(items), np.uint8).copy(), offsets)
+        return cls(np.frombuffer(b"".join(items), np.uint8).copy(), offsets, **options)
+
+    def options(self) -> dict:
+        """the constructor's decode-option arguments of this batch"""
+        return {}
 
     def __len__(self) -> int:
         return int(self.offsets.size - 1)
@@ -58,9 +64,9 @@ class EncodedBatch:
         return bytes(chunk.cpu().numpy()) if self.on_device else chunk.tobytes()
 
     def cuda(self, device: int | None = None):
-        """the same batch (same class) with its bytes in device memory"""
+        """the same batch (same class, same decode options) with its bytes in device memory"""
         import torch
-        return type(self)(torch.from_numpy(np.asarray(self.data)).cuda(device), self.offsets)
+        return type(self)(torch.from_numpy(np.asarray(self.data)).cuda(device), self.offsets, **self.options())
 
 
 def status_message(fmt: str, code: int) -> str:
@@ -95,7 +101,13 @@ def decode(fmt: str, batch: EncodedBatch, px: int, ctx: _ffi.Context | None, out
     if isinstance(out, np.ndarray) and not out.flags.c_contiguous:
         raise ValueError("out must be C-contiguous")
     st = np.zeros(n, np.int32)
-    entry = getattr(ctx.lib, f"bq_{fmt}_decode")
-    _ffi.check(ctx.handle, entry(ctx.handle, _ffi.ptr(batch.data), _ffi.ptr(batch.offsets), n, int(px), _ffi.ptr(out),
-                                 _ffi.ptr(st)), f"bq_{fmt}_decode")
+    name, flags = entry_point(f"bq_{fmt}_decode", batch)
+    _ffi.check(ctx.handle, getattr(ctx.lib, name)(ctx.handle, _ffi.ptr(batch.data), _ffi.ptr(batch.offsets), n, int(px),
+                                                  *flags, _ffi.ptr(out), _ffi.ptr(st)), name)
     return out
+
+
+def entry_point(name: str, batch: EncodedBatch):
+    """(entry point, extra arguments) that decode `batch` with its options: `name` itself, or `name`_ex and its
+    flags argument"""
+    return (name, ()) if batch.flags is None else (name + "_ex", (int(batch.flags),))

@@ -13,7 +13,7 @@ import os
 import numpy as np
 
 from . import _ffi
-from .jpeg import JpegBatch
+from .jpeg import JpegBatch, check_dct_method
 from .png import SIGNATURE as PNG_SIGNATURE
 from .png import PngBatch
 
@@ -44,12 +44,17 @@ def scan(buf, image_key="image_raw", slide_key="slide", x_key="loc_x", y_key="lo
         cap = n.value
 
 
-def read(paths, image_key="image_raw", slide_key="slide", x_key="loc_x", y_key="loc_y"):
+def read(paths, image_key="image_raw", slide_key="slide", x_key="loc_x", y_key="loc_y",
+         dct_method="INTEGER_ACCURATE", fancy_upscaling=True):
     """(batch, slides, loc_x, loc_y) over the records of `paths` (one path or a list), in file order.
     batch: a PngBatch when every image starts with the PNG signature, else a JpegBatch (whatever is not JPEG then fails
     in the JPEG decoder, naming the tile).  A set that mixes PNG with other images raises ValueError naming the first
     record (file, index in the file) whose format differs from record 0.  slides: list of str (UTF-8); loc_x / loc_y:
-    int64 arrays."""
+    int64 arrays.
+    dct_method / fancy_upscaling: the JpegBatch's decode options, as in `tf.image.decode_jpeg`
+    (`dct_method="INTEGER_FAST"` decodes as TensorFlow does by default).  A PngBatch ignores them: PNG is lossless and
+    `decode_png` has no such options."""
+    check_dct_method(dct_method)
     if isinstance(paths, (str, os.PathLike)):
         paths = [paths]
     parts, sizes, slides, locs = [], [], [], []
@@ -74,7 +79,8 @@ def read(paths, image_key="image_raw", slide_key="slide", x_key="loc_x", y_key="
     offsets[1:] = np.cumsum(sizes)
     data = np.concatenate(parts) if parts else np.zeros(0, np.uint8)
     loc = np.concatenate(locs) if locs else np.zeros((0, 2), np.int64)
-    return (PngBatch if first_png else JpegBatch)(data, offsets), slides, loc[:, 0].copy(), loc[:, 1].copy()
+    batch = PngBatch(data, offsets) if first_png else JpegBatch(data, offsets, dct_method, fancy_upscaling)
+    return batch, slides, loc[:, 0].copy(), loc[:, 1].copy()
 
 
 def crc32c(b) -> int:

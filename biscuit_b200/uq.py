@@ -24,7 +24,7 @@ import pandas as pd
 
 from . import _ffi
 from .hp import ModelConfig, nature2022
-from .encoded import EncodedBatch
+from .encoded import EncodedBatch, entry_point
 from .utils import uncertainty_header, y_pred_header, y_true_header
 
 FEATURES = 2048
@@ -128,8 +128,8 @@ class UncertaintyInterface:
         """tiles: NHWC [n, 299, 299, 3] -- uint8 raw RGB (decode + per-image standardisation fused into the first
         convolution), or float32 ALREADY passed through `tf.image.per_image_standardization` as the reference's call site
         does (results.py:255-257); numpy, or a CUDA torch tensor used in place.  Or a `jpeg.JpegBatch` / `png.PngBatch`
-        of JPEG / PNG tiles, decoded on the GPU in front of the backbone: the results equal `predict` on the decoded
-        uint8 tiles bit for bit.
+        of JPEG / PNG tiles, decoded on the GPU in front of the backbone (a JpegBatch with its `dct_method` /
+        `fancy_upscaling`): the results equal `predict` on the decoded uint8 tiles bit for bit.
         Returns (mean [n, C], std [n, C]) float32 -- population std over T dropout samples."""
         T = int(T or self.num_uq)
         encoded = tiles.FORMAT if isinstance(tiles, EncodedBatch) else None
@@ -160,9 +160,10 @@ class UncertaintyInterface:
             if isinstance(masks, np.ndarray):
                 masks = np.ascontiguousarray(masks, dtype=np.uint8)
         if encoded:
-            entry = getattr(self.lib, f"bq_predict_uq_{encoded}")
-            rc = entry(self.h, _ffi.ptr(tiles.data), _ffi.ptr(tiles.offsets), n, T, C.c_uint64(seed),
-                       C.c_uint64(tile_index_base), _ffi.ptr(masks), _ffi.ptr(mean), _ffi.ptr(std), _ffi.ptr(feats))
+            name, flags = entry_point(f"bq_predict_uq_{encoded}", tiles)
+            rc = getattr(self.lib, name)(self.h, _ffi.ptr(tiles.data), _ffi.ptr(tiles.offsets), n, *flags, T,
+                                         C.c_uint64(seed), C.c_uint64(tile_index_base), _ffi.ptr(masks), _ffi.ptr(mean),
+                                         _ffi.ptr(std), _ffi.ptr(feats))
         else:
             entry = self.lib.bq_predict_uq if dt == "uint8" else self.lib.bq_predict_uq_standardized
             rc = entry(self.h, _ffi.ptr(tiles), n, T, C.c_uint64(seed), C.c_uint64(tile_index_base), _ffi.ptr(masks),
@@ -262,7 +263,9 @@ def predict_tfrecords(interface: UncertaintyInterface, paths, y_true=None, outco
     """`predict_table` straight from Slideflow tile TFRecords: the records of `paths` in file order, JPEG or PNG tiles
     decoded on the GPU.  Tile indices of the dropout streams run across files, so the table equals one `predict_table` over all
     tiles.  y_true: per-tile labels, or a dict slide -> label.  Adds the `loc_x` / `loc_y` columns of each tile.
-    `keys` overrides the feature names (`image_key`, `slide_key`, `x_key`, `y_key`; see `tfrecord.read`)."""
+    `keys` goes to `tfrecord.read`: the feature names (`image_key`, `slide_key`, `x_key`, `y_key`) and the JPEG decode
+    options `dct_method` / `fancy_upscaling` (as in `tf.image.decode_jpeg`; `dct_method="INTEGER_FAST"` selects the
+    IDCT `decode_jpeg` uses by default, on whose output Slideflow TensorFlow models were trained; ignored for PNG)."""
     from . import tfrecord
     batch, slides, loc_x, loc_y = tfrecord.read(paths, **keys)
     if isinstance(y_true, dict):

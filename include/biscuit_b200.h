@@ -259,8 +259,15 @@ int bq_model_set_normalizer(bq_model* m, int32_t kind, const float target_means[
 /* ------------------------------------------------------------------------------------------------
  * compressed tiles: baseline JPEG decode on the GPU and TFRecord reading
  *   replaces the host side of Slideflow's evaluate route (TFRecord read + per-tile JPEG decode in front of
- *   interface(batch)).  Decoded pixels equal libjpeg-turbo's default decompression byte for byte (JDCT_ISLOW,
- *   fancy upsampling, jdcolor.c YCbCr->RGB), i.e. PIL.Image.open(...).convert("RGB").
+ *   interface(batch)).  By default (flags = 0) decoded pixels equal libjpeg-turbo's default decompression byte for byte
+ *   (JDCT_ISLOW, fancy upsampling, jdcolor.c YCbCr->RGB), i.e. PIL.Image.open(...).convert("RGB").  The flags of the
+ *   _ex entry points select the two decode options TensorFlow's decode_jpeg exposes, per call:
+ *     BQ_JPEG_IDCT_IFAST        libjpeg-turbo's JDCT_IFAST IDCT (jidctfst.c) instead of JDCT_ISLOW; TensorFlow's
+ *                               dct_method "INTEGER_FAST", and what its default dct_method "" selects;
+ *     BQ_JPEG_REPLICATE_CHROMA  4:2:2 / 4:2:0 chroma replicated (jdmerge.c) instead of fancy upsampling;
+ *                               TensorFlow's fancy_upscaling=False.  No effect on 4:4:4 tiles.
+ *   With both, pixels equal libjpeg-turbo's decode with dct_method = JDCT_IFAST and do_fancy_upsampling = FALSE byte
+ *   for byte.  Any other flag bit fails the call with BQ_ERR_ARG before anything is launched.
  *   Tiles are n JPEG files back to back: tile i = data[offsets[i], offsets[i + 1]); offsets is always host memory.
  *   Accepted: SOF0 / SOF1 8-bit Huffman, one interleaved scan of 3 components (YCbCr), sampling 4:4:4, 4:2:2 or 4:2:0,
  *   any DQT / DHT, restart intervals, APPn / COM segments (skipped), size px x px.
@@ -288,6 +295,11 @@ enum {
   BQ_JPEG_INVALID_CODE = 21,       /* a Huffman code that is in no table                               */
   BQ_JPEG_TRUNCATED_DATA = 22      /* the scan ends before its last MCU                                */
 };
+/* decode options of bq_jpeg_decode_ex / bq_predict_uq_jpeg_ex (see above) */
+enum {
+  BQ_JPEG_IDCT_IFAST = 1,
+  BQ_JPEG_REPLICATE_CHROMA = 2
+};
 /* one line of text per status code above */
 const char* bq_jpeg_status_string(int32_t status);
 /* Host only, no device needed: the marker parse bq_jpeg_decode runs first.  status[i] = BQ_JPEG_* of tile i.
@@ -299,6 +311,10 @@ int bq_jpeg_inspect(const uint8_t* data, const int64_t* offsets, int64_t n, int3
  * BQ_ERR_DATA after the batch (the other tiles are decoded; the rejected tile's pixels are 0). */
 int bq_jpeg_decode(bq_ctx* ctx, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t px, uint8_t* out_u8,
                    int32_t* status);
+/* bq_jpeg_decode with decode options: flags = BQ_JPEG_IDCT_IFAST | BQ_JPEG_REPLICATE_CHROMA or a subset (0 is
+ * bq_jpeg_decode).  The options apply to this call only. */
+int bq_jpeg_decode_ex(bq_ctx* ctx, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t px, int32_t flags,
+                      uint8_t* out_u8, int32_t* status);
 /* Subsequence statistics of the last bq_jpeg_decode on ctx, summed over its tiles: {tiles, subsequences,
  * synchronisation rounds (max over tiles), subsequences decoded again}. */
 int bq_jpeg_last_stats(bq_ctx* ctx, int64_t stats[4]);
@@ -307,6 +323,10 @@ int bq_jpeg_last_stats(bq_ctx* ctx, int64_t stats[4]);
  * micro-batch buffer the uint8 path stages into. */
 int bq_predict_uq_jpeg(bq_model* m, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t T, uint64_t seed,
                        uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std, float* features);
+/* bq_predict_uq_jpeg with the decode options of bq_jpeg_decode_ex (0 is bq_predict_uq_jpeg), for this call only. */
+int bq_predict_uq_jpeg_ex(bq_model* m, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t flags, int32_t T,
+                          uint64_t seed, uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std,
+                          float* features);
 
 /* PNG tiles, decoded on the GPU: the pixels equal PIL.Image.open(...).convert("RGB") (PNG is lossless, so also
  * TensorFlow's decode_png).  Same layout as the JPEG entry points: tile i = data[offsets[i], offsets[i + 1]), offsets

@@ -1,15 +1,20 @@
 """Compressed-tile input on one GPU: decode kernel times, subsequence statistics and end-to-end MC-dropout throughput of
 `predict(JpegBatch)` against `predict(uint8)`, plus the host's own Pillow decode rate.
 
-    python profiles/jpeg_bench.py [--tiles 10000] [--T 30] [--reps 3] [--out results.json]
+    python profiles/jpeg_bench.py [--tiles 10000] [--T 30] [--reps 3] [--dct-method INTEGER_ACCURATE INTEGER_FAST]
+                                  [--out results.json]
 
 Two encodings: quality 90 4:2:0 (Pillow's default sampling) and quality 100 4:4:4 (the synthetic worst case).  The
 10 k-tile inputs cycle 503 distinct `synth.tiles_u8` tiles, so one pass reads more bytes than the 126 MB L2 holds at
 quality 100 (and 0.34 GB at quality 90).  The two inputs kinds alternate within one run, pinned and pageable.
+`--dct-method` lists the IDCTs to measure (`JpegBatch(dct_method=...)`, fancy upsampling on, as in TensorFlow's
+decode_jpeg defaults); with more than one, the JPEG inputs of every method alternate in the same end-to-end loop and the
+results carry the method in their keys (`decode_ms_per_503` -> `decode_ms_per_503_INTEGER_FAST`, ...).
 """
 from __future__ import annotations
 
 import argparse
+import itertools
 import json
 import multiprocessing as mp
 import os
@@ -79,6 +84,7 @@ def main():
     ap.add_argument("--T", type=int, default=30)
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--pil-tiles", type=int, default=4000)
+    ap.add_argument("--dct-method", nargs="+", default=["INTEGER_ACCURATE"], choices=("INTEGER_ACCURATE", "INTEGER_FAST"))
     ap.add_argument("--out", default=None, help="also write the result JSON to this file")
     a = ap.parse_args()
 
@@ -94,36 +100,41 @@ def main():
     q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", "0"],
                        capture_output=True, text=True).stdout.strip()
     res = dict(gpu=q or torch.cuda.get_device_name(0), tiles=a.tiles, T=a.T, micro_batch=uq.BENCH_MICRO_BATCH,
-               host_cpus=os.cpu_count(), configs={})
+               host_cpus=os.cpu_count(), dct_methods=a.dct_method, configs={})
+    methods = {m: ("" if len(a.dct_method) == 1 else "_" + m) for m in a.dct_method}     # method -> key suffix
     ctx = _ffi.default_context(0)
     base = synth.tiles_u8(uq.BENCH_MICRO_BATCH, seed=7, n_slides=8)
     iface = uq.UncertaintyInterface(random_init(seed=1), max_batch=uq.BENCH_MICRO_BATCH, ctx=ctx)
     for name, quality, ss in CONFIGS:
         files = [jpeg_synth.jpeg_encode(t, quality, ss) for t in base]
-        mb = JpegBatch.from_bytes(files)
-        r = dict(bytes_per_tile=mb.nbytes / len(mb))
-        split = kernel_split(mb.cuda(), ctx)
-        st = jpeg.last_stats(ctx)
-        r["decode_ms_per_503"] = split
-        r["huffman_ms"] = split["unstuff"] + split["huffman"]
-        r["idct_color_ms"] = split["idct"] + split["color"]
-        r["decode_tiles_per_s"] = len(mb) / (split["call"] / 1e3)
-        r["decode_compressed_GBps"] = mb.nbytes / (split["call"] / 1e3) / 1e9
-        r["sync"] = dict(st, subsequences_per_tile=st["subsequences"] / max(1, st["tiles"]),
-                         redecoded_share=st["redecoded"] / max(1, st["subsequences"]))
-
+        r = {}
         idx = np.arange(a.tiles) % len(files)
         big = JpegBatch.from_bytes([files[i] for i in idx])
-        pixels = np.stack([jpeg_synth.pil_decode(b) for b in files])[idx]
-        pin_px = torch.empty(pixels.shape, dtype=torch.uint8).pin_memory().numpy()
-        pin_px[...] = pixels
         pin_data = torch.empty(big.data.shape, dtype=torch.uint8).pin_memory().numpy()
         pin_data[...] = big.data
-        inputs = {"uint8_pinned": pin_px, "jpeg_pinned": JpegBatch(pin_data, big.offsets),
-                  "uint8_pageable": pixels, "jpeg_pageable": big}
+        inputs = {}
+        for m, sfx in methods.items():
+            mb = JpegBatch.from_bytes(files, dct_method=m)
+            r["bytes_per_tile"] = mb.nbytes / len(mb)
+            split = kernel_split(mb.cuda(), ctx)
+            st = jpeg.last_stats(ctx)
+            r["decode_ms_per_503" + sfx] = split
+            r["huffman_ms" + sfx] = split["unstuff"] + split["huffman"]
+            r["idct_color_ms" + sfx] = split["idct"] + split["color"]
+            r["decode_tiles_per_s" + sfx] = len(mb) / (split["call"] / 1e3)
+            r["decode_compressed_GBps" + sfx] = mb.nbytes / (split["call"] / 1e3) / 1e9
+            r["sync"] = dict(st, subsequences_per_tile=st["subsequences"] / max(1, st["tiles"]),    # the same for
+                             redecoded_share=st["redecoded"] / max(1, st["subsequences"]))     # every method
+            # the uint8 route gets the pixels of the same decode (Pillow's for the default IDCT)
+            px = np.stack([jpeg_synth.pil_decode(b) for b in files]) if m == "INTEGER_ACCURATE" else jpeg.decode(mb, ctx=ctx)
+            px = px[idx]
+            pin_px = torch.empty(px.shape, dtype=torch.uint8).pin_memory().numpy()
+            pin_px[...] = px
+            inputs.update({"uint8_pinned" + sfx: pin_px, "jpeg_pinned" + sfx: JpegBatch(pin_data, big.offsets, m),
+                           "uint8_pageable" + sfx: px, "jpeg_pageable" + sfx: JpegBatch(big.data, big.offsets, m)})
         for k, x in inputs.items():                     # warm-up: every shape / route once
             iface.predict(x[:uq.BENCH_MICRO_BATCH] if k.startswith("uint8") else
-                          JpegBatch(x.data, x.offsets[:uq.BENCH_MICRO_BATCH + 1]), T=a.T, seed=0)
+                          JpegBatch(x.data, x.offsets[:uq.BENCH_MICRO_BATCH + 1], **x.options()), T=a.T, seed=0)
         times = {k: [] for k in inputs}
         outs = {}
         for _ in range(a.reps):
@@ -134,10 +145,11 @@ def main():
                 times[k].append(time.perf_counter() - t)
         r["e2e_tiles_per_s"] = {k: a.tiles / float(np.median(v)) for k, v in times.items()}
         r["e2e_spread"] = {k: [round(a.tiles / t) for t in v] for k, v in times.items()}
-        for kind in ("pinned", "pageable"):
-            r[f"jpeg_over_uint8_{kind}"] = r["e2e_tiles_per_s"][f"jpeg_{kind}"] / r["e2e_tiles_per_s"][f"uint8_{kind}"]
-            assert np.array_equal(outs[f"jpeg_{kind}"][0], outs[f"uint8_{kind}"][0])
-            assert np.array_equal(outs[f"jpeg_{kind}"][1], outs[f"uint8_{kind}"][1])
+        for kind, sfx in itertools.product(("pinned", "pageable"), methods.values()):
+            j, u = f"jpeg_{kind}{sfx}", f"uint8_{kind}{sfx}"
+            r[f"jpeg_over_uint8_{kind}{sfx}"] = r["e2e_tiles_per_s"][j] / r["e2e_tiles_per_s"][u]
+            assert np.array_equal(outs[j][0], outs[u][0])
+            assert np.array_equal(outs[j][1], outs[u][1])
         pil_files = [files[i % len(files)] for i in range(a.pil_tiles)]
         r["host_pil_tiles_per_s"] = host_pil_rate(pil_files, os.cpu_count() or 1)
         res["configs"][name] = r
