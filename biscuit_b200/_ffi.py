@@ -110,8 +110,13 @@ SIGNATURES = {
     "bq_png_status_string": (C.c_char_p, [C.c_int32]),
     "bq_png_inspect": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p]),
     "bq_png_decode": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]),
+    "bq_png_inspect_ex": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p]),
+    "bq_png_decode_ex": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p,
+                                   C.c_void_p]),
     "bq_predict_uq_png": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_uint64, C.c_uint64,
                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "bq_predict_uq_png_ex": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_uint64,
+                                       C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "bq_tfrecord_scan": (C.c_int, [C.c_void_p, C.c_int64, C.c_char_p, C.c_char_p, C.c_char_p, C.c_char_p, C.c_int64,
                                    C.POINTER(C.c_int64), C.c_void_p, C.c_void_p, C.c_void_p, C.c_char_p, C.c_int64]),
     "bq_crc32c": (C.c_uint32, [C.c_void_p, C.c_int64]),
@@ -120,6 +125,7 @@ SIGNATURES = {
 
 BQ_ERR_DATA = -6
 BQ_JPEG_IDCT_IFAST, BQ_JPEG_REPLICATE_CHROMA = 1, 2
+BQ_PNG_CONVERT_RGB = 1
 
 _lib = None
 _lock = threading.Lock()

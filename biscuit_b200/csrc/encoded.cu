@@ -29,9 +29,9 @@ __global__ void gather_heads_kernel(const uint8_t* __restrict__ data, const int6
 
 namespace {
 
-int parse_host(const bq_encoded& f, const uint8_t* b, int64_t len, int px, void* desc) {
+int parse_host(const bq_encoded& f, const uint8_t* b, int64_t len, int px, int32_t flags, void* desc) {
   const uint8_t tail[2] = {len >= 2 ? b[len - 2] : (uint8_t)0, len >= 1 ? b[len - 1] : (uint8_t)0};
-  return f.parse(b, len, len, tail, px, desc);
+  return f.parse(b, len, len, tail, px, flags, desc);
 }
 
 }  // namespace
@@ -80,7 +80,7 @@ int bq_encoded::prepare(bq_ctx* ctx, const uint8_t* data_, const int64_t* offset
   std::vector<int32_t> st((size_t)n, 0);
   if (!on_dev) {
     for (int64_t i = 0; i < n; ++i)
-      st[i] = parse_host(*this, data + offsets[i], offsets[i + 1] - offsets[i], px, d + i * db);
+      st[i] = parse_host(*this, data + offsets[i], offsets[i + 1] - offsets[i], px, flags, d + i * db);
   } else if (n > 0) {
     // device bytes: fetch each tile's first `head` bytes and last two; parse again from the whole tile when the headers
     // run past the head (large APPn segments, a large iCCP chunk)
@@ -98,11 +98,11 @@ int bq_encoded::prepare(bq_ctx* ctx, const uint8_t* data_, const int64_t* offset
     for (int64_t i = 0; i < n; ++i) {
       const int64_t len = offsets[i + 1] - offsets[i];
       const uint8_t* h = h_all.data() + (size_t)i * (head + 2);
-      st[i] = parse(h, len, std::min<int64_t>(len, head), h + head, px, d + i * db);
+      st[i] = parse(h, len, std::min<int64_t>(len, head), h + head, px, flags, d + i * db);
       if (st[i] == kNeedMore) {
         whole.resize((size_t)len);
         BQ_CUDA(ctx, cudaMemcpy(whole.data(), data + offsets[i], (size_t)len, cudaMemcpyDeviceToHost));
-        st[i] = parse(whole.data(), len, len, h + head, px, d + i * db);
+        st[i] = parse(whole.data(), len, len, h + head, px, flags, d + i * db);
       }
     }
   }
@@ -149,13 +149,13 @@ int bq_encoded::finish(bq_ctx* ctx, int32_t* status_host) {
 }
 
 int bq_encoded_inspect(const bq_encoded& f, const uint8_t* data, const int64_t* offsets, int64_t n, int px,
-                       int32_t* status) {
-  if (n < 0 || !status || (n > 0 && (!data || !offsets))) return BQ_ERR_ARG;
+                       int32_t flags, int32_t* status) {
+  if (n < 0 || !status || (n > 0 && (!data || !offsets)) || (flags & ~f.known_flags())) return BQ_ERR_ARG;
   std::vector<uint8_t> desc(f.desc_bytes());
   for (int64_t i = 0; i < n; ++i) {
     const int64_t len = offsets[i + 1] - offsets[i];
     if (offsets[i] < 0 || len < 0) return BQ_ERR_ARG;
-    status[i] = parse_host(f, data + offsets[i], len, px, desc.data());
+    status[i] = parse_host(f, data + offsets[i], len, px, flags, desc.data());
   }
   return BQ_OK;
 }

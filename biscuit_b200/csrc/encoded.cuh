@@ -24,11 +24,14 @@ struct bq_encoded {
   virtual bool px_ok(int px) const = 0;                        // tile sizes the kernels decode
   // Longest file the descriptor addresses; INT32_MAX when it holds a length in 32 bits ("tiles < 2 GB").
   virtual int64_t max_tile_bytes() const { return INT64_MAX; }
-  // Decode-option bits the format accepts in a call's `flags` (JPEG: BQ_JPEG_IDCT_IFAST | BQ_JPEG_REPLICATE_CHROMA).
+  // Decode-option bits the format accepts in a call's `flags` (JPEG: BQ_JPEG_IDCT_IFAST | BQ_JPEG_REPLICATE_CHROMA;
+  // PNG: BQ_PNG_CONVERT_RGB).
   virtual int32_t known_flags() const { return 0; }
-  // Header parse of one file b[0, len) of which the first `avail` bytes are at hand (tail2 = its last two bytes):
-  // fills the descriptor `desc` and returns the format's status code (0 = accepted), or kNeedMore.
-  virtual int parse(const uint8_t* b, int64_t len, int64_t avail, const uint8_t* tail2, int px, void* desc) const = 0;
+  // Header parse of one file b[0, len) of which the first `avail` bytes are at hand (tail2 = its last two bytes) under
+  // the call's decode options `flags`: fills the descriptor `desc` and returns the format's status code (0 =
+  // accepted), or kNeedMore.
+  virtual int parse(const uint8_t* b, int64_t len, int64_t avail, const uint8_t* tail2, int px, int32_t flags,
+                    void* desc) const = 0;
   virtual const char* status_string(int32_t code) const = 0;
   // After a successful parse: rebase every group's descriptors to its group, size and allocate the format's scratch.
   virtual int layout(bq_ctx* ctx) = 0;
@@ -74,7 +77,7 @@ struct bq_encoded {
 
 // Bodies of bq_{jpeg,png}_inspect and bq_{jpeg,png}_decode (ctx != NULL); decode stages groups of 512 tiles.
 int bq_encoded_inspect(const bq_encoded& f, const uint8_t* data, const int64_t* offsets, int64_t n, int px,
-                       int32_t* status);
+                       int32_t flags, int32_t* status);
 int bq_encoded_decode(bq_ctx* ctx, bq_encoded* s, const uint8_t* data, const int64_t* offsets, int64_t n, int px,
                       int32_t flags, uint8_t* out_u8, int32_t* status);
 

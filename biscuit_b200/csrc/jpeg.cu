@@ -208,7 +208,8 @@ struct Jpeg final : bq_encoded {
   size_t desc_bytes() const override { return sizeof(Tile); }
   int head_bytes() const override { return 2048; }
   bool px_ok(int px) const override { return px >= 16 && px <= 4096; }
-  int parse(const uint8_t* b, int64_t len, int64_t avail, const uint8_t* tail2, int px, void* desc) const override {
+  int parse(const uint8_t* b, int64_t len, int64_t avail, const uint8_t* tail2, int px, int32_t,
+            void* desc) const override {
     return parse_tile(b, len, avail, tail2, px, *(Tile*)desc);
   }
   const char* status_string(int32_t code) const override { return ::status_string(code); }
@@ -305,7 +306,7 @@ extern "C" {
 const char* bq_jpeg_status_string(int32_t status) { return status_string(status); }
 
 int bq_jpeg_inspect(const uint8_t* data, const int64_t* offsets, int64_t n, int32_t px, int32_t* status) {
-  return bq_encoded_inspect(Jpeg(), data, offsets, n, px, status);
+  return bq_encoded_inspect(Jpeg(), data, offsets, n, px, 0, status);
 }
 
 int bq_jpeg_decode(bq_ctx* ctx, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t px, uint8_t* out_u8,

@@ -1110,7 +1110,13 @@ int bq_predict_uq_jpeg_ex(bq_model* m, const uint8_t* data, const int64_t* offse
 
 int bq_predict_uq_png(bq_model* m, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t T, uint64_t seed,
                       uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std, float* features) {
-  return predict_impl(m, data, false, m ? bq_png_state(m->png) : nullptr, offsets, 0, n, T, seed, tile_index_base,
+  return bq_predict_uq_png_ex(m, data, offsets, n, 0, T, seed, tile_index_base, masks, mean, std, features);
+}
+
+int bq_predict_uq_png_ex(bq_model* m, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t flags, int32_t T,
+                         uint64_t seed, uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std,
+                         float* features) {
+  return predict_impl(m, data, false, m ? bq_png_state(m->png) : nullptr, offsets, flags, n, T, seed, tile_index_base,
                       masks, mean, std, features);
 }
 

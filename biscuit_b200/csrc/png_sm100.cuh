@@ -1,11 +1,13 @@
-// PNG decode kernels (sm_100a) for 8-bit RGB non-interlaced tiles.  Included by png.cu only.  Three launches per group
-// of tiles:
+// PNG decode kernels (sm_100a).  Included by png.cu only.  Three launches per group of tiles:
 //   (a) png_dechunk_kernel   one CTA per tile: walks the run of IDAT chunks and copies their payloads into one
 //                            contiguous zlib stream;
 //   (b) png_inflate_kernel   one warp per tile: DEFLATE (RFC 1951) with zlib's validity rules.  Lane 0 decodes the
 //                            Huffman symbols and writes literals; the warp copies each match;
-//   (c) png_unfilter_kernel  one warp per tile: reverses the five PNG filters over a diagonal wavefront of 32 rows,
-//                            checks the Adler-32 of the decompressed stream, writes NHWC uint8.
+//   (c) png_unfilter_kernel  one warp per tile, 8-bit RGB non-interlaced tiles (the default decode): reverses the five
+//                            PNG filters over a diagonal wavefront of 32 rows, checks the Adler-32 of the decompressed
+//                            stream, writes NHWC uint8;
+//       png_unfilter_any_kernel  the same for every colour type, bit depth and interlace (BQ_PNG_CONVERT_RGB), pass by
+//                            pass, converting each unfiltered row group to RGB8 before it writes it.
 #pragma once
 
 #include <stdint.h>
@@ -18,6 +20,12 @@ struct Tile {
   int64_t off;     // tile bytes = [off, off + len) of the group's byte buffer; its zlib stream goes to the same offset
   int32_t len;
   int32_t idat;    // first IDAT chunk (its length field), relative to the tile start
+  int64_t foff;    // its decompressed (filtered) stream = [foff, foff + raw) of the group's filtered scratch
+  int32_t raw;     // size of that stream, as IHDR implies
+  uint8_t colour, depth, interlace;
+  uint8_t bpp;     // bytes per filter unit: max(1, channels x depth / 8)
+  int32_t npal;    // PLTE entries (palette images); pal holds them, zero-filled to 256
+  uint8_t pal[768];
 };
 
 __device__ __forceinline__ uint32_t be32(const uint8_t* p) {
@@ -200,11 +208,11 @@ struct Bits {
 enum { kCtlMatch = 1, kCtlEob = 2 };
 
 // Tile `tile` of the group: zlib stream zbuf[off, off + zlen) (the 2-byte header was checked on the host) ->
-// filt[tile * raw, +raw), its Adler-32 trailer -> adler[tile].
+// filt[foff, foff + raw), its Adler-32 trailer -> adler[tile].
 __global__ void __launch_bounds__(32 * kInflateWarps) png_inflate_kernel(const Tile* __restrict__ tiles,
                                                                           const uint8_t* __restrict__ zbuf,
                                                                           const int32_t* __restrict__ zlen, int n_tiles,
-                                                                          int32_t raw, uint8_t* __restrict__ filt,
+                                                                          uint8_t* __restrict__ filt,
                                                                           uint32_t* __restrict__ adler,
                                                                           int32_t* __restrict__ status) {
   __shared__ Tables tabs[kInflateWarps];
@@ -212,7 +220,8 @@ __global__ void __launch_bounds__(32 * kInflateWarps) png_inflate_kernel(const T
   const int tile = blockIdx.x * kInflateWarps + warp;
   if (tile >= n_tiles || status[tile] != 0) return;   // whole warps leave together
   Tables& T = tabs[warp];
-  uint8_t* out = filt + (size_t)tile * raw;
+  const int32_t raw = tiles[tile].raw;
+  uint8_t* out = filt + tiles[tile].foff;
   Bits br;
   br.p = zbuf + tiles[tile].off + 2;
   br.end = zlen[tile] - 2;
@@ -465,6 +474,150 @@ __global__ void __launch_bounds__(32) png_unfilter_kernel(const uint8_t* __restr
     }
     for (int i = lane; i < rowb; i += 32) prev[i] = rows[(size_t)(nr - 1) * rowb + i];
     __syncwarp();
+  }
+#pragma unroll
+  for (int d = 16; d; d >>= 1) {
+    sa += __shfl_xor_sync(0xFFFFFFFFu, sa, d);
+    sb += __shfl_xor_sync(0xFFFFFFFFu, sb, d);
+  }
+  bad = __any_sync(0xFFFFFFFFu, bad);
+  if (lane == 0) {
+    const uint32_t A = (uint32_t)((1 + sa) % 65521), B = (uint32_t)(((uint64_t)raw + sb) % 65521);
+    if ((B << 16 | A) != adler[tile]) status[tile] = BQ_PNG_ADLER;
+    else if (bad) status[tile] = BQ_PNG_BAD_FILTER;
+  }
+}
+
+// ------------------------------------------------------------------------------------------------------------------
+// (c') unfilter + convert, any colour type / bit depth / interlace.  One warp per tile walks the Adam7 passes (one pass
+// when not interlaced) in stream order.  Within a pass it runs the wavefront of (c) over groups of 32 rows, on filter
+// units of bpp bytes (1 to 8, held in a uint64), with the pass's row length 1 + ceil(w x channels x depth / 8).  Once a
+// group is unfiltered in shared memory the warp converts each of its pixels to RGB8 -- sub-byte samples unpacked and
+// scaled (gray) or looked up (palette), 16-bit samples reduced to the high byte, gray replicated, alpha dropped -- and
+// writes it to (y0 + r dy, x0 + c dx).  The Adler-32 runs over the whole stream in stream order, across passes.
+// ------------------------------------------------------------------------------------------------------------------
+constexpr int kPalBytes = 768;
+
+// Adam7 passes 1-7 (indices 0-6): first column / row and their steps; index 7 is the whole non-interlaced image
+__constant__ uint8_t kAdam7[8][4] = {{0, 0, 8, 8}, {4, 0, 8, 8}, {0, 4, 4, 8}, {2, 0, 4, 4},
+                                     {0, 2, 2, 4}, {1, 0, 2, 2}, {0, 1, 1, 2}, {0, 0, 1, 1}};
+
+__host__ __device__ constexpr int png_channels(int colour) {
+  return colour == 2 ? 3 : colour == 4 ? 2 : colour == 6 ? 4 : 1;
+}
+
+// filtered row bytes of a pass `w` pixels wide
+__host__ __device__ constexpr int64_t row_bytes(int64_t w, int colour, int depth) {
+  return 1 + (w * png_channels(colour) * depth + 7) / 8;
+}
+
+// shared memory of png_unfilter_any_kernel for rows of at most `row` bytes
+__host__ __device__ constexpr size_t unfilter_any_smem(int64_t row) { return kPalBytes + (size_t)(kRows + 1) * row; }
+
+__device__ __forceinline__ uint64_t unfilter_unit(int ft, int bpp, uint64_t f, uint64_t a, uint64_t b, uint64_t c) {
+  uint64_t v = 0;
+  for (int k = 0; k < bpp; ++k) {
+    const int fa = (int)(a >> (8 * k)) & 255, fb = (int)(b >> (8 * k)) & 255, fc = (int)(c >> (8 * k)) & 255;
+    int pred = 0;
+    if (ft == 1) pred = fa;
+    else if (ft == 2) pred = fb;
+    else if (ft == 3) pred = (fa + fb) >> 1;
+    else if (ft == 4) {
+      const int pa = abs(fb - fc), pb = abs(fa - fc), pc = abs(fa + fb - 2 * fc);
+      pred = (pa <= pb && pa <= pc) ? fa : (pb <= pc ? fb : fc);
+    }
+    v |= (uint64_t)((((int)(f >> (8 * k)) & 255) + pred) & 255) << (8 * k);
+  }
+  return v;
+}
+
+__device__ __forceinline__ uint64_t load_unit(const uint8_t* p, int bpp) {
+  uint64_t v = 0;
+  for (int k = 0; k < bpp; ++k) v |= (uint64_t)p[k] << (8 * k);
+  return v;
+}
+
+__global__ void __launch_bounds__(32) png_unfilter_any_kernel(const Tile* __restrict__ tiles,
+                                                              const uint8_t* __restrict__ filt, int px,
+                                                              const uint32_t* __restrict__ adler,
+                                                              int32_t* __restrict__ status, uint8_t* __restrict__ out) {
+  extern __shared__ uint8_t sm[];
+  const int tile = blockIdx.x, lane = threadIdx.x;
+  if (status[tile] != 0) return;
+  const Tile& t = tiles[tile];
+  const int colour = t.colour, depth = t.depth, bpp = t.bpp, ch = png_channels(colour);
+  const int64_t raw = t.raw;
+  const uint8_t* f = filt + t.foff;
+  uint8_t* o = out + (size_t)tile * px * px * 3;
+  uint8_t* pal = sm;                                   // [256][3], zero past the PLTE entries
+  uint8_t* rows = sm + kPalBytes;
+  for (int i = lane; i < kPalBytes; i += 32) pal[i] = t.pal[i];
+  const int gray_scale = depth == 1 ? 255 : depth == 2 ? 85 : depth == 4 ? 17 : 1;
+  uint64_t sa = 0, sb = 0;
+  int64_t pos = 0;                                     // stream offset of the pass
+  int bad = 0;
+  for (int p = t.interlace ? 0 : 7; p < (t.interlace ? 7 : 8); ++p) {
+    const int x0 = kAdam7[p][0], y0 = kAdam7[p][1], dx = kAdam7[p][2], dy = kAdam7[p][3];
+    const int pw = px > x0 ? (px - x0 + dx - 1) / dx : 0, ph = px > y0 ? (px - y0 + dy - 1) / dy : 0;
+    if (pw == 0 || ph == 0) continue;                  // an empty pass has no bytes, not even filter bytes
+    const int rowb = (int)row_bytes(pw, colour, depth);
+    const int units = (rowb - 1) / bpp;                // sub-byte rows: one unit per byte
+    uint8_t* prev = rows + (size_t)kRows * rowb;       // the row above the group (zeros above the pass's row 0)
+    __syncwarp();
+    for (int i = lane; i < rowb; i += 32) prev[i] = 0;
+    for (int r0 = 0; r0 < ph; r0 += kRows) {
+      const int nr = min(kRows, ph - r0);
+      const int64_t base = pos + (int64_t)r0 * rowb;
+      const int n = nr * rowb;
+      for (int i = lane; i < n; i += 32) {
+        const uint32_t b = f[base + i];
+        rows[i] = (uint8_t)b;
+        sa += b;
+        sb += (uint64_t)(raw - base - i) * b;
+      }
+      __syncwarp();
+      uint8_t* my = rows + (size_t)lane * rowb;
+      int ft = lane < nr ? my[0] : 0;
+      if (ft > 4) { bad = 1; ft = 0; }
+      uint64_t cur = 0, upl = 0;                       // own previous unit; the up value of the previous step
+      for (int s = 0; s < units + nr - 1; ++s) {
+        const int x = s - lane;
+        uint64_t up = __shfl_up_sync(0xFFFFFFFFu, cur, 1);
+        if (lane == 0 && x >= 0 && x < units) up = load_unit(prev + 1 + bpp * x, bpp);
+        if (x >= 0 && x < units && lane < nr) {
+          uint8_t* q = my + 1 + bpp * x;
+          const uint64_t a = x ? cur : 0, c = x ? upl : 0;
+          cur = unfilter_unit(ft, bpp, load_unit(q, bpp), a, up, c);
+          for (int k = 0; k < bpp; ++k) q[k] = (uint8_t)(cur >> (8 * k));
+        }
+        upl = up;
+      }
+      __syncwarp();
+      for (int i = lane; i < nr * pw; i += 32) {
+        const int r = i / pw, c = i - r * pw;
+        const uint8_t* q = rows + (size_t)r * rowb + 1;
+        uint32_t R, G, B;
+        if (depth < 8) {
+          const int bit = c * depth;
+          const uint32_t v = (q[bit >> 3] >> (8 - depth - (bit & 7))) & ((1u << depth) - 1u);
+          if (colour == 3) { R = pal[3 * v]; G = pal[3 * v + 1]; B = pal[3 * v + 2]; }
+          else R = G = B = v * gray_scale;
+        } else {
+          const int sh = depth >> 4;                   // 16-bit samples: the high (first) byte
+          const uint8_t* e = q + ((size_t)c * ch << sh);
+          if (colour == 3) { R = pal[3 * e[0]]; G = pal[3 * e[0] + 1]; B = pal[3 * e[0] + 2]; }
+          else if (colour == 0 || colour == 4) R = G = B = e[0];
+          else { R = e[0]; G = e[1 << sh]; B = e[2 << sh]; }
+        }
+        uint8_t* d = o + ((size_t)(y0 + (r0 + r) * dy) * px + x0 + (size_t)c * dx) * 3;
+        d[0] = (uint8_t)R;
+        d[1] = (uint8_t)G;
+        d[2] = (uint8_t)B;
+      }
+      for (int i = lane; i < rowb; i += 32) prev[i] = rows[(size_t)(nr - 1) * rowb + i];
+      __syncwarp();
+    }
+    pos += (int64_t)ph * rowb;
   }
 #pragma unroll
   for (int d = 16; d; d >>= 1) {

@@ -17,6 +17,8 @@ class EncodedBatch:
     FORMAT: str          # "jpeg" / "png": the `bq_{FORMAT}_*` entry points that decode it
     # decode options as the `flags` of the `bq_{FORMAT}_*_ex` entry points; None: the format has none
     flags: int | None = None
+    # whether the header parse depends on those options, so that inspect takes them too (`bq_{FORMAT}_inspect_ex`)
+    PARSE_OPTIONS = False
 
     def __init__(self, data, offsets):
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
@@ -76,11 +78,12 @@ def status_message(fmt: str, code: int) -> str:
 def inspect(fmt: str, batch: EncodedBatch, px: int) -> np.ndarray:
     if batch.on_device:
         raise ValueError("inspect reads host bytes; the batch is in device memory")
-    entry = getattr(_ffi.load_library(), f"bq_{fmt}_inspect")
+    name, flags = entry_point(f"bq_{fmt}_inspect", batch) if batch.PARSE_OPTIONS else (f"bq_{fmt}_inspect", ())
     st = np.zeros(len(batch), np.int32)
-    rc = entry(_ffi.ptr(batch.data), _ffi.ptr(batch.offsets), len(batch), int(px), _ffi.ptr(st))
+    rc = getattr(_ffi.load_library(), name)(_ffi.ptr(batch.data), _ffi.ptr(batch.offsets), len(batch), int(px), *flags,
+                                             _ffi.ptr(st))
     if rc != 0:
-        raise ValueError(f"bq_{fmt}_inspect: bad argument")
+        raise ValueError(f"{name}: bad argument")
     return st
 
 

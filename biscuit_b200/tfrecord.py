@@ -45,7 +45,7 @@ def scan(buf, image_key="image_raw", slide_key="slide", x_key="loc_x", y_key="lo
 
 
 def read(paths, image_key="image_raw", slide_key="slide", x_key="loc_x", y_key="loc_y",
-         dct_method="INTEGER_ACCURATE", fancy_upscaling=True):
+         dct_method="INTEGER_ACCURATE", fancy_upscaling=True, png_convert_rgb=False):
     """(batch, slides, loc_x, loc_y) over the records of `paths` (one path or a list), in file order.
     batch: a PngBatch when every image starts with the PNG signature, else a JpegBatch (whatever is not JPEG then fails
     in the JPEG decoder, naming the tile).  A set that mixes PNG with other images raises ValueError naming the first
@@ -53,7 +53,9 @@ def read(paths, image_key="image_raw", slide_key="slide", x_key="loc_x", y_key="
     int64 arrays.
     dct_method / fancy_upscaling: the JpegBatch's decode options, as in `tf.image.decode_jpeg`
     (`dct_method="INTEGER_FAST"` decodes as TensorFlow does by default).  A PngBatch ignores them: PNG is lossless and
-    `decode_png` has no such options."""
+    `decode_png` has no such options.
+    png_convert_rgb: the PngBatch's `convert_rgb` (every colour type, bit depth and interlace, converted to RGB8 as
+    `decode_png(channels=3)` does); a JpegBatch ignores it."""
     check_dct_method(dct_method)
     if isinstance(paths, (str, os.PathLike)):
         paths = [paths]
@@ -79,7 +81,7 @@ def read(paths, image_key="image_raw", slide_key="slide", x_key="loc_x", y_key="
     offsets[1:] = np.cumsum(sizes)
     data = np.concatenate(parts) if parts else np.zeros(0, np.uint8)
     loc = np.concatenate(locs) if locs else np.zeros((0, 2), np.int64)
-    batch = PngBatch(data, offsets) if first_png else JpegBatch(data, offsets, dct_method, fancy_upscaling)
+    batch = PngBatch(data, offsets, png_convert_rgb) if first_png else JpegBatch(data, offsets, dct_method, fancy_upscaling)
     return batch, slides, loc[:, 0].copy(), loc[:, 1].copy()
 
 

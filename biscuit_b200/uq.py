@@ -129,7 +129,7 @@ class UncertaintyInterface:
         convolution), or float32 ALREADY passed through `tf.image.per_image_standardization` as the reference's call site
         does (results.py:255-257); numpy, or a CUDA torch tensor used in place.  Or a `jpeg.JpegBatch` / `png.PngBatch`
         of JPEG / PNG tiles, decoded on the GPU in front of the backbone (a JpegBatch with its `dct_method` /
-        `fancy_upscaling`): the results equal `predict` on the decoded uint8 tiles bit for bit.
+        `fancy_upscaling`, a PngBatch with its `convert_rgb`): the results equal `predict` on the decoded uint8 tiles bit for bit.
         Returns (mean [n, C], std [n, C]) float32 -- population std over T dropout samples."""
         T = int(T or self.num_uq)
         encoded = tiles.FORMAT if isinstance(tiles, EncodedBatch) else None
@@ -265,7 +265,9 @@ def predict_tfrecords(interface: UncertaintyInterface, paths, y_true=None, outco
     tiles.  y_true: per-tile labels, or a dict slide -> label.  Adds the `loc_x` / `loc_y` columns of each tile.
     `keys` goes to `tfrecord.read`: the feature names (`image_key`, `slide_key`, `x_key`, `y_key`) and the JPEG decode
     options `dct_method` / `fancy_upscaling` (as in `tf.image.decode_jpeg`; `dct_method="INTEGER_FAST"` selects the
-    IDCT `decode_jpeg` uses by default, on whose output Slideflow TensorFlow models were trained; ignored for PNG)."""
+    IDCT `decode_jpeg` uses by default, on whose output Slideflow TensorFlow models were trained; ignored for PNG), and
+    the PNG decode option `png_convert_rgb` (grayscale, palette, alpha, 16-bit and interlaced PNG tiles converted to
+    RGB8 as `decode_png(channels=3)` does; ignored for JPEG)."""
     from . import tfrecord
     batch, slides, loc_x, loc_y = tfrecord.read(paths, **keys)
     if isinstance(y_true, dict):

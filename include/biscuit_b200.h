@@ -332,7 +332,18 @@ int bq_predict_uq_jpeg_ex(bq_model* m, const uint8_t* data, const int64_t* offse
  * TensorFlow's decode_png).  Same layout as the JPEG entry points: tile i = data[offsets[i], offsets[i + 1]), offsets
  * in host memory.  Accepted: 8-bit RGB (colour type 2), non-interlaced, px x px, any zlib level / strategy / window,
  * IDAT split into chunks of any size, ancillary chunks and PLTE (skipped).  Every chunk before the first IDAT must pass
- * its CRC; IDAT CRCs are not checked (the zlib Adler-32 is). */
+ * its CRC; IDAT CRCs are not checked (the zlib Adler-32 is).
+ *   The flags of the _ex entry points select a decode option per call:
+ *     BQ_PNG_CONVERT_RGB  accept every colour type / bit depth pair of the PNG specification (gray 1/2/4/8/16, RGB
+ *                         8/16, palette 1/2/4/8, gray + alpha 8/16, RGBA 8/16), interlaced (Adam7) or not, and convert
+ *                         to RGB8 as TensorFlow's decode_png(channels=3) and Pillow's convert("RGB") do: gray copied to
+ *                         R, G and B (1/2/4-bit scaled by 255/85/17), alpha dropped (not composited), tRNS ignored,
+ *                         16-bit samples reduced to their high byte (Pillow instead clips 16-bit gray to 255), palette
+ *                         entries from PLTE (an index past the last entry gives black).  A palette image needs a PLTE
+ *                         before its first IDAT (BQ_PNG_NO_PLTE) of 1 to 256 entries (BQ_PNG_BAD_PLTE); an illegal
+ *                         colour type / depth pair is BQ_PNG_BAD_IHDR.  8-bit RGB tiles decode to the same bytes as
+ *                         without the option.
+ *   Any other flag bit fails the call with BQ_ERR_ARG before anything is launched. */
 enum {
   BQ_PNG_OK = 0,
   BQ_PNG_NOT_PNG = 1,              /* no PNG signature                                                */
@@ -347,12 +358,14 @@ enum {
   BQ_PNG_NO_IDAT = 10,             /* IEND before any IDAT                                             */
   BQ_PNG_BAD_ZLIB = 11,            /* zlib header: CM != 8, CINFO > 7 or bad FCHECK                    */
   BQ_PNG_PRESET_DICT = 12,         /* zlib FDICT set                                                   */
+  BQ_PNG_NO_PLTE = 13,             /* BQ_PNG_CONVERT_RGB: palette image without PLTE before its IDAT    */
+  BQ_PNG_BAD_PLTE = 14,            /* BQ_PNG_CONVERT_RGB: PLTE length 0, not a multiple of 3, > 256 x 3 */
   /* found on the device */
   BQ_PNG_TRUNCATED_DATA = 20,      /* the IDAT run or the DEFLATE stream ends early, or no Adler-32    */
   BQ_PNG_BAD_BLOCK = 21,           /* BTYPE 3, or a stored block with LEN != ~NLEN                     */
   BQ_PNG_BAD_HUFFMAN = 22,         /* over-subscribed / incomplete code, bad repeat, invalid symbol    */
   BQ_PNG_BAD_DISTANCE = 23,        /* a match reaching before the start of the stream                  */
-  BQ_PNG_WRONG_SIZE = 24,          /* decompressed size != px * (1 + 3 px)                             */
+  BQ_PNG_WRONG_SIZE = 24,          /* decompressed size != the size IHDR implies (px * (1 + 3 px) RGB8) */
   BQ_PNG_ADLER = 25,               /* Adler-32 mismatch                                                */
   BQ_PNG_BAD_FILTER = 26           /* a row filter type > 4                                            */
 };
@@ -361,6 +374,10 @@ const char* bq_png_status_string(int32_t status);
 /* Host only, no device needed: the chunk parse bq_png_decode runs first.  status[i] = BQ_PNG_* of tile i.  data must
  * be host memory.  Returns BQ_OK also when some tiles are rejected. */
 int bq_png_inspect(const uint8_t* data, const int64_t* offsets, int64_t n, int32_t px, int32_t* status);
+/* bq_png_inspect with the decode options of bq_png_decode_ex (0 is bq_png_inspect): the header parse depends on them.
+ * Unknown flag bits return BQ_ERR_ARG. */
+int bq_png_inspect_ex(const uint8_t* data, const int64_t* offsets, int64_t n, int32_t px, int32_t flags,
+                      int32_t* status);
 /* Decode n tiles into out_u8 = uint8 NHWC [n, px, px, 3] (host or device); data host or device (device bytes are read
  * in place).  status[i] (host, nullable) = BQ_PNG_* of tile i.  A rejected header fails the call with BQ_ERR_DATA
  * before anything is launched; a tile rejected on the device fails it with BQ_ERR_DATA after the batch (the other
@@ -368,9 +385,21 @@ int bq_png_inspect(const uint8_t* data, const int64_t* offsets, int64_t n, int32
  * more bytes than the image are rejected. */
 int bq_png_decode(bq_ctx* ctx, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t px, uint8_t* out_u8,
                   int32_t* status);
+/* decode options of bq_png_inspect_ex / bq_png_decode_ex / bq_predict_uq_png_ex (see above) */
+enum {
+  BQ_PNG_CONVERT_RGB = 1
+};
+/* bq_png_decode with decode options: flags = BQ_PNG_CONVERT_RGB or 0 (0 is bq_png_decode).  The options apply to this
+ * call only. */
+int bq_png_decode_ex(bq_ctx* ctx, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t px, int32_t flags,
+                     uint8_t* out_u8, int32_t* status);
 /* bq_predict_uq on PNG tiles: same outputs, seeds and tile indices as bq_predict_uq on the decoded uint8 tiles. */
 int bq_predict_uq_png(bq_model* m, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t T, uint64_t seed,
                       uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std, float* features);
+/* bq_predict_uq_png with the decode options of bq_png_decode_ex (0 is bq_predict_uq_png), for this call only. */
+int bq_predict_uq_png_ex(bq_model* m, const uint8_t* data, const int64_t* offsets, int64_t n, int32_t flags, int32_t T,
+                         uint64_t seed, uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std,
+                         float* features);
 
 /* TFRecord file (uncompressed) in a host buffer: record framing {u64 length, masked CRC32C of the length, payload,
  * masked CRC32C of the payload}, both CRCs verified (SSE4.2 crc32 when the CPU has it), payload parsed as a

@@ -2,11 +2,17 @@
 `predict(PngBatch)` against `predict(uint8)`, plus the host's own Pillow decode rate over all its cores.
 
     python profiles/png_bench.py [--tiles 10000] [--big-tiles 100000] [--T 30] [--reps 3] [--out results.json]
+    python profiles/png_bench.py --convert-only [--out results.json]
 
 Two encodings: Pillow `compress_level` 1 and 6 (Pillow's default).  The inputs cycle 503 distinct `synth.tiles_u8`
 tiles (about 200 KB of PNG each), so the 10 k-tile pass already reads about 2 GB, far more than the 126 MB L2.  The
 uint8 and PNG inputs alternate within one run, pinned and pageable, and their outputs must be equal.  One extra run at
 --big-tiles tiles reads both inputs from device memory, to show the rate holds over a long stream.
+
+Then the decode option `convert_rgb`: kernel times per 503-tile micro-batch for RGBA8, gray8 and palette8 (Pillow's
+encodings of the same tiles), RGB16 and interlaced RGB8 (tests/png_any_ref.py's writer, a random filter per row, zlib
+level 6), and Pillow's RGB8 at level 6 through the option's kernel.  Each decode is checked against Pillow's (RGB16:
+the tile's high bytes).  `--convert-only` runs this part alone.
 """
 from __future__ import annotations
 
@@ -56,7 +62,8 @@ def kernel_split(batch, ctx, reps=5):
     with profile(activities=[ProfilerActivity.CUDA]) as prof:
         for _ in range(reps):
             png.decode(batch, ctx=ctx, out=out)
-    names = {"dechunk": "png_dechunk_kernel", "inflate": "png_inflate_kernel", "unfilter": "png_unfilter_kernel"}
+    names = {"dechunk": "png_dechunk_kernel", "inflate": "png_inflate_kernel", "unfilter": "png_unfilter_kernel",
+             "unfilter_any": "png_unfilter_any_kernel"}
     ms = {k: 0.0 for k in names}
     for ev in prof.key_averages():
         for k, n in names.items():
@@ -73,6 +80,48 @@ def kernel_split(batch, ctx, reps=5):
     return ms
 
 
+def convert_rgb_split(base, ctx):
+    """decode ms per micro-batch of `base` tiles, per format, with the convert_rgb option (device bytes and output)"""
+    import io
+
+    import torch
+    from PIL import Image
+
+    from biscuit_b200 import png
+    from biscuit_b200.png import PngBatch
+    from oracle import png_synth
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import png_any_ref as R
+
+    def pil(t, mode):
+        bio = io.BytesIO()
+        img = Image.fromarray(t)
+        img = (img.convert("P", palette=Image.Palette.ADAPTIVE) if mode == "P" else
+               Image.fromarray(np.dstack([t, t[..., 1]]), "RGBA") if mode == "RGBA" else img.convert(mode))
+        img.save(bio, "PNG", compress_level=6)
+        return bio.getvalue()
+
+    formats = {
+        "rgb8_level6": [png_synth.pil_encode(t, 6) for t in base],
+        "rgba8": [pil(t, "RGBA") for t in base],
+        "gray8": [pil(t, "L") for t in base],
+        "palette8": [pil(t, "P") for t in base],
+        "rgb16": [R.encode(t.astype(np.uint16) << 8 | (t & 7), 2, 16, 0, "random", seed=i) for i, t in enumerate(base)],
+        "rgb8_adam7": [R.encode(t.astype(np.uint16), 2, 8, 1, "random", seed=i) for i, t in enumerate(base)],
+    }
+    out = {}
+    for k, files in formats.items():
+        mb = PngBatch.from_bytes(files, convert_rgb=True)
+        got = png.decode(mb, ctx=ctx)
+        want = base if k in ("rgb16", "rgb8_adam7") else np.stack([png_synth.pil_decode(b) for b in files])
+        assert np.array_equal(got, want), k
+        split = kernel_split(mb.cuda(), ctx)
+        out[k] = dict(bytes_per_tile=mb.nbytes / len(mb), decode_ms_per_503=split,
+                      decode_tiles_per_s=len(mb) / (split["call"] / 1e3))
+    torch.cuda.synchronize()
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--tiles", type=int, default=10000)
@@ -81,6 +130,7 @@ def main():
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--pil-tiles", type=int, default=4000)
     ap.add_argument("--out", default=None, help="also write the result JSON to this file")
+    ap.add_argument("--convert-only", action="store_true", help="only the convert_rgb decode times")
     a = ap.parse_args()
 
     import torch
@@ -99,7 +149,7 @@ def main():
     ctx = _ffi.default_context(0)
     base = synth.tiles_u8(uq.BENCH_MICRO_BATCH, seed=7, n_slides=8)
     iface = uq.UncertaintyInterface(random_init(seed=1), max_batch=uq.BENCH_MICRO_BATCH, ctx=ctx)
-    for level in LEVELS:
+    for level in () if a.convert_only else LEVELS:
         name = f"pil_level{level}"
         files = [png_synth.pil_encode(t, level) for t in base]
         mb = PngBatch.from_bytes(files)
@@ -163,6 +213,8 @@ def main():
         r["decode_over_host_pil"] = r["decode_tiles_per_s"] / r["host_pil_tiles_per_s"]
         res["configs"][name] = r
         print(name, json.dumps(r, indent=1), flush=True)
+    res["convert_rgb"] = convert_rgb_split(base, ctx)
+    print("convert_rgb", json.dumps(res["convert_rgb"], indent=1), flush=True)
     if a.out:
         with open(a.out, "w") as f:
             json.dump(res, f, indent=1)
