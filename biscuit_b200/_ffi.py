@@ -83,6 +83,8 @@ SIGNATURES = {
                                              C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "bq_model_debug_stage": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_char_p, C.c_void_p,
                                        C.c_int64, C.POINTER(C.c_int64)]),
+    "bq_model_debug_stage_standardized": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_char_p, C.c_void_p,
+                                                    C.c_int64, C.POINTER(C.c_int64)]),
     "bq_model_debug_h1": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p]),
     "bq_model_debug_tags": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int64]),
     "bq_stain_normalize": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p,

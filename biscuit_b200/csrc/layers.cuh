@@ -126,11 +126,15 @@ constexpr int kC1Tile = 16;
 constexpr int kC1In = 2 * kC1Tile + 1;
 // TIn = uint8_t: raw RGB, standardised here with the tile's (mean, 1/std).  TIn = float: the caller already applied
 // tf.image.per_image_standardization (the reference's literal call, results.py:255-257) -- values are used as they are.
+// A float tile holding a NaN or +-Inf would reach the output as an ordinary-looking number (fmaxf(NaN, 0) = 0), so the
+// float instantiation records the smallest call-global index i0 + img of such a tile in *nonfinite (atomicMin; the
+// caller resets the word to ~0 and reports it after the call).
 template <typename TIn>
 __global__ void __launch_bounds__(256)
 conv1_kernel(const TIn* __restrict__ tiles, const float* __restrict__ mean, const float* __restrict__ inv_std,
              const float* __restrict__ w /*[27][32]*/, const float* __restrict__ scale, const float* __restrict__ shift,
-             bf16* __restrict__ out, int in_px, int out_px) {
+             bf16* __restrict__ out, int in_px, int out_px, unsigned long long* __restrict__ nonfinite = nullptr,
+             int64_t i0 = 0) {
   __shared__ float patch[kC1In * kC1In * 3];
   __shared__ __align__(16) float ws[27 * 32];
   __shared__ float sc[32], sh[32];
@@ -142,15 +146,21 @@ conv1_kernel(const TIn* __restrict__ tiles, const float* __restrict__ mean, cons
   for (int i = threadIdx.x; i < 27 * 32; i += blockDim.x) ws[i] = w[i];
   if (threadIdx.x < 32) { sc[threadIdx.x] = scale[threadIdx.x]; sh[threadIdx.x] = shift[threadIdx.x]; }
   const int iy0 = oy0 * 2, ix0 = ox0 * 2;
+  bool finite = true;
   for (int i = threadIdx.x; i < kC1In * kC1In * 3; i += blockDim.x) {
     const int r = i / (kC1In * 3), rem = i - r * (kC1In * 3);
     const int y = iy0 + r, xc = ix0 * 3 + rem;
     float v = 0.f;
     if (y < in_px && xc < in_px * 3) {
       const float raw = (float)src[(int64_t)y * in_px * 3 + xc];
+      if constexpr (!kRaw) finite &= isfinite(raw);
       v = kRaw ? __fmul_rn(__fadd_rn(raw, -mu), is) : raw;
     }
     patch[i] = v;
+  }
+  // the patches of a tile's blocks cover every one of its values (the last block's reaches row / column 320 > 298)
+  if constexpr (!kRaw) {
+    if (!finite) atomicMin(nonfinite, (unsigned long long)(i0 + img));
   }
   __syncthreads();
   const int ty = threadIdx.x / kC1Tile, tx = threadIdx.x % kC1Tile;

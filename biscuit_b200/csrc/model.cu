@@ -257,6 +257,8 @@ struct bq_model {
   DevBuf tiles_dev2;
   DevBuf tiles_f32[2];                         // float32 staging for already-standardised host tiles (allocated on first use)
   bool input_f32 = false;                      // the current call feeds standardised float tiles: no statistics, no normaliser
+  DevBuf nonfinite;                            // uint64: smallest index in the call of a float tile holding NaN / Inf (~0: none)
+  int64_t call_i0 = 0;                         // index in the call of the micro-batch's first tile
   int norm_kind = 0;                           // BQ_NORM_*: stain normalisation in front of the tile statistics
   float norm_means[3] = {0, 0, 0}, norm_stds[3] = {1, 1, 1};
   DevBuf tiles_norm, norm_lut, norm_stats;     // normalised micro-batch, gamma table, per-tile LAB statistics
@@ -642,7 +644,8 @@ int run_op(bq_model* m, Op& op, int nb, int64_t out_off = 0) {
         bq::conv1_kernel<float><<<grid, 256, 0, ctx->stream>>>((const float*)m->tiles_src, (const float*)m->mean.p,
                                                               (const float*)m->inv_std.p, (const float*)m->conv1_w.p,
                                                               (const float*)m->conv1_scale.p, (const float*)m->conv1_shift.p,
-                                                              op.out, px, op.Ho);
+                                                              op.out, px, op.Ho, (unsigned long long*)m->nonfinite.p,
+                                                              m->call_i0);
       else
         bq::conv1_kernel<uint8_t><<<grid, 256, 0, ctx->stream>>>(m->tiles_src, (const float*)m->mean.p,
                                                                 (const float*)m->inv_std.p, (const float*)m->conv1_w.p,
@@ -1168,6 +1171,11 @@ static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, bq_en
     const int64_t cap = n < B ? n : B;                      // the interface is usually called tile by tile (results.py:249-257)
     for (auto& b : m->tiles_f32) { int rcf = bq_alloc(ctx, b, (size_t)cap * tile_bytes + 64); if (rcf) return rcf; }
   }
+  if (f32_input) {
+    const int rcn = bq_alloc(ctx, m->nonfinite, sizeof(uint64_t));
+    if (rcn) return rcn;
+    BQ_CUDA(ctx, cudaMemsetAsync(m->nonfinite.p, 0xFF, sizeof(uint64_t), ctx->stream));
+  }
   uint8_t* stage[2] = {(uint8_t*)(f32_input ? m->tiles_f32[0].p : m->tiles_dev.p), (uint8_t*)(f32_input ? m->tiles_f32[1].p : m->tiles_dev2.p)};
   auto issue_copy = [&](int64_t i0c, int slot) -> int {
     const int nbc = (int)((n - i0c < B) ? (n - i0c) : B);
@@ -1218,6 +1226,7 @@ static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, bq_en
         return rc;
       m->tiles_src = (const uint8_t*)m->tiles_norm.p;
     }
+    m->call_i0 = i0;
     if ((rc = run_backbone_graphed(m, nb))) return rc;
     if (!tiles_on_dev) {
       if (!compressed) BQ_CUDA(ctx, cudaEventRecord(m->consumed[slot], ctx->stream));
@@ -1257,21 +1266,38 @@ static int predict_impl(bq_model* m, const uint8_t* tiles, bool f32_input, bq_en
       }
     }
   }
+  uint64_t nonfinite = ~0ull;
+  if (f32_input) BQ_CUDA(ctx, cudaMemcpyAsync(&nonfinite, m->nonfinite.p, sizeof(nonfinite), cudaMemcpyDeviceToHost, ctx->stream));
   BQ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   if (compressed) return enc->finish(ctx, nullptr);
+  // every tile's outputs are written; a tile with a NaN / Inf then fails the call, as a corrupt JPEG / PNG tile does
+  if (nonfinite != ~0ull)
+    return bq_fail(ctx, BQ_ERR_DATA, "bq_predict_uq_standardized tile %lld: non-finite value", (long long)nonfinite);
   return BQ_OK;
 }
 
-int bq_model_debug_stage(bq_model* m, const uint8_t* tiles, int64_t n, const char* stage, float* out,
-                         int64_t out_capacity, int64_t out_shape[4]) {
-  if (!m) return BQ_ERR_ARG;
+// bq_model_debug_stage (uint8 tiles) and bq_model_debug_stage_standardized (m->input_f32: float tiles, staged in
+// tiles_f32[0]; the non-finite check runs but is not reported)
+static int debug_stage_impl(bq_model* m, const uint8_t* tiles, int64_t n, const char* stage, float* out,
+                            int64_t out_capacity, int64_t out_shape[4]) {
   bq_ctx* ctx = m->ctx;
   if (!m->weights_loaded) return bq_fail(ctx, BQ_ERR_STATE, "weights not loaded");
   if (!tiles || !stage || !out || !out_shape || n < 1 || n > m->max_batch)
     return bq_fail(ctx, BQ_ERR_ARG, "bq_model_debug_stage: bad argument (n must be <= max_batch)");
   BQ_CUDA(ctx, cudaSetDevice(ctx->device));
   int rc;
-  if ((rc = stage_tiles(m, tiles, (int)n))) return rc;
+  if (m->input_f32) {
+    const size_t tile_bytes = (size_t)m->px * m->px * 3 * sizeof(float);
+    if ((rc = bq_alloc(ctx, m->tiles_f32[0], (size_t)m->max_batch * tile_bytes + 64)) ||
+        (rc = bq_alloc(ctx, m->nonfinite, sizeof(uint64_t))))
+      return rc;
+    BQ_CUDA(ctx, cudaMemsetAsync(m->nonfinite.p, 0xFF, sizeof(uint64_t), ctx->stream));
+    BQ_CUDA(ctx, cudaMemcpyAsync(m->tiles_f32[0].p, tiles, (size_t)n * tile_bytes, cudaMemcpyDefault, ctx->stream));
+    m->tiles_src = (const uint8_t*)m->tiles_f32[0].p;
+    m->call_i0 = 0;
+  } else if ((rc = stage_tiles(m, tiles, (int)n))) {
+    return rc;
+  }
   const std::string tag(stage);
   const Op* op = nullptr;
   const int prof = m->profiling;
@@ -1300,6 +1326,21 @@ int bq_model_debug_stage(bq_model* m, const uint8_t* tiles, int64_t n, const cha
   if ((rc = bq_from_device(ctx, out, scr, total * 4))) return rc;
   BQ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return BQ_OK;
+}
+
+int bq_model_debug_stage(bq_model* m, const uint8_t* tiles, int64_t n, const char* stage, float* out,
+                         int64_t out_capacity, int64_t out_shape[4]) {
+  if (!m) return BQ_ERR_ARG;
+  return debug_stage_impl(m, tiles, n, stage, out, out_capacity, out_shape);
+}
+
+int bq_model_debug_stage_standardized(bq_model* m, const float* tiles, int64_t n, const char* stage, float* out,
+                                      int64_t out_capacity, int64_t out_shape[4]) {
+  if (!m) return BQ_ERR_ARG;
+  m->input_f32 = true;
+  const int rc = debug_stage_impl(m, (const uint8_t*)tiles, n, stage, out, out_capacity, out_shape);
+  m->input_f32 = false;
+  return rc;
 }
 
 int bq_model_debug_tags(bq_model* m, char* out, int64_t capacity) {

@@ -130,6 +130,8 @@ class UncertaintyInterface:
         does (results.py:255-257); numpy, or a CUDA torch tensor used in place.  Or a `jpeg.JpegBatch` / `png.PngBatch`
         of JPEG / PNG tiles, decoded on the GPU in front of the backbone (a JpegBatch with its `dct_method` /
         `fancy_upscaling`, a PngBatch with its `convert_rgb`): the results equal `predict` on the decoded uint8 tiles bit for bit.
+        Float32 tiles must be finite: a tile holding a NaN or +-Inf raises ValueError naming the smallest such tile index
+        in the call, after the batch has run (the other tiles' results are written into `out_mean` / `out_std` when given).
         Returns (mean [n, C], std [n, C]) float32 -- population std over T dropout samples."""
         T = int(T or self.num_uq)
         encoded = tiles.FORMAT if isinstance(tiles, EncodedBatch) else None
@@ -183,20 +185,31 @@ class UncertaintyInterface:
         return self.predict(tiles, **kw)
 
     # ------------------------------------------------------------------------------------
-    def debug_stage(self, tiles: np.ndarray, stage: str) -> np.ndarray:
+    def debug_stage(self, tiles, stage: str) -> np.ndarray:
         """Parity hook: NHWC float32 copy of the output of one op of the backbone plan, run up to that op.
+        tiles: [n <= max_batch, px, px, 3], numpy or torch (CPU or CUDA): uint8 takes the route of raw tiles, float32 the
+        route of standardised tiles (`predict` on float32), as `predict` dispatches them.
         Tags: 'block1_conv1', 'block1_conv2'; 'block{b}_sub' (stride-2 subsample) and 'block{b}_res' (1x1 residual GEMM)
         for b in 2, 3, 4, 13; 'block{b}_sepconv{i}_dw' (a depthwise output, where the depthwise runs as its own kernel);
         'block{b}_sepconv{i}' (a SeparableConv after BatchNorm and ReLU); 'block{b}' for a block output: blocks 2-4 and 13
         after max-pool + residual, blocks 5-12 after the third sepconv + residual (no separate 'block{b}_sepconv3' tag),
         and 'block14' = block14_sepconv2 (no separate tag)."""
         n = int(tiles.shape[0])
+        px = self.config.tile_px
+        if tuple(tiles.shape[1:]) != (px, px, 3):
+            raise ValueError(f"tiles must be [n, {px}, {px}, 3], got {tuple(tiles.shape)}")
+        dt = str(tiles.dtype).replace("torch.", "")
+        if dt not in ("uint8", "float32"):
+            raise TypeError("tiles must be uint8 (raw RGB) or float32 (already per-image standardised), got " + dt)
+        if isinstance(tiles, np.ndarray):
+            tiles = np.ascontiguousarray(tiles)
+        elif not tiles.is_contiguous():
+            raise ValueError("tiles must be contiguous (NHWC)")
+        entry = self.lib.bq_model_debug_stage if dt == "uint8" else self.lib.bq_model_debug_stage_standardized
         cap = n * 149 * 149 * 128
         out = np.empty(cap, np.float32)
         shape = (C.c_int64 * 4)()
-        tiles = np.ascontiguousarray(tiles, dtype=np.uint8)
-        _ffi.check(self.ctx.handle,
-                   self.lib.bq_model_debug_stage(self.h, _ffi.ptr(tiles), n, stage.encode(), _ffi.ptr(out), cap, shape),
+        _ffi.check(self.ctx.handle, entry(self.h, _ffi.ptr(tiles), n, stage.encode(), _ffi.ptr(out), cap, shape),
                    "bq_model_debug_stage")
         s = tuple(int(x) for x in shape)
         return out[: int(np.prod(s))].reshape(s).copy()

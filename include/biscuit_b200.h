@@ -174,7 +174,9 @@ int bq_predict_uq(bq_model* m, const uint8_t* tiles, int64_t n, int32_t T, uint6
 
 /* The reference's LITERAL call (results.py:255-257): tiles already passed through tf.image.per_image_standardization,
  * float32 NHWC [n, 299, 299, 3].  Same outputs; the tile statistics, the standardisation and the stain normaliser are
- * skipped (the first convolution reads the floats as they are). */
+ * skipped (the first convolution reads the floats as they are).  Every value must be finite: a tile holding a NaN or
+ * +-Inf fails the call with BQ_ERR_DATA after the batch, naming the smallest such tile index in the call
+ * ("bq_predict_uq_standardized tile 13: non-finite value"); the other tiles' outputs are written. */
 int bq_predict_uq_standardized(bq_model* m, const float* tiles, int64_t n, int32_t T, uint64_t seed,
                                uint64_t tile_index_base, const uint8_t* masks, float* mean, float* std, float* features);
 
@@ -182,6 +184,9 @@ int bq_predict_uq_standardized(bq_model* m, const float* tiles, int64_t n, int32
  * float32 (NHWC).  Used by tests to localise a mismatch; not part of the reference surface. */
 int bq_model_debug_stage(bq_model* m, const uint8_t* tiles, int64_t n, const char* stage, float* out,
                          int64_t out_capacity, int64_t out_shape[4]);
+/* the same on float32 tiles, through the route of bq_predict_uq_standardized (non-finite values are not reported) */
+int bq_model_debug_stage_standardized(bq_model* m, const float* tiles, int64_t n, const char* stage, float* out,
+                                      int64_t out_capacity, int64_t out_shape[4]);
 /* hidden_0 activations (bf16 as float32) of the first n tiles of the last bq_predict_uq call, when that call held them
  * in one head batch: [n, hidden_width], or [n, T, hidden_width] (one row per sample, T of that call) when dropout on
  * the pooled features is on.  `out` must hold that many floats. */

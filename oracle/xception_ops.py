@@ -18,7 +18,8 @@ Rounding points are taken from the kernels, not from oracle/xception_uq.py:
     K * 2^-23 * sum|a||w|: 2^-23 rather than fp32's unit roundoff 2^-24 allows for accumulation that truncates.
   * max-pool + add, subsample (layers.cuh): exact.
   * block1_conv1 (conv1_sm100.cuh): conv(W, x - m0) over W = hi + mid + lo on the tensor cores, then one fp32 FMA
-    with the per-tile constants g = scale / sd and h = shift - (m - m0) * sum(W) * g.
+    with the per-tile constants g = scale / sd and h = shift - (m - m0) * sum(W) * g.  On float tiles the caller already
+    standardised (conv1_kernel<float>, layers.cuh): 27 fp32 fmas from 0 in (ky, kx, ci) order, then the GEMM epilogue.
   * global average pool (layers.cuh): an n-term fp32 sum and one division.
   * MC-dropout head (gemm hidden_0 + head_sm100.cuh): intervals through the two bf16 activations h1, h2 and the fp32
     prelogits, the softmax bounded through its monotonicity in each logit, then the fp32 allowances of the per-chunk
@@ -110,7 +111,8 @@ class HeadWeights:
 # ------------------------------------------------------------------------------------------------------------------
 class Op:
     """kind: conv1 | conv2 | sub | res | sep (fused depthwise + pointwise) | dw | pw | pooladd.
-    `inputs`: the tags whose outputs feed the op ('tiles' = the uint8 tiles); `layer`: weight name."""
+    `inputs`: the tags whose outputs feed the op ('tiles' = the uint8 tiles, or float32 tiles the caller standardised);
+    `layer`: weight name."""
 
     def __init__(self, tag, kind, inputs, layer=None, relu_in=False, relu_out=False, residual=None):
         self.tag, self.kind, self.inputs, self.layer = tag, kind, list(inputs), layer
@@ -161,8 +163,10 @@ def plan(sepmid: bool = True):
 # share a CPU run of tests/test_backbone_ops_cpu.py found on one synthetic tile, rounded down, the smaller of the two
 # plans; a bound that widened for one op would show here.  The K * 2^-23 accumulation bound is what makes the
 # intervals of the 728- and 1024-deep GEMMs wider (block13_res: K = 728 with little cancellation).
+# "block1_conv1_f32" is block1_conv1 on float tiles (conv1_f32_ref): 0.85 x 0.9914, the smallest share over the four
+# input sets of tests/test_input_route_gpu.py (the +-1e4 set) measured on a B200.
 SINGLE_FLOOR = {
-    "hidden_0": 0.4,
+    "hidden_0": 0.4, "block1_conv1_f32": 0.84,
     "block1_conv1": 0.82, "block1_conv2": 0.75, "block2_res": 0.81, "block2_sepconv1": 0.83, "block2_sepconv2": 0.77,
     "block3_res": 0.74, "block3_sepconv1": 0.8, "block3_sepconv2": 0.69, "block4_res": 0.62, "block4_sepconv1": 0.76,
     "block4_sepconv2": 0.36, "block5_sepconv1": 0.6, "block5_sepconv2": 0.61, "block5": 0.5, "block6_sepconv1": 0.6,
@@ -257,6 +261,35 @@ def conv1_ref(tiles_u8: np.ndarray, ow: OpWeights):
     return z, E
 
 
+def gamma(k: int, u: float = U) -> float:
+    """gamma_k = k u / (1 - k u): the relative error bound of a k-step RN recurrence (Higham, Accuracy and Stability, 3.1)"""
+    return k * u / (1 - k * u)
+
+
+def conv1_f32_ref(tiles_f32, ow: OpWeights):
+    """block1_conv1 on float tiles the caller already standardised (conv1_kernel<float>, layers.cuh): z = BN(conv(W, x))
+    in float64 from the caller's fp32 values x and the fp32 weights W [3, 3, 3, 32] (3x3, stride 2, valid).
+
+    Rounding points of the kernel, per output and channel:
+      * acc = 0, then 27 fp32 fmas acc = RN(x * w + acc) in (ky, kx, ci) order.  Each step rounds once, relative error
+        <= u on the partial sum, so |acc - A| <= gamma_27 * S with A = sum x w and S = sum |x| |w| (Higham 3.1; the
+        bound holds for any summation order, so it does not rely on the order).  Subnormal partial sums add at most
+        2^-150 per step, covered by TINY.  The float64 conv that gives A is itself off by <= gamma_27(2^-53) * S, which
+        is added to the same E so that z is not taken as exact.
+      * RN(acc * scale), RN(+ shift): epilogue_bound.
+      * ReLU and RN to bf16: interval (both monotone).
+    tiles_f32: float32 NHWC [n, 299, 299, 3] (numpy or torch) -> (z, E) [n, 149, 149, 32] float64 on ow.device"""
+    dev = ow.device
+    x = torch.as_tensor(np.asarray(tiles_f32) if not torch.is_tensor(tiles_f32) else tiles_f32)
+    assert x.dtype == torch.float32, x.dtype
+    x = x.to(dev).to(torch.float64).permute(0, 3, 1, 2)
+    W = ow.conv1.to(torch.float64).permute(3, 2, 0, 1)                    # [32, 3, 3, 3] OIHW
+    A = F.conv2d(x, W, stride=2).permute(0, 2, 3, 1)
+    S = F.conv2d(x.abs(), W.abs(), stride=2).permute(0, 2, 3, 1)
+    E = (gamma(27) + gamma(27, 2.0 ** -53)) * S + 27 * TINY
+    return epilogue_bound(A, E, *ow.affine["block1_conv1"])
+
+
 def pooladd_exact(y: torch.Tensor, res: torch.Tensor) -> torch.Tensor:
     """MaxPool 3x3 s2 'same' (-inf padding) + residual: RN_bf16(fp32(max) + fp32(res))"""
     from oracle.xception_uq import _same_pad_s2
@@ -286,7 +319,8 @@ def op_ref(op: Op, ins: dict, ow: OpWeights):
     """-> ('exact', y_ref) or ('bound', (z, E)) for one plan op, from its input tensors `ins` (tag -> tensor)"""
     src = ins[op.inputs[0]]
     if op.kind == "conv1":
-        return "bound", conv1_ref(src, ow)
+        f32 = str(src.dtype).replace("torch.", "") == "float32"            # tiles the caller standardised
+        return "bound", conv1_f32_ref(src, ow) if f32 else conv1_ref(src, ow)
     if op.kind == "conv2":
         return "bound", conv2_ref(src, ow)
     if op.kind == "sub":
@@ -318,12 +352,12 @@ def interval(z, E, relu):
 
 
 def where(bad: torch.Tensor, shape):
-    """failing NHWC coordinates and histograms over image, row, column, channel block and work-item position"""
+    """failing NHWC coordinates and histograms over image, row, column, channel, channel block and work-item position"""
     idx = torch.nonzero(bad.reshape(shape)).cpu().numpy()
     n, h, w, c = shape
     i, y, x, ch = idx.T if len(idx) else (np.zeros(0, int),) * 4
     flat = (i * h + y) * w + x
-    keys = {"image": i, "row": y, "col": x, "c//64": ch // 64, "c//56": ch // 56,
+    keys = {"image": i, "row": y, "col": x, "channel": ch, "c//64": ch // 64, "c//56": ch // 56,
             "last n-block(64)": ch >= (c - 1) // 64 * 64, "gemm row%128": flat % 128}
     if (h, w) == (19, 19):
         keys["sepmid padded row%160"] = ((i * 20 + y) * 20 + x) % 160

@@ -73,3 +73,35 @@ def degenerate_tiles():
     t[2] = 200; t[2, 150, 150, 1] = 201                                 # a single pixel differs
     t[3] = (np.indices((299, 299)).sum(0) % 2 * 255).astype(np.uint8)[..., None]   # checkerboard 0 / 255
     return t
+
+
+def tf_standardize(tiles_u8):
+    """tf.image.per_image_standardization in numpy fp32: (x - mean) / max(std, 1 / sqrt(N)), a division (TF divides; the
+    oracle multiplies by the reciprocal)"""
+    x = tiles_u8.astype(np.float32)
+    n = np.float32(x[0].size)
+    m = x.mean((1, 2, 3), dtype=np.float32, keepdims=True)
+    var = np.maximum((x * x).mean((1, 2, 3), dtype=np.float32, keepdims=True) - m * m, np.float32(0))
+    sd = np.maximum(np.sqrt(var), np.float32(1) / np.sqrt(n))
+    return ((x - m) / sd).astype(np.float32)
+
+
+def float_tile_sets(weights):
+    """name -> 8 float32 NHWC tiles for the route of already-standardised input (`predict` on float32); in each set the
+    first four tiles are synthetic and the last four degenerate, except where noted"""
+    from oracle import synth, xception_uq as X
+    deg = degenerate_tiles()
+    u8 = [np.concatenate([synth.tiles_u8(4, seed=s, n_slides=2), deg]) for s in (0, 1, 2)]
+    nhwc = lambda t: t.permute(0, 2, 3, 1).contiguous().numpy()             # noqa: E731
+    rng = np.random.default_rng(7)
+    big = np.empty((8, 299, 299, 3), np.float32)
+    big[:4] = rng.uniform(-1e4, 1e4, (4, 299, 299, 3))                      # |x| up to 1e4
+    big[4:6] = np.where(rng.random((2, 299, 299, 3)) < 0.5, -1e4, 1e4)      # exactly +-1e4
+    big[6], big[7] = 1e4, -1e4                                              # constant
+    return {
+        # the oracle's (x - mean) * (1 / std): a constant tile becomes exact zeros, the single-pixel tile an outlier of ~518
+        "oracle": nhwc(X.XceptionUQOracle(weights).standardize(u8[0])),
+        "tf": tf_standardize(u8[1]),
+        "raw": u8[2].astype(np.float32),                                    # legal input, not standardised
+        "big": big,
+    }
